@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — MPTI episodes/s (2-way 5-shot, 2048 pts) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" = one pass of the episode hot path over one batch of `--episodes` (default 100) synthetic
 S3DIS-shape 2-way 5-shot episodes (BASELINE.json configs[2]), fed to the C ABI in chunks of
@@ -20,6 +20,9 @@ One JSON line on stdout (rank 0):
   cpu_baseline  the CPU oracle (restatement of the reference's path) on this box's host cores
 `--impl reference` times that CPU path alone (the reference is Python: oracle/mpti_oracle.py is
 its restatement; the reference tree itself cannot travel to the GPU box).
+`--dump-outputs DIR` writes what the last timed step of the headline path returned (rank 0) as
+DIR/logits.npy, loss.npy, pred.npy (float32): the inputs are seeded, so two builds of the project
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -93,6 +96,22 @@ def build_host_batch(n_episodes: int, seed0: int):
         qy[i] = ep.query_y
         classes[i] = ep.sampled_classes
     return sx, sy, qx, qy, classes
+
+
+DUMP_BYTES = 63 * 10**6  # array data; with the .npy headers the dump stays under 64 MB
+
+
+def dump_outputs(out_dir: str, outs):
+    """forward_episodes' outputs of every chunk of one step -> out_dir/{logits,loss,pred}.npy in
+    float32 (pred holds class indices, exact in float32), episodes in input order.  Past DUMP_BYTES
+    in all, only the first episodes are written."""
+    arrays = {k: torch.cat([o[k] for o in outs]).float().cpu().numpy()
+              for k in ("logits", "loss", "pred")}
+    per_episode = sum(a[0].nbytes for a in arrays.values())
+    keep = min(len(arrays["loss"]), DUMP_BYTES // per_episode)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[:keep])
 
 
 # ------------------------------------------------------------------------------------------------
@@ -388,7 +407,11 @@ def main():
                     help="skip the configs[3] / configs[4] / driver legs (profiling runs)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--workload", default="s3dis_2way_5shot", choices=sorted(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's logits / loss / pred as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the b200 path")
     workload_label = set_workload(args.workload)
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3  # timing rule: W >= 3
@@ -442,7 +465,7 @@ def main():
     ws = torch.empty(_lib.lib().r3dfs_mpti_workspace(cfg, chunk), dtype=torch.uint8, device=dev)
     flush = torch.empty(512 << 20, dtype=torch.uint8, device=dev)  # > 126 MB L2
     chunks = [(s, min(s + chunk, E_step)) for s in range(0, E_step, chunk)]
-    preds = [None] * len(chunks)
+    outs = [None] * len(chunks)  # what forward_episodes returned for each chunk of the last step
     n_stage = len(_lib.STAGES)
 
     def new_events():
@@ -465,6 +488,7 @@ def main():
                                              d_qx[a:b].transpose(2, 3), d_qy[a:b], eval=True,
                                              workspace=ws,
                                              stage_events=None if stage_ev is None else stage_ev[ci])
+                outs[ci] = out
                 ops.confusion_accumulate(out["pred"], d_qy[a:b], d_slot[a:b], step_counters)
         else:
             cur = torch.cuda.current_stream()
@@ -476,11 +500,11 @@ def main():
                     out = model.forward_episodes(d_sx[a:b].transpose(3, 4), d_sy[a:b],
                                                  d_qx[a:b].transpose(2, 3), d_qy[a:b], eval=True,
                                                  workspace=wss[ci % n_streams])
-                    preds[ci] = out["pred"]
+                    outs[ci] = out
             for s in streams:
                 cur.wait_stream(s)
             for ci, (a, b) in enumerate(chunks):
-                ops.confusion_accumulate(preds[ci], d_qy[a:b], d_slot[a:b], step_counters)
+                ops.confusion_accumulate(outs[ci]["pred"], d_qy[a:b], d_slot[a:b], step_counters)
         if dist is not None:
             dist.all_reduce(step_counters, op=dist.ReduceOp.SUM)  # the path's only collective
         counters.add_(step_counters)
@@ -541,6 +565,8 @@ def main():
     sync_all()
     wall_resident = time.perf_counter() - wall0
     launches = L.r3dfs_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs)
     # per-stage device times: the same K steps again, serialised on one stream with stage events
     for s in range(args.steps):
         flush.zero_()
@@ -687,11 +713,10 @@ def main():
                                     args.steps, args.warmup)
         set_workload(main_workload)
         torch.cuda.empty_cache()
-        # (20+ timed steps after 8 warm-up steps: with 3 + 10 the 4-GPU run still had NCCL's lazy
-        # set-up of the two new message sizes and the 3.4 GB workspace allocation inside the timed
-        # region — 26.3 ms per step against 17.9 for scripts/bench_train.py alone)
-        extra["train_step"] = train_leg(dev, dist, rank, world, max(20, 2 * args.steps),
-                                        max(8, args.warmup))
+        # (8+ warm-up steps: with 3 the 4-GPU run still had NCCL's lazy set-up of the two new
+        # message sizes and the 3.4 GB workspace allocation inside the timed region — 26.3 ms per
+        # step against 17.9 for scripts/bench_train.py alone)
+        extra["train_step"] = train_leg(dev, dist, rank, world, args.steps, max(8, args.warmup))
 
     cpu_base = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:

@@ -8,6 +8,11 @@ Files (small on purpose; episodes are regenerated from their seed, only outputs 
   golden_protonet.pt   ProtoNet_Contrast.forward (eval) outputs; `python -m oracle.make_golden protonet`
                        writes only this file
   golden_metric.json   evaluate_metric on a seeded random case (`python -m oracle.make_golden metric`)
+  golden_mdns.pt       grid_sampling / Mean_pl_support_y / Mean_pl_support_y_multi_scale on the
+                       support sets of tests.helpers.mdns_case (`python -m oracle.make_golden mdns`).
+                       The committed file was written through the oracle's restatements of those
+                       three methods, which the reference's own methods matched bit for bit on
+                       these inputs (the comparison was run live against the reference tree)
   golden_parity.pt     free-running parity cases (`python -m oracle.make_golden parity`): for the
                        four episode configurations above plus 10 seeds each of BASELINE.json
                        configs[2] (S3DIS-shape 2-way 5-shot) and configs[3] (ScanNet-shape 3-way
@@ -130,12 +135,47 @@ def metric(ref):
     print("golden_metric.json written", miou)
 
 
+MDNS_CASES = [(0, 2, 5), (1, 3, 5), (2, 2, 1)]  # (seed, n_way, k_shot) of tests.helpers.mdns_case
+MDNS_SCALES = [(1, 1, 1), (2, 2, 1)]
+
+
+def mdns(model_of):
+    """Noise-suppression internals (models/mpti.py:87-223, 316-371) on support sets whose
+    foreground points lie exactly on cell faces.  `model_of(n_way, k_shot)` returns an object with
+    the reference's grid_sampling / Mean_pl_support_y / Mean_pl_support_y_multi_scale methods."""
+    from tests.helpers import mdns_case
+    out = {}
+    for seed, n_way, k_shot in MDNS_CASES:
+        sx, sy, sf = mdns_case(seed, n_way, k_shot)
+        m = model_of(n_way, k_shot)
+        case = dict(seed=seed, n_way=n_way, k_shot=k_shot, scales={})
+        for scale in MDNS_SCALES:
+            cells = []
+            for w in range(n_way):
+                for k in range(k_shot):
+                    fg = sy[w, k] == 1
+                    s, a, n = m.grid_sampling(sx[w, k][:, fg].t(), sf[w, k][:, fg].t(), *scale)
+                    # cell indices < 4: int8 keeps the file small; tests compare after .long()
+                    cells.append(dict(seeds=s.clone(), assign=a.to(torch.int8).cpu(), count=int(n)))
+            with ref_shims.quiet():
+                flag = m.Mean_pl_support_y(sf, sy, sy, sx, *scale)[1]
+            case["scales"]["%dx%dx%d" % scale] = dict(cells=cells, flag=flag.clone())
+        with ref_shims.quiet():
+            pl, clean = m.Mean_pl_support_y_multi_scale(sf, sy, sy, sx)
+        case.update(pl=[p.clone() for p in pl], clean=clean.clone())
+        out["seed%d_%dway_%dshot" % (seed, n_way, k_shot)] = case
+    torch.save(out, os.path.join(GOLD, "golden_mdns.pt"))
+    print("golden_mdns.pt written")
+
+
 def main():
     ref = ref_shims.load_reference()
     torch.set_num_threads(os.cpu_count())
     sd = torch.load(os.path.join(GOLD, "weights_fixture.pt"))
     if sys.argv[1:] == ["metric"]:
         return metric(ref)
+    if sys.argv[1:] == ["mdns"]:
+        return mdns(lambda n_way, k_shot: ref.mpti.MPTI_SelfAtten(default_args(n_way, k_shot)))
     if sys.argv[1:] == ["protonet"]:
         return protonet(ref, sd)
     if sys.argv[1:] == ["parity"]:

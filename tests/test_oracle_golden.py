@@ -114,35 +114,32 @@ def test_protonet_oracle_matches_reference(fixture_sd, name):
 # ---------------------------------------------------------------------------------------------
 # pins added in round 2
 # ---------------------------------------------------------------------------------------------
-@pytest.mark.reference
 def test_mdns_internals_pinned_to_reference():
-    """O.grid_sampling / O.mdns_flags_one_scale / O.mdns_multi_scale against the reference's own
-    methods (models/mpti.py:316-371, 87-176, 178-223) on support sets whose foreground points lie
-    exactly on cell faces (inclusive bounds on both sides, later cells overwrite assignments)."""
-    from oracle import ref_shims
-    from r3dfsseg_b200.episodes import default_args
+    """O.grid_sampling / O.mdns_flags_one_scale / O.mdns_multi_scale against what the reference's
+    own methods (models/mpti.py:316-371, 87-176, 178-223) return on support sets whose foreground
+    points lie exactly on cell faces (inclusive bounds on both sides, later cells overwrite
+    assignments); stored in tests/golden/golden_mdns.pt by `python -m oracle.make_golden mdns`."""
+    import os
     from tests.helpers import mdns_case
-    ref = ref_shims.load_reference()
-    for seed, n_way, k_shot in ((0, 2, 5), (1, 3, 5), (2, 2, 1)):
-        sx, sy, sf = mdns_case(seed, n_way, k_shot)
-        m = ref.mpti.MPTI_SelfAtten(default_args(n_way, k_shot))
+    gold = torch.load(os.path.join(os.path.dirname(__file__), "golden", "golden_mdns.pt"))
+    assert len(gold) == 3
+    for g in gold.values():
+        n_way, k_shot = g["n_way"], g["k_shot"]
+        sx, sy, sf = mdns_case(g["seed"], n_way, k_shot)
         for (nx, ny, nz) in ((1, 1, 1), (2, 2, 1)):
+            ref = g["scales"]["%dx%dx%d" % (nx, ny, nz)]
             for w in range(n_way):
                 for k in range(k_shot):
                     fg = sy[w, k] == 1
                     sp, f = sx[w, k][:, fg].t(), sf[w, k][:, fg].t()
-                    s_ref, a_ref, n_ref = m.grid_sampling(sp, f, nx, ny, nz)
+                    cell = ref["cells"][w * k_shot + k]
                     s, a, n = O.grid_sampling(sp, f, nx, ny, nz)
-                    assert n == n_ref and torch.equal(a, a_ref.long().cpu())
-                    assert torch.equal(s, s_ref)
-            with ref_shims.quiet():
-                flag_ref = m.Mean_pl_support_y(sf, sy, sy, sx, nx, ny, nz)[1]
-            assert torch.equal(O.mdns_flags_one_scale(sf, sy, sx, nx, ny, nz), flag_ref)
-        with ref_shims.quiet():
-            pl_ref, clean_ref = m.Mean_pl_support_y_multi_scale(sf, sy, sy, sx)
+                    assert n == cell["count"] and torch.equal(a, cell["assign"].long())
+                    assert torch.equal(s, cell["seeds"])
+            assert torch.equal(O.mdns_flags_one_scale(sf, sy, sx, nx, ny, nz), ref["flag"])
         pl, clean = O.mdns_multi_scale(sf, sy, sx)
-        assert torch.equal(clean, clean_ref)
-        assert all(torch.equal(a, b) for a, b in zip(pl, pl_ref))
+        assert torch.equal(clean, g["clean"])
+        assert len(pl) == len(g["pl"]) and all(torch.equal(a, b) for a, b in zip(pl, g["pl"]))
 
 
 def _metric_case(seed=0, n_eps=7, n_way=3, n_q=3, N=257, pool=6):
@@ -160,34 +157,10 @@ def _metric_case(seed=0, n_eps=7, n_way=3, n_q=3, N=257, pool=6):
     return preds, gts, l2c, test_classes
 
 
-@pytest.mark.reference
-def test_confusion_counts_pinned_to_reference_evaluate_metric():
-    """O.confusion_counts + O.mean_iou == the reference's evaluate_metric (eval_noise.py:23-72),
-    per-class IoU included (read from its log lines)."""
-    import re
-    from oracle import ref_shims
-    ref = ref_shims.load_reference()
-    preds, gts, l2c, test_classes = _metric_case()
-
-    class Log:
-        lines = []
-
-        def cprint(self, s):
-            self.lines.append(s)
-
-    miou_ref = ref.evaluate_metric(Log(), preds, gts, l2c, test_classes)
-    counters = O.confusion_counts(preds, gts, l2c, test_classes)
-    assert O.mean_iou(counters) == pytest.approx(float(miou_ref), abs=1e-12)
-    ious = [float(re.search(r"IoU: ([0-9.]+)", s).group(1)) for s in Log.lines if "IoU:" in s]
-    gt, pos, tp = counters.astype(float)
-    assert len(ious) == counters.shape[1]
-    for c, v in enumerate(ious):
-        assert abs(tp[c] / (gt[c] + pos[c] - tp[c]) - v) < 1e-6
-
-
 def test_confusion_counts_golden():
-    """The same pin from the committed numbers (tests/golden/golden_metric.json, written from the
-    reference's evaluate_metric by `python -m oracle.make_golden metric`)."""
+    """O.confusion_counts + O.mean_iou == the reference's evaluate_metric (eval_noise.py:23-72),
+    per-class IoU included (read from its log lines), from the committed numbers
+    (tests/golden/golden_metric.json, written by `python -m oracle.make_golden metric`)."""
     import json
     import os
     g = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "golden_metric.json")))
@@ -196,6 +169,7 @@ def test_confusion_counts_golden():
     counters = O.confusion_counts(preds, gts, l2c, test_classes)
     assert abs(O.mean_iou(counters) - g["mean_iou"]) < 1e-12
     gt, pos, tp = counters.astype(float)
+    assert len(g["iou"]) == counters.shape[1]
     for c, v in enumerate(g["iou"]):
         assert abs(tp[c] / (gt[c] + pos[c] - tp[c]) - v) < 1e-6
 
