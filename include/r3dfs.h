@@ -327,6 +327,44 @@ int r3dfs_mpti_forward_features(const r3dfs_episode_cfg_t* h_cfg, int n_episodes
                                 float* loss, int32_t* pred, const r3dfs_episode_diag_t* h_diag,
                                 void* ws, size_t ws_bytes, r3dfs_stream_t stream);
 
+/* One support set, many query clouds: r3dfs_mpti_forward cut into its two halves, so that the
+ * part of an episode that depends on the support set alone runs once per set.  Chaining the two
+ * calls on the same episodes returns what r3dfs_mpti_forward returns, bit for bit.  Both accept
+ * the envelope of r3dfs_mpti_forward and return its error codes.
+ *
+ * Support half of MPTI_SelfAtten.forward, eval (models/mpti.py:433-435, 440-493): getFeatures of
+ * the n_sets * n_way * k_shot support clouds only, MDNS when cfg->mdns, fg/bg sets, FPS seeds,
+ * assignment, prototype means.  support_x / support_y as r3dfs_mpti_forward with n_sets sets.
+ *   proto:       (n_sets, n_way+1, n_subprototypes+1, 192) fp32, classes [bg, way 0, ...];
+ *                rows >= proto_count are zero
+ *   proto_count: (n_sets, n_way+1) int32
+ * h_diag: clean_flag and stage events as in r3dfs_mpti_forward (the graph stages are recorded
+ * at the end, with no work between them); the other fields are ignored. */
+size_t r3dfs_mpti_support_workspace(const r3dfs_episode_cfg_t* h_cfg, int n_sets);
+int r3dfs_mpti_support(const r3dfs_episode_cfg_t* h_cfg, const r3dfs_weights_t* h_w, int n_sets,
+                       const float* support_x, int64_t s_e, int64_t s_cloud, int64_t s_c,
+                       int64_t s_n, const int32_t* support_y, float* proto, int32_t* proto_count,
+                       const r3dfs_episode_diag_t* h_diag, void* ws, size_t ws_bytes,
+                       r3dfs_stream_t stream);
+
+/* Query half (models/mpti.py:436-437, 495-571): getFeatures of the E * n_query query clouds only,
+ * then graph, label propagation and head against given prototypes (layout of r3dfs_mpti_support).
+ * p_e / c_e = element stride between episodes in proto / proto_count; 0 = every episode uses the
+ * same support set (no copy).  proto must be 16-byte aligned and p_e a multiple of 4.  Counts are
+ * clamped to [0, n_subprototypes+1]; prototype rows at or past a set's count are read as zero.
+ * Uses n_way, n_query, n_points, n_subprototypes, k_connect, sigma, alpha, cg_* of h_cfg; k_shot
+ * and mdns are ignored, and the workspace does not depend on k_shot.  query_x, query_y, outputs
+ * and h_diag as r3dfs_mpti_forward (proto_count: the clamped counts; clean_flag is not written;
+ * the stages mdns, sets and fps are recorded with no work between them, proto = the copy of the
+ * given prototypes into the graph). */
+size_t r3dfs_mpti_query_workspace(const r3dfs_episode_cfg_t* h_cfg, int n_episodes);
+int r3dfs_mpti_query(const r3dfs_episode_cfg_t* h_cfg, const r3dfs_weights_t* h_w, int n_episodes,
+                     const float* proto, int64_t p_e, const int32_t* proto_count, int64_t c_e,
+                     const float* query_x, int64_t q_e, int64_t q_cloud, int64_t q_c, int64_t q_n,
+                     const int64_t* query_y, float* logits, float* loss, int32_t* pred,
+                     const r3dfs_episode_diag_t* h_diag, void* ws, size_t ws_bytes,
+                     r3dfs_stream_t stream);
+
 /* ProtoNet + MDNS (reference models/protonet.py:357-945 ProtoNet_Contrast.forward, train=False):
  * same encoder and noise suppression as MPTI, then masked average pooling of the support
  * features (:878-890), one prototype per way from the kept shots + one background prototype

@@ -108,6 +108,15 @@ SIGNATURES = {
     "r3dfs_mpti_forward_features": (C.c_int, [C.POINTER(EpisodeCfg), i32, vp, i64, i64, i64, i64, vp,
                                               vp, vp, vp, vp, vp, vp, C.POINTER(EpisodeDiag), vp,
                                               sz, vp]),
+    "r3dfs_mpti_support_workspace": (sz, [C.POINTER(EpisodeCfg), i32]),
+    "r3dfs_mpti_support": (C.c_int, [C.POINTER(EpisodeCfg), C.POINTER(Weights), i32,
+                                     vp, i64, i64, i64, i64, vp, vp, vp,
+                                     C.POINTER(EpisodeDiag), vp, sz, vp]),
+    "r3dfs_mpti_query_workspace": (sz, [C.POINTER(EpisodeCfg), i32]),
+    "r3dfs_mpti_query": (C.c_int, [C.POINTER(EpisodeCfg), C.POINTER(Weights), i32,
+                                   vp, i64, vp, i64,
+                                   vp, i64, i64, i64, i64, vp,
+                                   vp, vp, vp, C.POINTER(EpisodeDiag), vp, sz, vp]),
     "r3dfs_confusion_accumulate": (C.c_int, [vp, vp, vp, i32, i32, i64, i32, vp, vp]),
     "r3dfs_protonet_forward": (C.c_int, [C.POINTER(EpisodeCfg), C.POINTER(Weights), i32,
                                          vp, i64, i64, i64, i64, vp,

@@ -63,6 +63,26 @@ __global__ void graph_init_kernel(const int32_t* __restrict__ proto_cnt, int S, 
   for (int c = 0; c < nc; ++c) Y[((int64_t)g * nn + i) * nc + c] = (v && c == lab) ? 1.f : 0.f;
 }
 
+// given prototypes -> prototype slots of the node matrix (the query half of a split episode): slot
+// s*slot + p of episode e = row (s*slot + p) of proto + e*p_e when p < count, 0 otherwise, and 0 up
+// to ppad; count = proto_count[e*c_e + s] clamped to [0, slot].  One float4 per thread.
+__global__ void proto_rows_kernel(const float* __restrict__ proto, int64_t p_e,
+                                  const int32_t* __restrict__ proto_count, int64_t c_e, int S,
+                                  int slot, int ppad, int64_t f_rows, float* __restrict__ F,
+                                  int32_t* __restrict__ proto_cnt) {
+  constexpr int D4 = R3DFS_FEAT_DIM / 4;
+  const int e = blockIdx.y;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < S) proto_cnt[e * S + i] = min(max(proto_count[e * c_e + i], 0), slot);
+  if (i >= ppad * D4) return;
+  const int r = i / D4, s = r / slot;
+  int cnt = 0;
+  if (s < S) cnt = min(max(proto_count[e * c_e + s], 0), slot);
+  float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (r - s * slot < cnt) v = reinterpret_cast<const float4*>(proto + e * p_e)[i];
+  reinterpret_cast<float4*>(F + e * f_rows * R3DFS_FEAT_DIM)[i] = v;
+}
+
 __global__ void i32_to_i64_kernel(const int32_t* __restrict__ a, int64_t* __restrict__ b,
                                   int64_t n) {
   const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -628,13 +648,8 @@ int episode_dims(const r3dfs_episode_cfg_t* c, EpisodeDims& d) {
   return 0;
 }
 
-void carve_episode(WsBump& ws, const r3dfs_episode_cfg_t* c, const EpisodeDims& d, int E,
-                          int in_dim, int dg_k, EpisodeWs& w) {
-  const int64_t M = (int64_t)E * d.cpe * c->n_points;
-  const size_t G = E, nn = d.nn, k = c->k_connect;
-  w.xp = ws.take<float>(M * in_dim);
-  carve_encoder(ws, M, dg_k, w.enc);
-  w.F = ws.take<float>((size_t)E * d.ep_rows * R3DFS_FEAT_DIM);
+// buffers of the support part (noise suppression, set compaction, prototypes) for G episodes
+static void carve_support_bufs(WsBump& ws, const EpisodeDims& d, size_t G, EpisodeWs& w) {
   w.fg_cnt = ws.take<int32_t>(G * d.C);
   w.keep = ws.take<int32_t>(G * d.C);
   w.set_off = ws.take<int32_t>(G * d.S);
@@ -646,7 +661,6 @@ void carve_episode(WsBump& ws, const r3dfs_episode_cfg_t* c, const EpisodeDims& 
   w.picks = ws.take<int32_t>(G * d.S * d.slot);
   w.pick_cnt = ws.take<int32_t>(G * d.S);
   w.seeds = ws.take<int32_t>(G * d.S * d.slot);
-  w.proto_cnt = ws.take<int32_t>(G * d.S);
   w.assign = ws.take<int32_t>(G * d.ns_pts);
   {
     const size_t ch = multi_prototypes_chunks(d.ns_pts);
@@ -656,6 +670,12 @@ void carve_episode(WsBump& ws, const r3dfs_episode_cfg_t* c, const EpisodeDims& 
   }
   w.cell_mean = ws.take<float>(G * d.C * 5 * R3DFS_FEAT_DIM);
   w.cell_cnt = ws.take<int32_t>(G * d.C * 5);
+}
+
+// buffers of the query part (graph, label propagation) for G episodes
+static void carve_graph_bufs(WsBump& ws, const r3dfs_episode_cfg_t* c, const EpisodeDims& d,
+                             size_t G, EpisodeWs& w) {
+  const size_t nn = d.nn, k = c->k_connect;
   w.valid = ws.take<uint8_t>(G * nn);
   w.Y = ws.take<float>(G * nn * d.nc);
   w.norms = ws.take<float>(G * nn);
@@ -680,6 +700,42 @@ void carve_episode(WsBump& ws, const r3dfs_episode_cfg_t* c, const EpisodeDims& 
   w.AP = ws.take<float>(G * nn * 8);
 }
 
+void carve_episode(WsBump& ws, const r3dfs_episode_cfg_t* c, const EpisodeDims& d, int E,
+                          int in_dim, int dg_k, EpisodeWs& w) {
+  const int64_t M = (int64_t)E * d.cpe * c->n_points;
+  w.xp = ws.take<float>(M * in_dim);
+  carve_encoder(ws, M, dg_k, w.enc);
+  w.F = ws.take<float>((size_t)E * d.ep_rows * R3DFS_FEAT_DIM);
+  carve_support_bufs(ws, d, E, w);
+  w.proto_cnt = ws.take<int32_t>((size_t)E * d.S);
+  carve_graph_bufs(ws, c, d, E, w);
+}
+
+// support call: the support clouds' encoder buffers, their feature rows (n_sets blocks of ns_pts
+// rows) and the support part's buffers; no graph buffers (proto_cnt is the caller's output)
+static void carve_support(WsBump& ws, const r3dfs_episode_cfg_t* c, const EpisodeDims& d,
+                          int n_sets, int in_dim, int dg_k, EpisodeWs& w) {
+  const int64_t M = (int64_t)n_sets * d.C * c->n_points;
+  w = EpisodeWs{};
+  w.xp = ws.take<float>(M * in_dim);
+  carve_encoder(ws, M, dg_k, w.enc);
+  w.F = ws.take<float>((size_t)n_sets * d.ns_pts * R3DFS_FEAT_DIM);
+  carve_support_bufs(ws, d, n_sets, w);
+}
+
+// query call: the query clouds' encoder buffers, nodes-only feature blocks (nn rows per episode:
+// prototype slots, then query points), the clamped prototype counts and the graph buffers
+static void carve_query(WsBump& ws, const r3dfs_episode_cfg_t* c, const EpisodeDims& d, int E,
+                        int in_dim, int dg_k, EpisodeWs& w) {
+  const int64_t M = (int64_t)E * c->n_query * c->n_points;
+  w = EpisodeWs{};
+  w.xp = ws.take<float>(M * in_dim);
+  carve_encoder(ws, M, dg_k, w.enc);
+  w.F = ws.take<float>((size_t)E * d.nn * R3DFS_FEAT_DIM);
+  w.proto_cnt = ws.take<int32_t>((size_t)E * d.S);
+  carve_graph_bufs(ws, c, d, E, w);
+}
+
 // floats of the D2 area of G graphs: the n x n distance matrix, or the solver scratch if that is larger
 size_t episode_d2_floats(size_t G, size_t nn, int k) {
   const size_t dense = G * nn * nn, solver = (lp_solver_scratch_bytes(G, nn, k) + 3) / 4;
@@ -695,45 +751,54 @@ size_t r3dfs_mpti_workspace(const r3dfs_episode_cfg_t* cfg, int n_episodes) {
   return ws.off + 4096;
 }
 
-// graph half of the episode: F already holds the query + support features (rows ppad.. of every
-// episode block); everything after getFeatures in models/mpti.py:440-571.
-int episode_graph_half(const r3dfs_episode_cfg_t* cfg, const EpisodeDims& d, int E,
-                              const EpisodeWs& w, const float* support_x, int64_t s_e,
-                              int64_t s_cloud, int64_t s_c, int64_t s_n, const int32_t* support_y,
-                              const int64_t* query_y, float* logits, float* loss, int32_t* pred,
-                              const r3dfs_episode_diag_t* diag, cudaStream_t st, bool latency) {
+// support part of the episode (models/mpti.py:440-493): noise suppression, fg/bg sets, FPS seeds,
+// assignment, prototype means.  F rows [sup_off, sup_off + ns_pts) of every f_rows-row block hold
+// the support features; prototype p of set s of episode e is written to row
+// e * proto_rows + s * slot + p of `proto` (rows p >= w.proto_cnt are not written).
+static int episode_support_part(const r3dfs_episode_cfg_t* cfg, const EpisodeDims& d, int E,
+                                const EpisodeWs& w, int64_t f_rows, int64_t sup_off,
+                                const float* support_x, int64_t s_e, int64_t s_cloud, int64_t s_c,
+                                int64_t s_n, const int32_t* support_y, float* proto,
+                                int64_t proto_rows, float* clean_flag, cudaStream_t st,
+                                const StageRec* sr) {
   const int N = cfg->n_points, D = R3DFS_FEAT_DIM;
-  StageRec srv{diag ? (cudaEvent_t*)diag->h_stage_events : nullptr};
-  const StageRec* sr = srv.ev ? &srv : nullptr;
-  cudaError_t ce = cudaMemset2DAsync(w.F, sizeof(float) * d.ep_rows * D, 0,
-                                     sizeof(float) * (size_t)d.ppad * D, E, st);
-  if (ce != cudaSuccess) return (int)ce;
   // noise suppression over support shots (eval only, models/mpti.py:440-442)
-  const int64_t sup_off = d.nn;
   if (cfg->mdns) {
-    R3DFS_TRY(launch_mdns(support_x, s_e, s_cloud, s_c, s_n, support_y, w.F, d.ep_rows, sup_off, E,
+    R3DFS_TRY(launch_mdns(support_x, s_e, s_cloud, s_c, s_n, support_y, w.F, f_rows, sup_off, E,
                           cfg->n_way, cfg->k_shot, N, D, w.cell_mean, w.cell_cnt, w.fg_cnt, w.keep,
-                          diag ? diag->clean_flag : nullptr, st));
+                          clean_flag, st));
   } else {
     fill_i32_kernel<<<nblk((int64_t)E * d.C), 256, 0, st>>>(w.keep, (int64_t)E * d.C, 1);
     R3DFS_CHECK_LAUNCH();
   }
   if (sr) sr->mark(R3DFS_ST_MDNS, st);
-  // prototype sets -> FPS seeds -> assignment -> means, into the prototype slots of F
-  R3DFS_TRY(launch_set_compaction(w.F, d.ep_rows, sup_off, E, cfg->n_way, cfg->k_shot, N, D,
+  // prototype sets -> FPS seeds -> assignment -> means
+  R3DFS_TRY(launch_set_compaction(w.F, f_rows, sup_off, E, cfg->n_way, cfg->k_shot, N, D,
                                   support_y, w.keep, w.fg_cnt, w.set_off, w.set_n, w.cloud_bg_off,
                                   w.cloud_fg_off, w.setfeat, st));
   if (sr) sr->mark(R3DFS_ST_SETS, st);
   R3DFS_TRY(launch_multi_prototypes(w.setfeat, D, w.set_off, w.set_n, E * d.S, d.ns_pts,
                                     cfg->n_subprototypes, w.picks, w.pick_cnt, w.seeds,
                                     w.proto_cnt, w.assign, w.partial, w.pcount, w.seed_stats, d.S,
-                                    d.ep_rows, w.F, D, st, sr, w.fps_spill, d.S));
+                                    proto_rows, proto, D, st, sr, w.fps_spill, d.S));
   if (sr) sr->mark(R3DFS_ST_PROTO, st);
+  return 0;
+}
+
+// query part of the episode (models/mpti.py:493-571): F holds, in blocks of f_rows rows per
+// episode, the prototype slots (rows [0, ppad), zero where no prototype) and the query features
+// (rows [ppad, nn)); w.proto_cnt the prototype count of every set.  Graph, label propagation, head.
+static int episode_query_part(const r3dfs_episode_cfg_t* cfg, const EpisodeDims& d, int E,
+                              const EpisodeWs& w, int64_t f_rows, const int64_t* query_y,
+                              float* logits, float* loss, int32_t* pred,
+                              const r3dfs_episode_diag_t* diag, cudaStream_t st,
+                              const StageRec* sr, bool latency) {
+  const int D = R3DFS_FEAT_DIM;
   // graph: nodes = [prototype slots | query points]
   graph_init_kernel<<<dim3(nblk(d.nn), E), 256, 0, st>>>(w.proto_cnt, d.S, d.slot, d.ppad, d.nn,
                                                          d.nc, w.valid, w.Y);
   R3DFS_CHECK_LAUNCH();
-  R3DFS_TRY(launch_affinity(w.F, d.ep_rows, 0, w.valid, E, d.nn, D, cfg->k_connect, cfg->sigma,
+  R3DFS_TRY(launch_affinity(w.F, f_rows, 0, w.valid, E, d.nn, D, cfg->k_connect, cfg->sigma,
                             w.norms, w.D2, w.nbr, w.sim, st, sr));
   R3DFS_TRY(launch_label_propagate(w.nbr, w.sim, w.valid, E, d.nn, cfg->k_connect, w.Y, d.nc,
                                    cfg->alpha, cfg->cg_tol, cfg->cg_max_iter, w.in_cnt, w.in_ptr,
@@ -747,11 +812,61 @@ int episode_graph_half(const r3dfs_episode_cfg_t* cfg, const EpisodeDims& d, int
   R3DFS_TRY(launch_query_head(w.Z, E, d.nn, d.ppad, d.nq_pts, d.nc, query_y, logits, loss, pred, st));
   if (sr) sr->mark(R3DFS_ST_HEAD, st);
   if (diag && diag->proto_count) {
-    ce = cudaMemcpyAsync(diag->proto_count, w.proto_cnt, sizeof(int32_t) * (size_t)E * d.S,
-                         cudaMemcpyDeviceToDevice, st);
+    cudaError_t ce = cudaMemcpyAsync(diag->proto_count, w.proto_cnt,
+                                     sizeof(int32_t) * (size_t)E * d.S, cudaMemcpyDeviceToDevice, st);
     if (ce != cudaSuccess) return (int)ce;
   }
   return 0;
+}
+
+// graph half of the episode: F already holds the query + support features (rows ppad.. of every
+// episode block); everything after getFeatures in models/mpti.py:440-571.  The prototypes go
+// straight into the prototype slots of F.
+int episode_graph_half(const r3dfs_episode_cfg_t* cfg, const EpisodeDims& d, int E,
+                              const EpisodeWs& w, const float* support_x, int64_t s_e,
+                              int64_t s_cloud, int64_t s_c, int64_t s_n, const int32_t* support_y,
+                              const int64_t* query_y, float* logits, float* loss, int32_t* pred,
+                              const r3dfs_episode_diag_t* diag, cudaStream_t st, bool latency) {
+  const int D = R3DFS_FEAT_DIM;
+  StageRec srv{diag ? (cudaEvent_t*)diag->h_stage_events : nullptr};
+  const StageRec* sr = srv.ev ? &srv : nullptr;
+  cudaError_t ce = cudaMemset2DAsync(w.F, sizeof(float) * d.ep_rows * D, 0,
+                                     sizeof(float) * (size_t)d.ppad * D, E, st);
+  if (ce != cudaSuccess) return (int)ce;
+  R3DFS_TRY(episode_support_part(cfg, d, E, w, d.ep_rows, d.nn, support_x, s_e, s_cloud, s_c, s_n,
+                                 support_y, w.F, d.ep_rows, diag ? diag->clean_flag : nullptr, st,
+                                 sr));
+  return episode_query_part(cfg, d, E, w, d.ep_rows, query_y, logits, loss, pred, diag, st, sr,
+                            latency);
+}
+
+size_t r3dfs_mpti_support_workspace(const r3dfs_episode_cfg_t* cfg, int n_sets) {
+  EpisodeDims d;
+  if (episode_dims(cfg, d) != 0 || n_sets <= 0) return 0;
+  WsBump ws(nullptr, ~(size_t)0);
+  EpisodeWs w;
+  carve_support(ws, cfg, d, n_sets, 64, 32, w);
+  return ws.off + 4096;
+}
+
+// the query call uses no k_shot: its dims are taken with k_shot = 1, so that neither the envelope
+// check nor the workspace depends on it
+static int query_dims(const r3dfs_episode_cfg_t* cfg, r3dfs_episode_cfg_t& qc, EpisodeDims& d) {
+  if (!cfg) return R3DFS_E_BADARG;
+  qc = *cfg;
+  qc.k_shot = 1;
+  qc.mdns = 0;
+  return episode_dims(&qc, d);
+}
+
+size_t r3dfs_mpti_query_workspace(const r3dfs_episode_cfg_t* cfg, int n_episodes) {
+  r3dfs_episode_cfg_t qc;
+  EpisodeDims d;
+  if (query_dims(cfg, qc, d) != 0 || n_episodes <= 0) return 0;
+  WsBump ws(nullptr, ~(size_t)0);
+  EpisodeWs w;
+  carve_query(ws, &qc, d, n_episodes, 64, 32, w);
+  return ws.off + 4096;
 }
 
 extern "C" {
@@ -871,6 +986,93 @@ int r3dfs_mpti_forward_features(const r3dfs_episode_cfg_t* cfg, int E, const flo
   if (ce != cudaSuccess) return (int)ce;
   return episode_graph_half(cfg, d, E, w, support_x, s_e, s_cloud, s_c, s_n, support_y, query_y,
                             logits, loss, pred, diag, st);
+}
+
+// stage events a half does not run are recorded where it stands, so every interval is defined
+static void mark_stages(const StageRec* sr, int first, int last, cudaStream_t st) {
+  if (!sr) return;
+  for (int i = first; i <= last; ++i) sr->mark(i, st);
+}
+
+int r3dfs_mpti_support(const r3dfs_episode_cfg_t* cfg, const r3dfs_weights_t* hw, int n_sets,
+                       const float* support_x, int64_t s_e, int64_t s_cloud, int64_t s_c,
+                       int64_t s_n, const int32_t* support_y, float* proto, int32_t* proto_count,
+                       const r3dfs_episode_diag_t* diag, void* wsp, size_t ws_bytes,
+                       r3dfs_stream_t stream) {
+  EpisodeDims d;
+  R3DFS_TRY(episode_dims(cfg, d));
+  R3DFS_TRY(check_weights(hw));
+  if (!support_x || !support_y || !proto || !proto_count || !wsp || n_sets <= 0)
+    return R3DFS_E_BADARG;
+  if ((int64_t)n_sets * d.C > 65535) return R3DFS_E_UNSUPPORTED;
+  if (ws_bytes < r3dfs_mpti_support_workspace(cfg, n_sets)) return R3DFS_E_WORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int N = cfg->n_points, in_dim = hw->in_dim, D = R3DFS_FEAT_DIM;
+  WsBump ws(wsp, ws_bytes);
+  EpisodeWs w;
+  carve_support(ws, cfg, d, n_sets, in_dim, hw->dgcnn_k, w);
+  if (!ws.ok()) return R3DFS_E_WORKSPACE;
+  w.proto_cnt = proto_count;
+  StageRec srv{diag ? (cudaEvent_t*)diag->h_stage_events : nullptr};
+  const StageRec* sr = srv.ev ? &srv : nullptr;
+  if (sr) sr->mark(R3DFS_ST_BEGIN, st);
+  const int64_t proto_rows = (int64_t)d.S * d.slot;
+  cudaError_t ce = cudaMemsetAsync(proto, 0, sizeof(float) * (size_t)n_sets * proto_rows * D, st);
+  if (ce != cudaSuccess) return (int)ce;
+  const int64_t tsup = (int64_t)n_sets * d.C * N * in_dim;
+  gather_clouds_kernel<<<nblk(tsup), 256, 0, st>>>(support_x, d.C, in_dim, N, s_e, s_cloud, s_c,
+                                                   s_n, d.C, 0, w.xp, tsup);
+  R3DFS_CHECK_LAUNCH();
+  if (sr) sr->mark(R3DFS_ST_INPUT, st);
+  // features of the support clouds only (models/mpti.py:433-435), ns_pts rows per set
+  RowMap fmap{d.C, N, (int64_t)d.ns_pts, 0};
+  R3DFS_TRY(encoder_forward(hw, w.xp, (int64_t)n_sets * d.C, N, w.enc, w.F, fmap, nullptr, st, sr));
+  R3DFS_TRY(episode_support_part(cfg, d, n_sets, w, d.ns_pts, 0, support_x, s_e, s_cloud, s_c, s_n,
+                                 support_y, proto, proto_rows, diag ? diag->clean_flag : nullptr,
+                                 st, sr));
+  mark_stages(sr, R3DFS_ST_DIST, R3DFS_ST_HEAD, st);
+  return 0;
+}
+
+int r3dfs_mpti_query(const r3dfs_episode_cfg_t* cfg, const r3dfs_weights_t* hw, int E,
+                     const float* proto, int64_t p_e, const int32_t* proto_count, int64_t c_e,
+                     const float* query_x, int64_t q_e, int64_t q_cloud, int64_t q_c, int64_t q_n,
+                     const int64_t* query_y, float* logits, float* loss, int32_t* pred,
+                     const r3dfs_episode_diag_t* diag, void* wsp, size_t ws_bytes,
+                     r3dfs_stream_t stream) {
+  r3dfs_episode_cfg_t qc;
+  EpisodeDims d;
+  R3DFS_TRY(query_dims(cfg, qc, d));
+  R3DFS_TRY(check_weights(hw));
+  if (!proto || !proto_count || !query_x || !logits || !wsp || E <= 0 || p_e < 0 || c_e < 0)
+    return R3DFS_E_BADARG;
+  if ((int64_t)E * qc.n_query > 65535) return R3DFS_E_UNSUPPORTED;
+  if (((uintptr_t)proto & 15) != 0 || (p_e & 3) != 0) return R3DFS_E_ALIGN;
+  if (ws_bytes < r3dfs_mpti_query_workspace(cfg, E)) return R3DFS_E_WORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int N = qc.n_points, in_dim = hw->in_dim;
+  WsBump ws(wsp, ws_bytes);
+  EpisodeWs w;
+  carve_query(ws, &qc, d, E, in_dim, hw->dgcnn_k, w);
+  if (!ws.ok()) return R3DFS_E_WORKSPACE;
+  StageRec srv{diag ? (cudaEvent_t*)diag->h_stage_events : nullptr};
+  const StageRec* sr = srv.ev ? &srv : nullptr;
+  if (sr) sr->mark(R3DFS_ST_BEGIN, st);
+  const int64_t tq = (int64_t)E * qc.n_query * N * in_dim;
+  gather_clouds_kernel<<<nblk(tq), 256, 0, st>>>(query_x, qc.n_query, in_dim, N, q_e, q_cloud, q_c,
+                                                 q_n, qc.n_query, 0, w.xp, tq);
+  R3DFS_CHECK_LAUNCH();
+  if (sr) sr->mark(R3DFS_ST_INPUT, st);
+  // features of the query clouds only (models/mpti.py:436-437), after the prototype slots
+  RowMap fmap{qc.n_query, N, (int64_t)d.nn, (int64_t)d.ppad};
+  R3DFS_TRY(encoder_forward(hw, w.xp, (int64_t)E * qc.n_query, N, w.enc, w.F, fmap, nullptr, st,
+                            sr));
+  mark_stages(sr, R3DFS_ST_MDNS, R3DFS_ST_FPS, st);
+  proto_rows_kernel<<<dim3(nblk((int64_t)d.ppad * (R3DFS_FEAT_DIM / 4)), E), 256, 0, st>>>(
+      proto, p_e, proto_count, c_e, d.S, d.slot, d.ppad, d.nn, w.F, w.proto_cnt);
+  R3DFS_CHECK_LAUNCH();
+  if (sr) sr->mark(R3DFS_ST_PROTO, st);
+  return episode_query_part(&qc, d, E, w, d.nn, query_y, logits, loss, pred, diag, st, sr, false);
 }
 
 }  // extern "C"

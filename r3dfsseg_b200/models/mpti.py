@@ -5,11 +5,15 @@
 arity; in eval mode the whole episode — features, multi-scale degree-based noise suppression,
 FPS multi-prototypes, k-NN Gaussian affinity graph, label propagation, loss — is ONE call into
 libr3dfs.so (`r3dfs_mpti_forward`), with no host synchronisation inside.  `forward_episodes`
-runs a batch of independent episodes through the same call.  State-dict keys are the reference's.
+runs a batch of independent episodes through the same call.  `encode_support` / `segment` split
+that call in two, so that a labelled support set is encoded once and any number of query clouds
+are segmented against it (`r3dfs_mpti_support` / `r3dfs_mpti_query`).  State-dict keys are the
+reference's.
 """
 from __future__ import annotations
 
-from typing import Optional
+from dataclasses import dataclass
+from typing import Optional, Sequence, Tuple
 
 import torch
 import torch.nn as nn
@@ -43,6 +47,28 @@ class BaseLearner(nn.Module):
             act = ops.ACT_RELU if i != self.num_convs - 1 else ops.ACT_NONE
             h = ops.op.linear(h.contiguous(), seq[0].weight.reshape(seq[0].weight.shape[0], -1), s, t, act)
         return h.reshape(B, N, -1).transpose(1, 2)
+
+
+@dataclass
+class SupportSet:
+    """What `MPTI_SelfAtten.encode_support` keeps of S support sets: the prototypes
+    (S, n_way+1, n_subprototypes+1, 192) of classes [bg, way 0, ...] (rows past a set's count are
+    zero), their counts proto_count (S, n_way+1) int32, the noise-suppression flags clean_flag
+    (S, n_way, k_shot) (1 = shot kept; all ones without MDNS), the configuration they were built
+    with, and the signature of the weights and BatchNorm statistics they were encoded under."""
+    prototypes: torch.Tensor
+    proto_count: torch.Tensor
+    clean_flag: torch.Tensor
+    n_way: int
+    k_shot: int
+    n_points: int
+    n_subprototypes: int
+    mdns: bool
+    weights_sig: Tuple
+
+    @property
+    def n_sets(self) -> int:
+        return int(self.prototypes.shape[0])
 
 
 class MPTI_SelfAtten(nn.Module):
@@ -85,11 +111,16 @@ class MPTI_SelfAtten(nn.Module):
             if self._packed is None:
                 raise RuntimeError("call model.pack_weights() once before tracing the module")
             return self._packed
-        sig = tuple((t.data_ptr(), t._version) for t in self.state_dict(keep_vars=True).values())
+        sig = self._state_sig()
         if self._packed is None or sig != self._packed_sig:
             self._packed = ops.PackedWeights(self)
             self._packed_sig = sig
         return self._packed
+
+    def _state_sig(self) -> Tuple:
+        # storage and version counter of every parameter and buffer: changes with any in-place
+        # update (optimizer step, load_state_dict, BatchNorm statistics)
+        return tuple((t.data_ptr(), t._version) for t in self.state_dict(keep_vars=True).values())
 
     def pack_weights(self) -> ops.PackedWeights:
         """Folds the BatchNorm statistics into per-channel scale/shift and packs the 31 weight
@@ -138,6 +169,76 @@ class MPTI_SelfAtten(nn.Module):
                                 want_diag=want_diag, workspace=workspace,
                                 support_feat=support_feat, query_feat=query_feat,
                                 stage_events=stage_events)
+
+    # ---------------------------------------------------------------------------------------
+    def encode_support(self, support_x, support_y, eval=True) -> SupportSet:
+        """Support half of forward (models/mpti.py:433-435, 440-493), run once for a labelled
+        support set: (n_way, k_shot, C, N) / (n_way, k_shot, N) for one set, or a leading S for
+        S sets.  eval=True runs the noise suppression, exactly as forward(eval=True).  The result
+        is handed to `segment` as often as wanted."""
+        if self.training:
+            raise NotImplementedError("r3dfsseg_b200: stand-alone call in training mode; use "
+                                      "forward(..., train=True) for the training step or .eval()")
+        if support_x.dim() == 4:
+            support_x, support_y = support_x.unsqueeze(0), support_y.unsqueeze(0)
+        if support_x.dim() != 5 or support_y.dim() != 4:
+            raise ValueError("support_x must be (n_way, k_shot, C, N) or (S, n_way, k_shot, C, N)")
+        S, n_way, k_shot, _, N = support_x.shape
+        if (n_way, N) != (self.n_way, self.n_points):
+            raise ValueError(f"support set of {n_way} ways x {N} points for a model of "
+                             f"{self.n_way} ways x {self.n_points} points")
+        pw = self._weights()
+        sig = None if torch.compiler.is_compiling() else self._packed_sig
+        # the envelope is checked for one query cloud per way (the reference's episodes)
+        proto, count, clean = ops.op.mpti_support(pw.tensors, self.in_channels, int(self.encoder.k),
+                                                  support_x, support_y, n_way,
+                                                  self.n_subprototypes, self.k_connect, bool(eval))
+        return SupportSet(proto, count, clean, int(n_way), int(k_shot), int(N),
+                          int(self.n_subprototypes), bool(eval), sig)
+
+    def segment(self, support: SupportSet, query_x, query_y=None,
+                set_index: Optional[Sequence[int]] = None):
+        """Query half of forward (models/mpti.py:436-437, 495-571) against an encoded support set.
+        query_x (E, n_query, C, N) [query_y (E, n_query, N)]: episode i uses set i when the
+        support holds E sets, the one set when it holds one (read in place), or set set_index[i].
+        Returns dict(logits (E, n_query, N, n_way+1), loss (E), pred (E, n_query, N)), equal bit
+        for bit to forward_episodes on the same supports.  A 3-D query_x (n_query, C, N) is one
+        episode and returns what forward returns: (query_pred (n_query, n_way+1, N), loss)."""
+        if self.training:
+            raise NotImplementedError("r3dfsseg_b200: stand-alone call in training mode; use "
+                                      "forward(..., train=True) for the training step or .eval()")
+        if (support.n_way, support.n_points, support.n_subprototypes) != \
+                (self.n_way, self.n_points, self.n_subprototypes):
+            raise ValueError(
+                f"support set built for n_way={support.n_way} n_points={support.n_points} "
+                f"n_subprototypes={support.n_subprototypes}; the model has n_way={self.n_way} "
+                f"n_points={self.n_points} n_subprototypes={self.n_subprototypes}")
+        single = query_x.dim() == 3
+        if single:
+            query_x = query_x.unsqueeze(0)
+            query_y = None if query_y is None else query_y.unsqueeze(0)
+        E, S = query_x.shape[0], support.n_sets
+        proto, count, shared = support.prototypes, support.proto_count, False
+        if set_index is not None:
+            idx = [int(i) for i in set_index]
+            if len(idx) != E or any(i < 0 or i >= S for i in idx):
+                raise ValueError(f"set_index must hold {E} indices in [0, {S}); got {idx}")
+            sel = torch.tensor(idx, dtype=torch.int64, device=proto.device)
+            proto, count = proto.index_select(0, sel), count.index_select(0, sel)
+        elif S == 1:
+            shared = True
+        elif S != E:
+            raise ValueError(f"{S} support sets for {E} query episodes: pass set_index")
+        pw = self._weights()
+        if not torch.compiler.is_compiling() and self._packed_sig != support.weights_sig:
+            raise RuntimeError("the weights or BatchNorm statistics changed after the support set "
+                               "was encoded: its prototypes are stale, call encode_support again")
+        r = ops.op.mpti_query(pw.tensors, self.in_channels, int(self.encoder.k), proto, count,
+                              query_x, query_y, shared, support.k_shot, self.k_connect,
+                              float(self.sigma), self.lp_alpha, self.cg_max_iter, self.cg_tol, None)
+        if single:
+            return r[0][0].transpose(1, 2), r[1][0]
+        return {"logits": r[0], "loss": r[1], "pred": r[2]}
 
     def forward(self, support_x, support_y, query_x, query_y, gt_support_y=None, gt_query_y=None,
                 train=False, logger=None, step=None, path=None, sampled_classes=None,

@@ -386,6 +386,26 @@ def make_cfg(n_way: int, k_shot: int, n_query: int, n_points: int, n_subprototyp
                       float(alpha), int(bool(mdns)), int(cg_max_iter), float(cg_tol))
 
 
+def _envelope_error(cfg: EpisodeCfg) -> "_lib.R3dfsError":
+    """What a workspace query of 0 means for an episode configuration."""
+    return _lib.R3dfsError(
+        "episode configuration outside what libr3dfs is built for: n_way 1..7, k_shot 1..32, "
+        "n_points >= 64, n_subprototypes 1..127, k_connect 1..1024 and < n_queries * n_points, "
+        "graph nodes = roundup64((n_way + 1) * (n_subprototypes + 1)) + n_queries * n_points <= 8192 "
+        "(the merged rows index columns with 16 bits and the CG kernels stage 8192 nodes); got "
+        f"n_way={cfg.n_way} k_shot={cfg.k_shot} n_query={cfg.n_query} n_points={cfg.n_points} "
+        f"n_subprototypes={cfg.n_subprototypes} k_connect={cfg.k_connect}")
+
+
+def _stage_event_array(stage_events: Optional[Sequence["torch.cuda.Event"]]):
+    """Raw cudaEvent_t handles of caller-owned torch events (created by a first record())."""
+    if stage_events is None:
+        return None
+    if len(stage_events) != len(_lib.STAGES):
+        raise ValueError(f"need {len(_lib.STAGES)} stage events")
+    return (C.c_void_p * len(stage_events))(*[int(e.cuda_event) for e in stage_events])
+
+
 def _mpti_forward_raw(pw: Optional[PackedWeights], cfg: EpisodeCfg, support_x: torch.Tensor,
                  support_y: torch.Tensor, query_x: torch.Tensor, query_y: Optional[torch.Tensor],
                  want_diag: bool = False, workspace: Optional[torch.Tensor] = None,
@@ -414,22 +434,11 @@ def _mpti_forward_raw(pw: Optional[PackedWeights], cfg: EpisodeCfg, support_x: t
     L = _lib.lib()
     need = L.r3dfs_mpti_workspace(C.byref(cfg), E)
     if need == 0:
-        raise _lib.R3dfsError(
-            "episode configuration outside what libr3dfs is built for: n_way 1..7, k_shot 1..32, "
-            "n_points >= 64, n_subprototypes 1..127, k_connect 1..1024 and < n_queries * n_points, "
-            "graph nodes = roundup64((n_way + 1) * (n_subprototypes + 1)) + n_queries * n_points <= 8192 "
-            "(the merged rows index columns with 16 bits and the CG kernels stage 8192 nodes); got "
-            f"n_way={cfg.n_way} k_shot={cfg.k_shot} n_query={cfg.n_query} n_points={cfg.n_points} "
-            f"n_subprototypes={cfg.n_subprototypes} k_connect={cfg.k_connect}")
+        raise _envelope_error(cfg)
     ws = workspace if workspace is not None and workspace.numel() >= need else _ws(need, dev)
     diag = None
     dstruct = None
-    ev_arr = None
-    if stage_events is not None:
-        # raw cudaEvent_t handles of caller-owned torch events (created by a first record())
-        if len(stage_events) != len(_lib.STAGES):
-            raise ValueError(f"need {len(_lib.STAGES)} stage events")
-        ev_arr = (C.c_void_p * len(stage_events))(*[int(e.cuda_event) for e in stage_events])
+    ev_arr = _stage_event_array(stage_events)
     if want_diag or ev_arr is not None:
         dstruct = EpisodeDiag(None, None, None, None, None)
     if want_diag:
@@ -508,13 +517,7 @@ def protonet_forward(pw: PackedWeights, cfg: EpisodeCfg, support_x: torch.Tensor
     L = _lib.lib()
     need = L.r3dfs_mpti_workspace(C.byref(cfg), E)
     if need == 0:
-        raise _lib.R3dfsError(
-            "episode configuration outside what libr3dfs is built for: n_way 1..7, k_shot 1..32, "
-            "n_points >= 64, n_subprototypes 1..127, k_connect 1..1024 and < n_queries * n_points, "
-            "graph nodes = roundup64((n_way + 1) * (n_subprototypes + 1)) + n_queries * n_points <= 8192 "
-            "(the merged rows index columns with 16 bits and the CG kernels stage 8192 nodes); got "
-            f"n_way={cfg.n_way} k_shot={cfg.k_shot} n_query={cfg.n_query} n_points={cfg.n_points} "
-            f"n_subprototypes={cfg.n_subprototypes} k_connect={cfg.k_connect}")
+        raise _envelope_error(cfg)
     ws = workspace if workspace is not None and workspace.numel() >= need else _ws(need, dev)
     with torch.cuda.device(dev):
         check(L.r3dfs_protonet_forward(
@@ -525,6 +528,107 @@ def protonet_forward(pw: PackedWeights, cfg: EpisodeCfg, support_x: torch.Tensor
             _p(query_y), 0, _p(logits), _p(loss), _p(pred), _p(clean), _p(ws), ws.numel(),
             _stream()), "r3dfs_protonet_forward")
     return {"logits": logits, "loss": loss, "pred": pred, "clean_flag": clean}
+
+
+def _mpti_support_raw(pw: PackedWeights, cfg: EpisodeCfg, support_x: torch.Tensor,
+                      support_y: torch.Tensor, want_diag: bool = False,
+                      stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
+    """The support half of S episodes in one call (r3dfs_mpti_support).
+    support_x (S, n_way, k_shot, C, N) any strides with uniform cloud stride, support_y
+    (S, n_way, k_shot, N).  Returns (proto (S, n_way+1, n_subprototypes+1, 192), proto_count
+    (S, n_way+1) int32, clean_flag (S, n_way, k_shot) or None without want_diag)."""
+    dev = _need_cuda(support_x, support_y)
+    support_x = _f32(support_x)
+    S, n_way, k_shot, Cin, N = support_x.shape
+    if (n_way, k_shot, N) != (cfg.n_way, cfg.k_shot, cfg.n_points):
+        raise ValueError("support tensors do not match the episode configuration")
+    if support_x.stride(1) != k_shot * support_x.stride(2):
+        support_x = support_x.contiguous()
+    support_y = support_y.to(torch.int32).contiguous()
+    nc = n_way + 1
+    proto = torch.empty((S, nc, cfg.n_subprototypes + 1, 192), dtype=torch.float32, device=dev)
+    count = torch.empty((S, nc), dtype=torch.int32, device=dev)
+    clean = torch.ones((S, n_way, k_shot), dtype=torch.float32, device=dev) if want_diag else None
+    L = _lib.lib()
+    need = L.r3dfs_mpti_support_workspace(C.byref(cfg), S)
+    if need == 0:
+        raise _envelope_error(cfg)
+    ws = _ws(need, dev)
+    ev_arr = _stage_event_array(stage_events)
+    dstruct = None
+    if want_diag or ev_arr is not None:
+        dstruct = EpisodeDiag(None, None if clean is None else clean.data_ptr(), None, None, None)
+        if ev_arr is not None:
+            dstruct.h_stage_events = C.cast(ev_arr, C.POINTER(C.c_void_p))
+    with torch.cuda.device(dev):
+        check(L.r3dfs_mpti_support(
+            C.byref(cfg), C.byref(pw.struct), S,
+            _p(support_x), support_x.stride(0), support_x.stride(2), support_x.stride(3),
+            support_x.stride(4), _p(support_y), _p(proto), _p(count),
+            C.byref(dstruct) if dstruct is not None else None, _p(ws), ws.numel(), _stream()),
+            "r3dfs_mpti_support")
+    return proto, count, clean
+
+
+def _mpti_query_raw(pw: PackedWeights, cfg: EpisodeCfg, proto: torch.Tensor,
+                    proto_count: torch.Tensor, query_x: torch.Tensor,
+                    query_y: Optional[torch.Tensor] = None, shared: bool = False,
+                    want_diag: bool = False, workspace: Optional[torch.Tensor] = None,
+                    stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
+    """The query half of E episodes in one call (r3dfs_mpti_query) against the prototypes of
+    `mpti_support`.  proto (S, n_way+1, n_subprototypes+1, 192), proto_count (S, n_way+1):
+    S == E (episode i uses set i), or S == 1 with shared=True (every episode uses set 0, read in
+    place).  query_x (E, n_query, C, N) any strides, query_y (E, n_query, N) or None.
+    Returns dict(logits (E, n_query, N, n_way+1), loss (E), pred (E, n_query, N) int32 [, diag
+    (proto_count, cg_iters, cg_resid)])."""
+    dev = _need_cuda(proto, proto_count, query_x, query_y)
+    query_x = _f32(query_x)
+    E, nq, Cin, N = query_x.shape
+    nc, slot = cfg.n_way + 1, cfg.n_subprototypes + 1
+    if (nq, N) != (cfg.n_query, cfg.n_points):
+        raise ValueError("query tensors do not match the episode configuration")
+    proto = _f32(proto).contiguous()
+    proto_count = proto_count.to(torch.int32).contiguous()
+    S = proto.shape[0]
+    if tuple(proto.shape[1:]) != (nc, slot, 192) or tuple(proto_count.shape) != (S, nc):
+        raise ValueError("prototypes do not match the episode configuration")
+    if S != (1 if shared else E):
+        raise ValueError(f"{S} prototype sets for {E} episodes (shared={shared})")
+    p_e, c_e = (0, 0) if shared else (nc * slot * 192, nc)
+    if query_y is not None:
+        query_y = query_y.to(torch.int64).contiguous()
+    logits = torch.empty((E, nq, N, nc), dtype=torch.float32, device=dev)
+    loss = torch.zeros((E,), dtype=torch.float32, device=dev)
+    pred = torch.empty((E, nq, N), dtype=torch.int32, device=dev)
+    L = _lib.lib()
+    need = L.r3dfs_mpti_query_workspace(C.byref(cfg), E)
+    if need == 0:
+        raise _envelope_error(cfg)
+    ws = workspace if workspace is not None and workspace.numel() >= need else _ws(need, dev)
+    ev_arr = _stage_event_array(stage_events)
+    diag = dstruct = None
+    if want_diag or ev_arr is not None:
+        dstruct = EpisodeDiag(None, None, None, None, None)
+    if want_diag:
+        diag = {"proto_count": torch.zeros((E, nc), dtype=torch.int32, device=dev),
+                "cg_iters": torch.zeros((E,), dtype=torch.int32, device=dev),
+                "cg_resid": torch.zeros((E,), dtype=torch.float32, device=dev)}
+        dstruct.proto_count = diag["proto_count"].data_ptr()
+        dstruct.cg_iters = diag["cg_iters"].data_ptr()
+        dstruct.cg_resid = diag["cg_resid"].data_ptr()
+    if ev_arr is not None:
+        dstruct.h_stage_events = C.cast(ev_arr, C.POINTER(C.c_void_p))
+    with torch.cuda.device(dev):
+        check(L.r3dfs_mpti_query(
+            C.byref(cfg), C.byref(pw.struct), E, _p(proto), p_e, _p(proto_count), c_e,
+            _p(query_x), query_x.stride(0), query_x.stride(1), query_x.stride(2), query_x.stride(3),
+            _p(query_y), _p(logits), _p(loss), _p(pred),
+            C.byref(dstruct) if dstruct is not None else None, _p(ws), ws.numel(), _stream()),
+            "r3dfs_mpti_query")
+    out = {"logits": logits, "loss": loss, "pred": pred}
+    if diag is not None:
+        out["diag"] = diag
+    return out
 
 
 def confusion_accumulate(pred: torch.Tensor, gt: torch.Tensor, class_slot: torch.Tensor,
@@ -745,6 +849,56 @@ def _(weights, in_dim, dgcnn_k, support_x, support_y, query_x, query_y, n_subpro
             f((E, n_way, k_shot)), f((E,), **i32), f((E,)))
 
 
+@torch.library.custom_op("r3dfs::mpti_support", mutates_args=(), device_types="cuda")
+def _mpti_support_op(weights: Sequence[torch.Tensor], in_dim: int, dgcnn_k: int,
+                     support_x: torch.Tensor, support_y: torch.Tensor, n_query: int,
+                     n_subprototypes: int, k_connect: int, mdns: bool
+                     ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Support half of S episodes (reference models/mpti.py:433-435, 440-493, eval) as ONE op:
+    -> (proto (S, n_way+1, n_subprototypes+1, 192), proto_count (S, n_way+1) int32,
+    clean_flag (S, n_way, k_shot)).  n_query / k_connect only enter the envelope check."""
+    S, n_way, k_shot, _, N = support_x.shape
+    cfg = make_cfg(n_way, k_shot, n_query, N, n_subprototypes, k_connect, mdns=mdns)
+    return _mpti_support_raw(_WeightsView(weights, in_dim, dgcnn_k), cfg, support_x, support_y,
+                             want_diag=True)
+
+
+@_mpti_support_op.register_fake
+def _(weights, in_dim, dgcnn_k, support_x, support_y, n_query, n_subprototypes, k_connect, mdns):
+    S, n_way, k_shot, _, N = support_x.shape
+    f = support_x.new_empty
+    return (f((S, n_way + 1, n_subprototypes + 1, 192)), f((S, n_way + 1), dtype=torch.int32),
+            f((S, n_way, k_shot)))
+
+
+@torch.library.custom_op("r3dfs::mpti_query", mutates_args=("workspace",), device_types="cuda")
+def _mpti_query_op(weights: Sequence[torch.Tensor], in_dim: int, dgcnn_k: int, proto: torch.Tensor,
+                   proto_count: torch.Tensor, query_x: torch.Tensor,
+                   query_y: Optional[torch.Tensor], shared: bool, k_shot: int, k_connect: int,
+                   sigma: float, alpha: float, cg_max_iter: int, cg_tol: float,
+                   workspace: Optional[torch.Tensor]
+                   ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Query half of E episodes (reference models/mpti.py:436-437, 495-571, eval) against given
+    prototypes as ONE op: -> (logits (E, n_query, N, n_way+1), loss (E), pred (E, n_query, N)
+    int32, cg_iters (E) int32, cg_resid (E)).  n_way and n_subprototypes come from proto's shape;
+    k_shot (of the support set) only appears in error messages, the query half does not use it."""
+    E, nq, _, N = query_x.shape
+    n_way, n_sub = proto.shape[1] - 1, proto.shape[2] - 1
+    cfg = make_cfg(n_way, k_shot, nq, N, n_sub, k_connect, sigma, alpha, False, cg_max_iter, cg_tol)
+    out = _mpti_query_raw(_WeightsView(weights, in_dim, dgcnn_k), cfg, proto, proto_count, query_x,
+                          query_y, shared, want_diag=True, workspace=workspace)
+    d = out["diag"]
+    return out["logits"], out["loss"], out["pred"], d["cg_iters"], d["cg_resid"]
+
+
+@_mpti_query_op.register_fake
+def _(weights, in_dim, dgcnn_k, proto, proto_count, query_x, query_y, shared, k_shot, k_connect,
+      sigma, alpha, cg_max_iter, cg_tol, workspace):
+    E, nq, _, N = query_x.shape
+    f, i32 = query_x.new_empty, dict(dtype=torch.int32)
+    return (f((E, nq, N, proto.shape[1])), f((E,)), f((E, nq, N), **i32), f((E,), **i32), f((E,)))
+
+
 # the registered ops, for module code (traceable by torch.compile / fake tensors)
 op = torch.ops.r3dfs
 
@@ -766,4 +920,37 @@ def mpti_forward(pw: Optional[PackedWeights], cfg: EpisodeCfg, support_x: torch.
     out = {"logits": r[0], "loss": r[1], "pred": r[2]}
     if want_diag:
         out["diag"] = {"proto_count": r[3], "clean_flag": r[4], "cg_iters": r[5], "cg_resid": r[6]}
+    return out
+
+
+def mpti_support(pw: PackedWeights, cfg: EpisodeCfg, support_x: torch.Tensor,
+                 support_y: torch.Tensor, want_diag: bool = False,
+                 stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
+    """Support half of S episodes, encoded once (see _mpti_support_raw): -> (proto, proto_count,
+    clean_flag or None).  The plain case goes through the registered op `r3dfs::mpti_support`."""
+    if stage_events is not None:
+        return _mpti_support_raw(pw, cfg, support_x, support_y, want_diag, stage_events)
+    proto, count, clean = op.mpti_support(pw.tensors, pw.struct.in_dim, pw.struct.dgcnn_k,
+                                          support_x, support_y, cfg.n_query, cfg.n_subprototypes,
+                                          cfg.k_connect, bool(cfg.mdns))
+    return proto, count, clean if want_diag else None
+
+
+def mpti_query(pw: PackedWeights, cfg: EpisodeCfg, proto: torch.Tensor, proto_count: torch.Tensor,
+               query_x: torch.Tensor, query_y: Optional[torch.Tensor] = None, shared: bool = False,
+               want_diag: bool = False, workspace: Optional[torch.Tensor] = None,
+               stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
+    """Query half of E episodes against given prototypes (see _mpti_query_raw); returns the dict
+    of `mpti_forward`.  The plain case goes through the registered op `r3dfs::mpti_query`."""
+    if stage_events is not None:
+        return _mpti_query_raw(pw, cfg, proto, proto_count, query_x, query_y, shared, want_diag,
+                               workspace, stage_events)
+    if (proto.shape[1], proto.shape[2]) != (cfg.n_way + 1, cfg.n_subprototypes + 1):
+        raise ValueError("prototypes do not match the episode configuration")
+    r = op.mpti_query(pw.tensors, pw.struct.in_dim, pw.struct.dgcnn_k, proto, proto_count, query_x,
+                      query_y, bool(shared), cfg.k_shot, cfg.k_connect, cfg.sigma, cfg.alpha,
+                      cfg.cg_max_iter, cfg.cg_tol, workspace)
+    out = {"logits": r[0], "loss": r[1], "pred": r[2]}
+    if want_diag:
+        out["diag"] = {"cg_iters": r[3], "cg_resid": r[4]}
     return out
