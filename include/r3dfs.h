@@ -365,6 +365,65 @@ int r3dfs_mpti_query(const r3dfs_episode_cfg_t* h_cfg, const r3dfs_weights_t* h_
                      const r3dfs_episode_diag_t* h_diag, void* ws, size_t ws_bytes,
                      r3dfs_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Segmenting a whole scan against one support set
+ * ---------------------------------------------------------------------------------------- */
+
+/* A scan of M points is cut into overlapping xy blocks, every block into chunks of N = n_points
+ * points laid out as the reference's loader lays out a block (dataloaders/loader.py:201-219); the
+ * chunks are segmented as 1-query episodes (r3dfs_mpti_query, n_query = 1, p_e = 0) and the chunk
+ * logits are merged back onto the points.  Three calls share one workspace, which must not be
+ * touched between them: plan -> chunks -> (query) -> merge.
+ *
+ *   points: (M, 6) fp32 by element strides (s_m, s_c): x y z in metres (any origin), r g b in
+ *           0..255 (the S3DIS / ScanNet .npy convention).
+ * Every operation below is an fp32 operation rounded to nearest, written out (no contraction).
+ *
+ * Grid.  Blocks are xy columns over the full height.  r = overlap (1..4), stride = block_size / r,
+ *   x0 = min x, ext_x = max x - x0; n_cells_x = max(1, floor(ext_x / stride + 0.5)) (the last cell
+ *   absorbs a remainder under half a stride); a point's cell u = min(floor((x - x0) / stride),
+ *   n_cells_x - 1); n_bx = max(1, n_cells_x - r + 1); the point lies in every block
+ *   ix in [max(0, u - r + 1), min(u, n_bx - 1)], the same in y; block id b = ix * n_by + iy.
+ *   Every point lies in 1 to r^2 blocks.
+ * Chunks.  Empty blocks make none; a block of n_b members makes C_b = ceil(n_b / N).  Members are
+ *   ranked by k(i) = lowbias32(i ^ lowbias32(seed)) (i = point index; lowbias32(x): x ^= x >> 16;
+ *   x *= 0x7feb352d; x ^= x >> 15; x *= 0x846ca68b; x ^= x >> 16 on uint32, a bijection: no ties).
+ *   Rank rho goes to chunk rho mod C_b, slot rho div C_b, so every chunk is a uniform sample of the
+ *   block.  Chunk j has count_j = ceil((n_b - j) / C_b) members; slot s >= count_j repeats slot
+ *   s mod count_j (the loader's sampling with replacement of a small block).  Chunks are numbered
+ *   by ascending block id, then j.
+ * Chunk cloud (N, 9) point-major, over the chunk's own points: m = min xyz, xyz' = xyz - m,
+ *   e = max xyz', XYZ = e > 0 ? xyz' / e : 0 per axis (the reference divides 0 by 0 on a flat axis),
+ *   rgb' = rgb / 255; channels xyz' | rgb' | XYZ.
+ * Merge.  A point's logits = the sum, in ascending block id, of the logits row at its own slot of
+ *   each block that holds it (repeats excluded), sequential fp32 adds from 0, divided once by the
+ *   number of contributions; pred = argmax (first maximum, as the episode head); coverage = the
+ *   number of contributions (1..r^2).
+ *
+ * Limits: r^2 * M < 2^31, 64 <= N <= 65536 (R3DFS_E_UNSUPPORTED).  The chunks go through
+ * r3dfs_mpti_query in batches of at most 65535 (its E * n_query limit). */
+size_t r3dfs_scene_workspace(int64_t M, int overlap); /* 0 outside the limits; host only */
+
+/* Builds the grid, the memberships and the chunk layout in the workspace and writes the number of
+ * chunks to the DEVICE int64 *n_chunks: -1 when an x or y coordinate is not finite or the grid has
+ * 2^31 blocks or more.  block_size > 0 and finite.  Reading n_chunks back is the one host
+ * synchronisation a scene needs. */
+int r3dfs_scene_plan(const float* points, int64_t M, int64_t s_m, int64_t s_c, float block_size,
+                     int overlap, uint32_t seed, int n_points, int64_t* n_chunks, void* ws,
+                     size_t ws_bytes, r3dfs_stream_t stream);
+
+/* chunk_x: (n_chunks, N, 9) point-major chunk clouds; chunk_src: (n_chunks, N) int32, the point of
+ * every slot.  n_chunks (host) = the value plan wrote; chunks past it are written as 0 / -1. */
+int r3dfs_scene_chunks(const float* points, int64_t M, int64_t s_m, int64_t s_c, int overlap,
+                       int n_points, int64_t n_chunks, float* chunk_x, int32_t* chunk_src,
+                       void* ws, size_t ws_bytes, r3dfs_stream_t stream);
+
+/* logits: (n_chunks, N, n_cls) fp32 (r3dfs_mpti_query's logits of the chunks in order), n_cls <= 8.
+ * point_logits: (M, n_cls) fp32; point_pred (M) int32 and coverage (M) int32 may be NULL. */
+int r3dfs_scene_merge(const float* logits, int64_t M, int overlap, int n_points, int64_t n_chunks,
+                      int n_cls, float* point_logits, int32_t* point_pred, int32_t* coverage,
+                      void* ws, size_t ws_bytes, r3dfs_stream_t stream);
+
 /* ProtoNet + MDNS (reference models/protonet.py:357-945 ProtoNet_Contrast.forward, train=False):
  * same encoder and noise suppression as MPTI, then masked average pooling of the support
  * features (:878-890), one prototype per way from the kept shots + one background prototype

@@ -78,6 +78,57 @@ def make_cloud(rng: np.random.Generator, objects: List[int], n_pts: int = N_POIN
     return pts, cls
 
 
+def make_scene(seed: int, size_xy=(6.0, 4.0), points_per_m2: float = 10000.0,
+               classes: Optional[List[int]] = None, dataset: str = "s3dis"):
+    """A synthetic room scan in the style of `make_cloud`: floor, four walls, uniform clutter and
+    Gaussian blobs of the given classes (default: two per class of the dataset's pool), with
+    x y z in metres from an arbitrary origin and r g b in 0..255 (the S3DIS / ScanNet .npy
+    convention).  Returns (points (M, 6) float32, cls (M,) int64 with -1 = background), in a random
+    point order; M = round(points_per_m2 * area)."""
+    rng = np.random.default_rng(seed)
+    sx, sy = float(size_xy[0]), float(size_xy[1])
+    M = int(round(points_per_m2 * sx * sy))
+    if classes is None:
+        classes = list(range(CLASS_POOL[dataset])) * 2
+    n_obj = int(0.25 * M) // max(1, len(classes)) if classes else 0
+    n_floor = int(0.4 * M)
+    n_wall = int(0.2 * M)
+    n_clut = M - n_floor - n_wall - n_obj * len(classes)
+    xyz, rgb, cls = [], [], []
+    xyz.append(np.stack([rng.uniform(0, sx, n_floor), rng.uniform(0, sy, n_floor),
+                         np.abs(rng.normal(0, 0.01, n_floor))], 1))
+    rgb.append(np.tile([0.55, 0.5, 0.45], (n_floor, 1)))
+    # walls: a point on the perimeter, pushed a little into the room
+    t = rng.uniform(0, 2 * (sx + sy), n_wall)
+    d = np.abs(rng.normal(0, 0.01, n_wall))
+    wx = np.where(t < sx, t, np.where(t < sx + sy, sx - d, np.where(t < 2 * sx + sy,
+                                                                    2 * sx + sy - t, d)))
+    wy = np.where(t < sx, d, np.where(t < sx + sy, t - sx, np.where(t < 2 * sx + sy, sy - d,
+                                                                    2 * (sx + sy) - t)))
+    xyz.append(np.stack([wx, wy, rng.uniform(0, 3, n_wall)], 1))
+    rgb.append(np.tile([0.8, 0.8, 0.75], (n_wall, 1)))
+    xyz.append(np.stack([rng.uniform(0, sx, n_clut), rng.uniform(0, sy, n_clut),
+                         rng.uniform(0, 3, n_clut)], 1))
+    rgb.append(rng.uniform(0.2, 0.8, size=(n_clut, 3)))
+    cls.append(np.full(n_floor + n_wall + n_clut, -1, np.int64))
+    for c in classes:
+        col, sig, h = _class_style(c)
+        ctr = np.array([rng.uniform(0.5, sx - 0.5), rng.uniform(0.5, sy - 0.5), h])
+        p = ctr + rng.normal(0, 1, size=(n_obj, 3)) * sig
+        p[:, 0] = np.clip(p[:, 0], 0, sx)
+        p[:, 1] = np.clip(p[:, 1], 0, sy)
+        p[:, 2] = np.clip(p[:, 2], 0, 3)
+        xyz.append(p)
+        rgb.append(np.tile(col, (n_obj, 1)))
+        cls.append(np.full(n_obj, int(c), np.int64))
+    xyz = np.concatenate(xyz, 0) + rng.uniform(-50, 50, size=3)   # arbitrary origin
+    rgb = np.clip(np.concatenate(rgb, 0) + rng.normal(0, 0.05, size=(M, 3)), 0, 1) * 255.0
+    cls = np.concatenate(cls, 0)
+    perm = rng.permutation(M)
+    pts = np.concatenate([xyz, rgb], 1)[perm].astype(np.float32)
+    return pts, cls[perm]
+
+
 @dataclasses.dataclass
 class Episode:
     """Host-side episode, laid out like the reference's collate output

@@ -240,6 +240,67 @@ class MPTI_SelfAtten(nn.Module):
             return r[0][0].transpose(1, 2), r[1][0]
         return {"logits": r[0], "loss": r[1], "pred": r[2]}
 
+    def segment_scene(self, support: SupportSet, points, block_size=1.0, overlap=1, seed=0,
+                      chunk_batch=64):
+        """Labels every point of a whole scan against one encoded support set.
+        points: (M, 6) CUDA tensor, x y z in metres (any origin) and r g b in 0..255, the S3DIS /
+        ScanNet .npy convention.  The scan is cut into xy blocks of block_size metres that overlap
+        `overlap`-fold per axis (1..4), every block into chunks of n_points points normalised as the
+        reference's loader normalises a block, the chunks are segmented `chunk_batch` at a time as
+        1-query episodes against `support` (r3dfs_mpti_query), and each point's logits are averaged
+        over the blocks that hold it.  `seed` picks which points share a chunk.  The contract,
+        exact to the bit, is in include/r3dfs.h ("Segmenting a whole scan").
+        Returns dict(logits (M, n_way+1), pred (M,) int32, coverage (M,) int32 = blocks holding the
+        point, n_chunks).  Eager only: the chunk count depends on the data and is read back once.
+        Results are reproducible for a given chunk_batch; another chunk_batch can change the
+        logits in the last bits, as the query kernels round differently at another batch size."""
+        if self.training:
+            raise NotImplementedError("r3dfsseg_b200: stand-alone call in training mode; use "
+                                      "forward(..., train=True) for the training step or .eval()")
+        if (support.n_way, support.n_points, support.n_subprototypes) != \
+                (self.n_way, self.n_points, self.n_subprototypes):
+            raise ValueError(
+                f"support set built for n_way={support.n_way} n_points={support.n_points} "
+                f"n_subprototypes={support.n_subprototypes}; the model has n_way={self.n_way} "
+                f"n_points={self.n_points} n_subprototypes={self.n_subprototypes}")
+        if support.n_sets != 1:
+            raise ValueError(f"a scene is segmented against one support set; got {support.n_sets}")
+        if not isinstance(points, torch.Tensor) or not points.is_cuda:
+            raise ValueError("points must be a CUDA tensor")
+        if points.dim() != 2 or points.shape[1] != 6 or points.shape[0] == 0:
+            raise ValueError(f"points must be (M, 6) with M > 0; got {tuple(points.shape)}")
+        if int(overlap) != overlap or not 1 <= overlap <= 4:
+            raise ValueError(f"overlap must be an integer in 1..4; got {overlap}")
+        if not float(block_size) > 0.0 or float(block_size) == float("inf"):
+            raise ValueError(f"block_size must be a positive number of metres; got {block_size}")
+        if int(seed) != seed or not 0 <= seed < 2 ** 32:
+            raise ValueError(f"seed must be a uint32; got {seed}")
+        if int(chunk_batch) < 1 or chunk_batch > 65535:
+            raise ValueError(f"chunk_batch must be in 1..65535; got {chunk_batch}")
+        pw = self._weights()
+        if self._packed_sig != support.weights_sig:
+            raise RuntimeError("the weights or BatchNorm statistics changed after the support set "
+                               "was encoded: its prototypes are stale, call encode_support again")
+        N, nc = self.n_points, self.n_classes
+        plan = ops.scene_plan(points, N, float(block_size), int(overlap), int(seed))
+        E = int(plan.n_chunks.item())
+        if E < 0:
+            raise ValueError("points hold a non-finite x or y coordinate, or the scan spans 2^31 "
+                             "blocks or more")
+        chunk_x, _ = ops.scene_chunks(plan, E)
+        query_x = chunk_x.view(E, 1, N, 9).transpose(2, 3)   # (E, 1, 9, N), point-major memory
+        logits = torch.empty((E, N, nc), dtype=torch.float32, device=points.device)
+        B = int(chunk_batch)
+        for b0 in range(0, E, B):
+            r = ops.op.mpti_query(pw.tensors, self.in_channels, int(self.encoder.k),
+                                  support.prototypes, support.proto_count, query_x[b0:b0 + B], None,
+                                  True, support.k_shot, self.k_connect, float(self.sigma),
+                                  self.lp_alpha, self.cg_max_iter, self.cg_tol, None)
+            logits[b0:b0 + B] = r[0][:, 0]
+        out = ops.scene_merge(plan, logits, E)
+        out["n_chunks"] = E
+        return out
+
     def forward(self, support_x, support_y, query_x, query_y, gt_support_y=None, gt_query_y=None,
                 train=False, logger=None, step=None, path=None, sampled_classes=None,
                 bg_pcd_x=None, bg_pcd_y=None, support_c=None, support_flag=None, pcd_1024=None,

@@ -8,6 +8,7 @@ as torch custom ops in the `r3dfs::` namespace (CUDA implementation only).
 from __future__ import annotations
 
 import ctypes as C
+from dataclasses import dataclass
 from typing import List, Optional, Sequence, Tuple
 
 import torch
@@ -628,6 +629,81 @@ def _mpti_query_raw(pw: PackedWeights, cfg: EpisodeCfg, proto: torch.Tensor,
     out = {"logits": logits, "loss": loss, "pred": pred}
     if diag is not None:
         out["diag"] = diag
+    return out
+
+
+# ------------------------------------------------------------------------------------------------
+# whole scans (r3dfs_scene_*: blocks -> chunks of n_points -> query episodes -> merge)
+# ------------------------------------------------------------------------------------------------
+@dataclass
+class ScenePlan:
+    """One scan planned by r3dfs_scene_plan: the workspace holding its chunk layout (read by
+    `scene_chunks` and `scene_merge`, which must get the same points), and the chunk count as a
+    (1,) int64 device tensor (-1: an x or y coordinate is not finite, or the grid is too large)."""
+    points: torch.Tensor
+    workspace: torch.Tensor
+    n_chunks: torch.Tensor
+    overlap: int
+    n_points: int
+
+
+def scene_plan(points: torch.Tensor, n_points: int, block_size: float = 1.0, overlap: int = 1,
+               seed: int = 0) -> ScenePlan:
+    """Grid, block memberships and chunk layout of an (M, 6) scan (x y z in metres, r g b in
+    0..255; any strides) for chunks of n_points points.  Enqueued only: nothing is read back."""
+    dev = _need_cuda(points)
+    points = _f32(points)
+    if points.dim() != 2 or points.shape[1] != 6:
+        raise ValueError(f"points must be (M, 6) = x y z r g b; got {tuple(points.shape)}")
+    M = int(points.shape[0])
+    L = _lib.lib()
+    need = L.r3dfs_scene_workspace(M, int(overlap))
+    if need == 0:
+        raise _lib.R3dfsError(f"scene of {M} points at overlap {overlap} is outside what libr3dfs "
+                              "is built for: overlap 1..4 and overlap^2 * M < 2^31")
+    ws = _ws(need, dev)
+    n_chunks = torch.empty((1,), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        check(L.r3dfs_scene_plan(_p(points), M, points.stride(0), points.stride(1),
+                                 float(block_size), int(overlap), int(seed), int(n_points),
+                                 _p(n_chunks), _p(ws), ws.numel(), _stream()), "r3dfs_scene_plan")
+    return ScenePlan(points, ws, n_chunks, int(overlap), int(n_points))
+
+
+def scene_chunks(plan: ScenePlan, n_chunks: int):
+    """-> chunk_x (n_chunks, N, 9) point-major chunk clouds, chunk_src (n_chunks, N) int32 (the
+    scan point of every slot).  n_chunks = the plan's count, read back by the caller."""
+    pts = plan.points
+    N = plan.n_points
+    chunk_x = torch.empty((n_chunks, N, 9), dtype=torch.float32, device=pts.device)
+    chunk_src = torch.empty((n_chunks, N), dtype=torch.int32, device=pts.device)
+    L = _lib.lib()
+    with torch.cuda.device(pts.device):
+        check(L.r3dfs_scene_chunks(_p(pts), pts.shape[0], pts.stride(0), pts.stride(1),
+                                   plan.overlap, N, int(n_chunks), _p(chunk_x), _p(chunk_src),
+                                   _p(plan.workspace), plan.workspace.numel(), _stream()),
+              "r3dfs_scene_chunks")
+    return chunk_x, chunk_src
+
+
+def scene_merge(plan: ScenePlan, logits: torch.Tensor, n_chunks: int):
+    """Chunk logits (n_chunks, N, n_cls) -> dict(logits (M, n_cls) = mean over the blocks holding
+    each point, pred (M,) int32, coverage (M,) int32 = number of those blocks)."""
+    dev = _need_cuda(logits)
+    logits = _f32(logits).contiguous()
+    if tuple(logits.shape[:2]) != (n_chunks, plan.n_points) or logits.dim() != 3:
+        raise ValueError(f"expected chunk logits ({n_chunks}, {plan.n_points}, n_cls); got "
+                         f"{tuple(logits.shape)}")
+    M, nc = int(plan.points.shape[0]), int(logits.shape[2])
+    out = {"logits": torch.empty((M, nc), dtype=torch.float32, device=dev),
+           "pred": torch.empty((M,), dtype=torch.int32, device=dev),
+           "coverage": torch.empty((M,), dtype=torch.int32, device=dev)}
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        check(L.r3dfs_scene_merge(_p(logits), M, plan.overlap, plan.n_points, int(n_chunks), nc,
+                                  _p(out["logits"]), _p(out["pred"]), _p(out["coverage"]),
+                                  _p(plan.workspace), plan.workspace.numel(), _stream()),
+              "r3dfs_scene_merge")
     return out
 
 
