@@ -424,6 +424,40 @@ int r3dfs_scene_merge(const float* logits, int64_t M, int overlap, int n_points,
                       int n_cls, float* point_logits, int32_t* point_pred, int32_t* coverage,
                       void* ws, size_t ws_bytes, r3dfs_stream_t stream);
 
+/* Support shots from a labelled scan (the reference's class2scans index, dataloaders/s3dis.py /
+ * scannet.py, and sample_pointcloud(..., support=True), dataloaders/loader.py:201-219), on a scan
+ * planned by r3dfs_scene_plan with the same points, block_size, overlap, seed and N = n_points.
+ *   labels: (M) int32 class of every point; h_classes: HOST array of n_way distinct class ids.
+ * Counts.  For every non-empty block b with n_b members, count_w(b) = members i with
+ *   labels[i] == classes[w].
+ * Eligibility.  b is eligible for way w iff count_w(b) > max(floor(n_b * min_ratio), min_points),
+ *   the product in fp64 (as Python's int(n_b * 0.05)); the reference uses min_points = 100,
+ *   min_ratio = 0.05.  n_eligible[w] = the number of eligible blocks.
+ * Choice.  Way w ranks its eligible blocks by lowbias32(b ^ lowbias32(lowbias32(seed) + w + 1))
+ *   (uint32, wrapping): a bijection of the block id, different for every way.  Its shots are the
+ *   k_shot eligible blocks with the smallest keys, in ascending key order; a block may serve
+ *   several ways.  shot_block (n_way, k_shot) int32 = the block id of every shot.
+ * Shot cloud.  The block's members in the plan's rank order k(i); slot s holds rank
+ *   s mod min(n_b, N): for n_b >= N the N lowest-ranked members, each once (the reference's
+ *   sampling without replacement), for a smaller block its members repeated.  For n_b <= N it is
+ *   the block's single chunk of r3dfs_scene_chunks.  Normalised as a chunk cloud.
+ *   support_x: (n_way, k_shot, N, 9) point-major; support_src (n_way, k_shot, N) int32 = the point
+ *   of every slot; support_y (n_way, k_shot, N) int32 = labels[src] == classes[w].
+ * Missing shots (n_eligible[w] < k_shot) are a zero cloud with src -1, block -1 and mask 0.  When
+ *   the plan reported a grid error (n_chunks = -1), every n_eligible is -1.
+ * The plan workspace is only read: chunks and merge on it return what they returned before.
+ * Deterministic, no atomics, no host synchronisation.  ws: r3dfs_scene_support_workspace bytes
+ * (under 1 MB, independent of M).  1 <= n_way <= 7 and 1 <= k_shot <= 32 (else
+ * R3DFS_E_UNSUPPORTED); duplicate classes, min_points < 0, or min_ratio outside [0, 1] or not
+ * finite give R3DFS_E_BADARG.  Every check happens before anything is launched. */
+size_t r3dfs_scene_support_workspace(int n_way, int k_shot); /* 0 outside the limits; host only */
+int r3dfs_scene_support(const float* points, int64_t M, int64_t s_m, int64_t s_c,
+                        const int32_t* labels, const int32_t* h_classes, int n_way, int k_shot,
+                        int min_points, double min_ratio, uint32_t seed, int overlap, int n_points,
+                        float* support_x, int32_t* support_y, int32_t* support_src,
+                        int32_t* shot_block, int32_t* n_eligible, const void* plan_ws,
+                        size_t plan_ws_bytes, void* ws, size_t ws_bytes, r3dfs_stream_t stream);
+
 /* ProtoNet + MDNS (reference models/protonet.py:357-945 ProtoNet_Contrast.forward, train=False):
  * same encoder and noise suppression as MPTI, then masked average pooling of the support
  * features (:878-890), one prototype per way from the kept shots + one background prototype

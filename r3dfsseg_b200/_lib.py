@@ -121,6 +121,10 @@ SIGNATURES = {
     "r3dfs_scene_plan": (C.c_int, [vp, i64, i64, i64, f32, i32, C.c_uint32, i32, vp, vp, sz, vp]),
     "r3dfs_scene_chunks": (C.c_int, [vp, i64, i64, i64, i32, i32, i64, vp, vp, vp, sz, vp]),
     "r3dfs_scene_merge": (C.c_int, [vp, i64, i32, i32, i64, i32, vp, vp, vp, vp, sz, vp]),
+    "r3dfs_scene_support_workspace": (sz, [i32, i32]),
+    "r3dfs_scene_support": (C.c_int, [vp, i64, i64, i64, vp, C.POINTER(C.c_int32), i32, i32, i32,
+                                      C.c_double, C.c_uint32, i32, i32, vp, vp, vp, vp, vp, vp, sz,
+                                      vp, sz, vp]),
     "r3dfs_confusion_accumulate": (C.c_int, [vp, vp, vp, i32, i32, i64, i32, vp, vp]),
     "r3dfs_protonet_forward": (C.c_int, [C.POINTER(EpisodeCfg), C.POINTER(Weights), i32,
                                          vp, i64, i64, i64, i64, vp,

@@ -2,7 +2,11 @@
 // overlapping xy blocks, split every block into chunks of n_points sampled points normalised as the
 // reference's loader does, and merge the per-chunk logits back onto the scan's points.
 //
-// r3dfs_scene_plan builds every index the two other calls need and leaves it in the workspace:
+// r3dfs_scene_support ("Support shots from a labelled scan") reads the same plan to cut support
+// shots out of a labelled scan: per-block class counts, a seeded choice of blocks per class, and
+// shot clouds built by the chunk clouds' code.
+//
+// r3dfs_scene_plan builds every index the other calls need and leaves it in the workspace:
 //   bbox -> grid -> per-point membership counts -> scan -> one record (block << 32 | key, position)
 //   per membership -> LSD radix sort -> block segments -> chunk counts -> scan -> (chunk, slot) of
 //   every membership, stored back at its position in point order.
@@ -453,30 +457,16 @@ __global__ void scene_member_kernel(int64_t n, int N, SceneHdr* __restrict__ hp,
 }
 
 // ---- chunk clouds ------------------------------------------------------------------------------
-// One CTA per chunk.  Slot q of chunk j of a block with n_b members in C_b chunks holds the member
-// of rank (q mod count_j) * C_b + j, count_j = ceil((n_b - j) / C_b).
-__global__ __launch_bounds__(256) void scene_chunk_kernel(
-    const float* __restrict__ pts, int64_t s_m, int64_t s_c, int N,
-    const SceneHdr* __restrict__ hp, const int32_t* __restrict__ vals,
-    const int32_t* __restrict__ mem_point, const int32_t* __restrict__ seg_start,
-    const int32_t* __restrict__ chunk_off, const int32_t* __restrict__ chunk_seg,
-    float* __restrict__ chunk_x, int32_t* __restrict__ chunk_src) {
-  const int64_t c = blockIdx.x;
-  float* out = chunk_x + c * N * 9;
-  int32_t* src = chunk_src + c * N;
-  if (c >= hp->n_chunks) {  // more chunks asked for than the plan made
-    for (int q = threadIdx.x; q < N; q += blockDim.x) {
-      src[q] = -1;
-      for (int k = 0; k < 9; ++k) out[(int64_t)q * 9 + k] = 0.f;
-    }
-    return;
-  }
-  const int32_t s = chunk_seg[c], c0 = chunk_off[s], cb = chunk_off[s + 1] - c0;
-  const int32_t j = (int32_t)c - c0, p0 = seg_start[s], nb = seg_start[s + 1] - p0;
-  const int32_t cnt = (nb - j + cb - 1) / cb;
+// A cloud of N slots over `count` members of one block: slot q holds the member of sorted record
+// first + (q mod count) * stride + offset, normalised over those members.  One CTA of 256 threads.
+__device__ __forceinline__ void scene_cloud(const float* __restrict__ pts, int64_t s_m, int64_t s_c,
+                                            int N, const int32_t* __restrict__ vals,
+                                            const int32_t* __restrict__ mem_point, int32_t first,
+                                            int32_t stride, int32_t offset, int32_t count,
+                                            float* __restrict__ out, int32_t* __restrict__ src) {
   float mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
-  for (int q = threadIdx.x; q < cnt; q += blockDim.x) {
-    const int64_t i = mem_point[vals[p0 + (int64_t)q * cb + j]];
+  for (int q = threadIdx.x; q < count; q += blockDim.x) {
+    const int64_t i = mem_point[vals[first + (int64_t)q * stride + offset]];
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
       const float v = pts[i * s_m + k * s_c];
@@ -512,7 +502,7 @@ __global__ __launch_bounds__(256) void scene_chunk_kernel(
   }
   __syncthreads();
   for (int q = threadIdx.x; q < N; q += blockDim.x) {
-    const int32_t i = mem_point[vals[p0 + (int64_t)(q % cnt) * cb + j]];
+    const int32_t i = mem_point[vals[first + (int64_t)(q % count) * stride + offset]];
     const float* pt = pts + (int64_t)i * s_m;
     float* o = out + (int64_t)q * 9;
 #pragma unroll
@@ -524,6 +514,36 @@ __global__ __launch_bounds__(256) void scene_chunk_kernel(
     }
     src[q] = i;
   }
+}
+
+// a cloud with no members: zeros, src -1
+__device__ __forceinline__ void scene_cloud_empty(int N, float* __restrict__ out,
+                                                  int32_t* __restrict__ src) {
+  for (int q = threadIdx.x; q < N; q += blockDim.x) {
+    src[q] = -1;
+    for (int k = 0; k < 9; ++k) out[(int64_t)q * 9 + k] = 0.f;
+  }
+}
+
+// One CTA per chunk.  Slot q of chunk j of a block with n_b members in C_b chunks holds the member
+// of rank (q mod count_j) * C_b + j, count_j = ceil((n_b - j) / C_b).
+__global__ __launch_bounds__(256) void scene_chunk_kernel(
+    const float* __restrict__ pts, int64_t s_m, int64_t s_c, int N,
+    const SceneHdr* __restrict__ hp, const int32_t* __restrict__ vals,
+    const int32_t* __restrict__ mem_point, const int32_t* __restrict__ seg_start,
+    const int32_t* __restrict__ chunk_off, const int32_t* __restrict__ chunk_seg,
+    float* __restrict__ chunk_x, int32_t* __restrict__ chunk_src) {
+  const int64_t c = blockIdx.x;
+  float* out = chunk_x + c * N * 9;
+  int32_t* src = chunk_src + c * N;
+  if (c >= hp->n_chunks) {  // more chunks asked for than the plan made
+    scene_cloud_empty(N, out, src);
+    return;
+  }
+  const int32_t s = chunk_seg[c], c0 = chunk_off[s], cb = chunk_off[s + 1] - c0;
+  const int32_t j = (int32_t)c - c0, p0 = seg_start[s], nb = seg_start[s + 1] - p0;
+  const int32_t cnt = (nb - j + cb - 1) / cb;
+  scene_cloud(pts, s_m, s_c, N, vals, mem_point, p0, cb, j, cnt, out, src);
 }
 
 // ---- merge ---------------------------------------------------------------------------------------
@@ -563,6 +583,190 @@ __global__ void scene_merge_kernel(const float* __restrict__ logits, int64_t M, 
   }
   if (pred) pred[i] = am;
   if (coverage) coverage[i] = cov;
+}
+
+// ---- support shots -----------------------------------------------------------------------------
+// Each way keeps the eligible blocks with the 32 smallest keys (k_shot <= 32) as a sorted list of
+// (key << 32 | segment), one entry per lane; keys are a bijection of the block id, so no two
+// entries of a way are equal.  Empty entries are ~0.  A fixed grid of CTAs keeps one list per way
+// and CTA; one CTA per way merges them.
+constexpr int SUP_CTAS = 128, SUP_T = 256, SUP_WARPS = SUP_T / 32, SUP_U = 8;
+constexpr int MAX_WAY = 7, MAX_SHOT = 32;
+constexpr uint64_t TOP_EMPTY = ~0ull;
+
+struct SupportSel {
+  int32_t cls[MAX_WAY];
+  uint32_t wkey[MAX_WAY];  // lowbias32(lowbias32(seed) + w + 1)
+  int32_t n_way, min_points;
+  double min_ratio;
+};
+
+struct SupportWs {
+  uint64_t* part_top;  // (SUP_CTAS, n_way, 32) per-CTA lists
+  int32_t* part_n;     // (SUP_CTAS, n_way) per-CTA eligible counts
+  int32_t* shot_seg;   // (n_way, k_shot) segment of every shot, -1 = missing
+};
+
+void carve_support(WsBump& ws, int n_way, int k_shot, SupportWs& w) {
+  w.part_top = ws.take<uint64_t>((size_t)SUP_CTAS * n_way * MAX_SHOT);
+  w.part_n = ws.take<int32_t>((size_t)SUP_CTAS * n_way);
+  w.shot_seg = ws.take<int32_t>((size_t)n_way * k_shot);
+}
+
+// v (warp-uniform) into the lane-distributed sorted list
+__device__ __forceinline__ uint64_t top_insert(uint64_t list, uint64_t v) {
+  const int lane = threadIdx.x & 31;
+  const int pos = __popc(__ballot_sync(0xffffffffu, list < v));
+  const uint64_t up = __shfl_up_sync(0xffffffffu, list, 1);
+  return lane < pos ? list : lane == pos ? v : up;
+}
+
+// number of entries of the sorted 32-entry list x below v
+__device__ __forceinline__ int count_below(const uint64_t* x, uint64_t v) {
+  int n = 0;
+#pragma unroll
+  for (int st = 16; st > 0; st >>= 1)
+    if (x[n + st - 1] < v) n += st;
+  return n + (x[n] < v ? 1 : 0);
+}
+
+// out = the 32 smallest of the sorted lists a and b (shared memory; out may be a).  One warp.
+__device__ __forceinline__ void top_merge(uint64_t* a, const uint64_t* b, uint64_t* out) {
+  const int lane = threadIdx.x & 31;
+  const uint64_t va = a[lane], vb = b[lane];
+  const int ra = lane + count_below(b, va), rb = lane + count_below(a, vb);
+  __syncwarp();
+  if (ra < 32) out[ra] = va;
+  if (rb < 32) out[rb] = vb;
+  __syncwarp();
+}
+
+// One warp per block segment: counts its members of every way's class (vals -> mem_point ->
+// labels, each membership read once), tests eligibility and inserts the block into the warp's
+// lists; then the CTA merges its warps' lists.  Segment s goes to CTA s mod SUP_CTAS, so the few
+// segments of a small scan spread over the SMs.
+__global__ __launch_bounds__(SUP_T) void scene_support_count_kernel(
+    const SceneHdr* __restrict__ hp, const uint64_t* __restrict__ keys,
+    const int32_t* __restrict__ vals, const int32_t* __restrict__ mem_point,
+    const int32_t* __restrict__ seg_start, const int32_t* __restrict__ labels, SupportSel sel,
+    uint64_t* __restrict__ part_top, int32_t* __restrict__ part_n) {
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int32_t n_seg = hp->n_seg;
+  uint64_t top[MAX_WAY];
+  int n_el[MAX_WAY];
+#pragma unroll
+  for (int w = 0; w < MAX_WAY; ++w) {
+    top[w] = TOP_EMPTY;
+    n_el[w] = 0;
+  }
+  for (int32_t s = wid * SUP_CTAS + blockIdx.x; s < n_seg; s += SUP_CTAS * SUP_WARPS) {
+    const int32_t p0 = seg_start[s], nb = seg_start[s + 1] - p0;
+    int cnt[MAX_WAY];
+#pragma unroll
+    for (int w = 0; w < MAX_WAY; ++w) cnt[w] = 0;
+    for (int32_t base = 0; base < nb; base += 32 * SUP_U) {
+      int32_t t[SUP_U];
+#pragma unroll
+      for (int u = 0; u < SUP_U; ++u) {
+        const int32_t q = base + u * 32 + lane;
+        t[u] = q < nb ? vals[p0 + q] : -1;
+      }
+#pragma unroll
+      for (int u = 0; u < SUP_U; ++u) t[u] = t[u] >= 0 ? mem_point[t[u]] : -1;
+#pragma unroll
+      for (int u = 0; u < SUP_U; ++u) {
+        if (t[u] < 0) continue;
+        const int32_t l = labels[t[u]];
+#pragma unroll
+        for (int w = 0; w < MAX_WAY; ++w) cnt[w] += (w < sel.n_way && l == sel.cls[w]) ? 1 : 0;
+      }
+    }
+    // max(floor(n_b * min_ratio), min_points), the product in fp64 as Python's int(n_b * 0.05)
+    const double thr = fmax(floor((double)nb * sel.min_ratio), (double)sel.min_points);
+    const uint32_t b = (uint32_t)(keys[p0] >> 32);
+#pragma unroll
+    for (int w = 0; w < MAX_WAY; ++w) {
+      if (w >= sel.n_way) continue;
+      const int c = __reduce_add_sync(0xffffffffu, cnt[w]);
+      if ((double)c > thr) {
+        ++n_el[w];
+        top[w] = top_insert(top[w], ((uint64_t)lowbias32(b ^ sel.wkey[w]) << 32) | (uint32_t)s);
+      }
+    }
+  }
+  __shared__ uint64_t s_top[SUP_WARPS][MAX_WAY][32];
+  __shared__ int s_n[SUP_WARPS][MAX_WAY];
+#pragma unroll
+  for (int w = 0; w < MAX_WAY; ++w) {
+    s_top[wid][w][lane] = top[w];
+    if (lane == 0) s_n[wid][w] = n_el[w];
+  }
+  __syncthreads();
+  if (wid >= sel.n_way) return;
+  const int w = wid;
+  for (int o = 1; o < SUP_WARPS; ++o) top_merge(s_top[0][w], s_top[o][w], s_top[0][w]);
+  const int n = __reduce_add_sync(0xffffffffu, lane < SUP_WARPS ? s_n[lane][w] : 0);
+  part_top[((int64_t)blockIdx.x * sel.n_way + w) * 32 + lane] = s_top[0][w][lane];
+  if (lane == 0) part_n[blockIdx.x * sel.n_way + w] = n;
+}
+
+// One CTA per way: merges the SUP_CTAS lists, keeps the first k_shot entries as the way's shots.
+__global__ __launch_bounds__(SUP_T) void scene_support_pick_kernel(
+    const SceneHdr* __restrict__ hp, const uint64_t* __restrict__ keys,
+    const int32_t* __restrict__ seg_start, const uint64_t* __restrict__ part_top,
+    const int32_t* __restrict__ part_n, int n_way, int k_shot, int32_t* __restrict__ shot_seg,
+    int32_t* __restrict__ shot_block, int32_t* __restrict__ n_eligible) {
+  __shared__ uint64_t s_p[SUP_CTAS][32];
+  __shared__ int s_n[SUP_WARPS];
+  const int w = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  for (int i = threadIdx.x; i < SUP_CTAS * 32; i += SUP_T)
+    s_p[i >> 5][i & 31] = part_top[((int64_t)(i >> 5) * n_way + w) * 32 + (i & 31)];
+  int n = 0;
+  for (int g = threadIdx.x; g < SUP_CTAS; g += SUP_T) n += part_n[g * n_way + w];
+  n = __reduce_add_sync(0xffffffffu, n);
+  if (lane == 0) s_n[wid] = n;
+  __syncthreads();
+  for (int g = wid + SUP_WARPS; g < SUP_CTAS; g += SUP_WARPS) top_merge(s_p[wid], s_p[g], s_p[wid]);
+  __syncthreads();
+  if (wid != 0) return;
+  for (int o = 1; o < SUP_WARPS; ++o) top_merge(s_p[0], s_p[o], s_p[0]);
+  const bool err = hp->err != 0;
+  if (lane < k_shot) {
+    const uint64_t v = s_p[0][lane];
+    const int32_t s = err || v == TOP_EMPTY ? -1 : (int32_t)(uint32_t)v;
+    shot_seg[w * k_shot + lane] = s;
+    shot_block[w * k_shot + lane] = s < 0 ? -1 : (int32_t)(keys[seg_start[s]] >> 32);
+  }
+  if (lane == 0) {
+    int tot = 0;
+    for (int i = 0; i < SUP_WARPS; ++i) tot += s_n[i];
+    n_eligible[w] = err ? -1 : tot;
+  }
+}
+
+// One CTA per shot: the block's first min(n_b, N) members in rank order, repeated to N slots, by
+// the chunk clouds' code; mask = label == the way's class.
+__global__ __launch_bounds__(256) void scene_support_cloud_kernel(
+    const float* __restrict__ pts, int64_t s_m, int64_t s_c, int N,
+    const int32_t* __restrict__ labels, const __grid_constant__ SupportSel sel, int k_shot,
+    const int32_t* __restrict__ vals, const int32_t* __restrict__ mem_point,
+    const int32_t* __restrict__ seg_start, const int32_t* __restrict__ shot_seg,
+    float* __restrict__ support_x, int32_t* __restrict__ support_y,
+    int32_t* __restrict__ support_src) {
+  const int64_t g = blockIdx.x;
+  float* out = support_x + g * N * 9;
+  int32_t* src = support_src + g * N;
+  int32_t* y = support_y + g * N;
+  const int32_t s = shot_seg[g];
+  if (s < 0) {
+    scene_cloud_empty(N, out, src);
+    for (int q = threadIdx.x; q < N; q += blockDim.x) y[q] = 0;
+    return;
+  }
+  const int32_t p0 = seg_start[s], nb = seg_start[s + 1] - p0;
+  scene_cloud(pts, s_m, s_c, N, vals, mem_point, p0, 1, 0, min(nb, N), out, src);
+  const int32_t cls = sel.cls[g / k_shot];
+  for (int q = threadIdx.x; q < N; q += blockDim.x) y[q] = labels[src[q]] == cls ? 1 : 0;
 }
 
 int scene_common_checks(int64_t M, int overlap, int n_points) {
@@ -660,6 +864,60 @@ int r3dfs_scene_merge(const float* logits, int64_t M, int overlap, int n_points,
   scene_merge_kernel<<<nblk(M), 256, 0, st>>>(logits, M, n_points, n_cls, n_chunks, w.off,
                                                w.mem_chunk, w.mem_slot, point_logits, point_pred,
                                                coverage);
+  R3DFS_CHECK_LAUNCH();
+  return 0;
+}
+
+size_t r3dfs_scene_support_workspace(int n_way, int k_shot) {
+  if (n_way < 1 || n_way > MAX_WAY || k_shot < 1 || k_shot > MAX_SHOT) return 0;
+  WsBump ws(nullptr, 0);
+  SupportWs w;
+  carve_support(ws, n_way, k_shot, w);
+  return align_up(ws.off, 256);
+}
+
+int r3dfs_scene_support(const float* points, int64_t M, int64_t s_m, int64_t s_c,
+                        const int32_t* labels, const int32_t* h_classes, int n_way, int k_shot,
+                        int min_points, double min_ratio, uint32_t seed, int overlap, int n_points,
+                        float* support_x, int32_t* support_y, int32_t* support_src,
+                        int32_t* shot_block, int32_t* n_eligible, const void* plan_ws,
+                        size_t plan_ws_bytes, void* wsp, size_t ws_bytes, r3dfs_stream_t stream) {
+  if (!points || !labels || !h_classes || !support_x || !support_y || !support_src ||
+      !shot_block || !n_eligible || !plan_ws || !wsp)
+    return R3DFS_E_BADARG;
+  R3DFS_TRY(scene_common_checks(M, overlap, n_points));
+  if (n_way < 1 || n_way > MAX_WAY || k_shot < 1 || k_shot > MAX_SHOT) return R3DFS_E_UNSUPPORTED;
+  if (min_points < 0 || !(min_ratio >= 0.0 && min_ratio <= 1.0)) return R3DFS_E_BADARG;
+  SupportSel sel{};
+  for (int w = 0; w < n_way; ++w) {
+    for (int v = 0; v < w; ++v)
+      if (h_classes[v] == h_classes[w]) return R3DFS_E_BADARG;
+    sel.cls[w] = h_classes[w];
+    sel.wkey[w] = lowbias32(lowbias32(seed) + (uint32_t)w + 1u);
+  }
+  sel.n_way = n_way;
+  sel.min_points = min_points;
+  sel.min_ratio = min_ratio;
+  if (plan_ws_bytes < r3dfs_scene_workspace(M, overlap)) return R3DFS_E_WORKSPACE;
+  if (ws_bytes < r3dfs_scene_support_workspace(n_way, k_shot)) return R3DFS_E_WORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  WsBump pws(const_cast<void*>(plan_ws), plan_ws_bytes);
+  SceneWs p;
+  carve_scene(pws, M, overlap, p);
+  WsBump ws(wsp, ws_bytes);
+  SupportWs w;
+  carve_support(ws, n_way, k_shot, w);
+  scene_support_count_kernel<<<SUP_CTAS, SUP_T, 0, st>>>(p.hdr, p.keys[0], p.vals[0], p.mem_point,
+                                                         p.seg_start, labels, sel, w.part_top,
+                                                         w.part_n);
+  R3DFS_CHECK_LAUNCH();
+  scene_support_pick_kernel<<<n_way, SUP_T, 0, st>>>(p.hdr, p.keys[0], p.seg_start, w.part_top,
+                                                     w.part_n, n_way, k_shot, w.shot_seg,
+                                                     shot_block, n_eligible);
+  R3DFS_CHECK_LAUNCH();
+  scene_support_cloud_kernel<<<n_way * k_shot, 256, 0, st>>>(
+      points, s_m, s_c, n_points, labels, sel, k_shot, p.vals[0], p.mem_point, p.seg_start,
+      w.shot_seg, support_x, support_y, support_src);
   R3DFS_CHECK_LAUNCH();
   return 0;
 }

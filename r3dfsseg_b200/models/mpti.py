@@ -7,8 +7,9 @@ FPS multi-prototypes, k-NN Gaussian affinity graph, label propagation, loss — 
 libr3dfs.so (`r3dfs_mpti_forward`), with no host synchronisation inside.  `forward_episodes`
 runs a batch of independent episodes through the same call.  `encode_support` / `segment` split
 that call in two, so that a labelled support set is encoded once and any number of query clouds
-are segmented against it (`r3dfs_mpti_support` / `r3dfs_mpti_query`).  State-dict keys are the
-reference's.
+are segmented against it (`r3dfs_mpti_support` / `r3dfs_mpti_query`).  `segment_scene` labels a
+whole scan against such a set, and `support_from_scene` cuts the support clouds out of a labelled
+scan (`r3dfs_scene_*`).  State-dict keys are the reference's.
 """
 from __future__ import annotations
 
@@ -299,6 +300,61 @@ class MPTI_SelfAtten(nn.Module):
             logits[b0:b0 + B] = r[0][:, 0]
         out = ops.scene_merge(plan, logits, E)
         out["n_chunks"] = E
+        return out
+
+    def support_from_scene(self, points, labels, classes, k_shot=None, block_size=1.0, overlap=1,
+                           seed=0, min_points=100, min_ratio=0.05):
+        """Cuts a support set out of a labelled scan, as the reference's loader builds support
+        shots (class2scans + sample_pointcloud(support=True)).
+        points: (M, 6) CUDA tensor as for segment_scene; labels: (M,) int32 or int64 CUDA tensor of
+        class ids; classes: the model's n_way distinct class ids, one per way.  The scan is cut into
+        the blocks segment_scene uses (block_size, overlap, seed); a block can serve class c when it
+        holds more than max(floor(n_b * min_ratio), min_points) points of c.  Each way takes the
+        k_shot such blocks with the smallest seeded keys and samples n_points of each, normalised
+        as a chunk cloud; the mask is label == c.  The contract is in include/r3dfs.h ("Support
+        shots from a labelled scan").
+        Returns dict(support_x (n_way, k_shot, 9, N), support_y (n_way, k_shot, N) int32, src,
+        block (n_way, k_shot), n_eligible (n_way,)) for encode_support(s["support_x"],
+        s["support_y"]).  Shots of several scans combine with torch.cat along dim 1.  Raises
+        ValueError when a class has fewer than k_shot eligible blocks.  Eager only: n_eligible is
+        read back once."""
+        k_shot = self.k_shot if k_shot is None else k_shot
+        if not isinstance(points, torch.Tensor) or not points.is_cuda:
+            raise ValueError("points must be a CUDA tensor")
+        if points.dim() != 2 or points.shape[1] != 6 or points.shape[0] == 0:
+            raise ValueError(f"points must be (M, 6) with M > 0; got {tuple(points.shape)}")
+        if not isinstance(labels, torch.Tensor) or labels.device != points.device or \
+                labels.dtype not in (torch.int32, torch.int64) or \
+                tuple(labels.shape) != (points.shape[0],):
+            raise ValueError(f"labels must be an int32 or int64 ({points.shape[0]},) tensor on "
+                             f"{points.device}")
+        classes = list(classes)
+        if len(classes) != self.n_way or any(int(c) != c or not -2 ** 31 <= c < 2 ** 31
+                                             for c in classes) or len(set(classes)) != len(classes):
+            raise ValueError(f"classes must be {self.n_way} distinct int32 class ids; got {classes}")
+        if int(k_shot) != k_shot or not 1 <= k_shot <= 32:
+            raise ValueError(f"k_shot must be an integer in 1..32; got {k_shot}")
+        if int(overlap) != overlap or not 1 <= overlap <= 4:
+            raise ValueError(f"overlap must be an integer in 1..4; got {overlap}")
+        if not float(block_size) > 0.0 or float(block_size) == float("inf"):
+            raise ValueError(f"block_size must be a positive number of metres; got {block_size}")
+        if int(seed) != seed or not 0 <= seed < 2 ** 32:
+            raise ValueError(f"seed must be a uint32; got {seed}")
+        if int(min_points) != min_points or not 0 <= min_points < 2 ** 31:
+            raise ValueError(f"min_points must be a non-negative int32; got {min_points}")
+        if not 0.0 <= float(min_ratio) <= 1.0:
+            raise ValueError(f"min_ratio must be in [0, 1]; got {min_ratio}")
+        plan = ops.scene_plan(points, self.n_points, float(block_size), int(overlap), int(seed))
+        out = ops.scene_support(plan, labels, [int(c) for c in classes], int(k_shot), int(seed),
+                                int(min_points), float(min_ratio))
+        n_el = out["n_eligible"].tolist()
+        if any(n < 0 for n in n_el):
+            raise ValueError("points hold a non-finite x or y coordinate, or the scan spans 2^31 "
+                             "blocks or more")
+        short = [f"class {c}: {n} eligible blocks" for c, n in zip(classes, n_el) if n < k_shot]
+        if short:
+            raise ValueError(f"too few blocks for k_shot={k_shot} ({'; '.join(short)}); lower "
+                             "min_points / min_ratio or k_shot, or add shots from another scan")
         return out
 
     def forward(self, support_x, support_y, query_x, query_y, gt_support_y=None, gt_query_y=None,

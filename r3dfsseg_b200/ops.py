@@ -707,6 +707,46 @@ def scene_merge(plan: ScenePlan, logits: torch.Tensor, n_chunks: int):
     return out
 
 
+def scene_support(plan: ScenePlan, labels: torch.Tensor, classes: Sequence[int], k_shot: int,
+                  seed: int = 0, min_points: int = 100, min_ratio: float = 0.05):
+    """Support shots of a labelled scan (r3dfs_scene_support): for every class, the k_shot blocks
+    with the smallest seeded keys among those holding more than max(floor(n_b * min_ratio),
+    min_points) of its points, each sampled to the plan's n_points and normalised as a chunk.
+    `plan` must come from scene_plan with the same seed; labels (M,) int32 or int64 class ids.
+    Enqueued only.  Returns dict(support_x (n_way, k_shot, 9, N), a view over point-major memory
+    that encode_support takes as it is; support_y (n_way, k_shot, N) int32 masks; src
+    (n_way, k_shot, N) int32 scan point of every slot; block (n_way, k_shot) int32 block id, -1 for
+    a missing shot; n_eligible (n_way,) int32 device tensor, -1 when the plan found no valid grid)."""
+    pts = plan.points
+    dev = _need_cuda(labels)
+    M, N = int(pts.shape[0]), plan.n_points
+    if tuple(labels.shape) != (M,):
+        raise ValueError(f"labels must be ({M},); got {tuple(labels.shape)}")
+    labels = labels.to(torch.int32).contiguous()
+    n_way, k_shot = len(classes), int(k_shot)
+    L = _lib.lib()
+    need = L.r3dfs_scene_support_workspace(n_way, k_shot)
+    if need == 0:
+        raise _lib.R3dfsError(f"{n_way} classes x {k_shot} shots is outside what libr3dfs is built "
+                              "for: 1..7 classes, 1..32 shots")
+    ws = _ws(need, dev)
+    x = torch.empty((n_way, k_shot, N, 9), dtype=torch.float32, device=dev)
+    out = {"support_x": x.transpose(2, 3),
+           "support_y": torch.empty((n_way, k_shot, N), dtype=torch.int32, device=dev),
+           "src": torch.empty((n_way, k_shot, N), dtype=torch.int32, device=dev),
+           "block": torch.empty((n_way, k_shot), dtype=torch.int32, device=dev),
+           "n_eligible": torch.empty((n_way,), dtype=torch.int32, device=dev)}
+    h_cls = (C.c_int32 * n_way)(*[int(c) for c in classes])
+    with torch.cuda.device(dev):
+        check(L.r3dfs_scene_support(
+            _p(pts), M, pts.stride(0), pts.stride(1), _p(labels), h_cls, n_way, k_shot,
+            int(min_points), float(min_ratio), int(seed), plan.overlap, N, _p(x),
+            _p(out["support_y"]), _p(out["src"]), _p(out["block"]), _p(out["n_eligible"]),
+            _p(plan.workspace), plan.workspace.numel(), _p(ws), ws.numel(), _stream()),
+            "r3dfs_scene_support")
+    return out
+
+
 def confusion_accumulate(pred: torch.Tensor, gt: torch.Tensor, class_slot: torch.Tensor,
                          counters: torch.Tensor) -> None:
     """evaluate_metric counters (eval_noise.py:35-62), accumulated in place into the (3, n_slots)
