@@ -751,6 +751,12 @@ size_t r3dfs_mpti_workspace(const r3dfs_episode_cfg_t* cfg, int n_episodes) {
   return ws.off + 4096;
 }
 
+// the stage recorder of diag's events, or nullptr when it names none
+static const StageRec* stage_rec(const r3dfs_episode_diag_t* diag, StageRec& srv) {
+  srv.ev = diag ? (cudaEvent_t*)diag->h_stage_events : nullptr;
+  return srv.ev ? &srv : nullptr;
+}
+
 // support part of the episode (models/mpti.py:440-493): noise suppression, fg/bg sets, FPS seeds,
 // assignment, prototype means.  F rows [sup_off, sup_off + ns_pts) of every f_rows-row block hold
 // the support features; prototype p of set s of episode e is written to row
@@ -828,8 +834,8 @@ int episode_graph_half(const r3dfs_episode_cfg_t* cfg, const EpisodeDims& d, int
                               const int64_t* query_y, float* logits, float* loss, int32_t* pred,
                               const r3dfs_episode_diag_t* diag, cudaStream_t st, bool latency) {
   const int D = R3DFS_FEAT_DIM;
-  StageRec srv{diag ? (cudaEvent_t*)diag->h_stage_events : nullptr};
-  const StageRec* sr = srv.ev ? &srv : nullptr;
+  StageRec srv;
+  const StageRec* sr = stage_rec(diag, srv);
   cudaError_t ce = cudaMemset2DAsync(w.F, sizeof(float) * d.ep_rows * D, 0,
                                      sizeof(float) * (size_t)d.ppad * D, E, st);
   if (ce != cudaSuccess) return (int)ce;
@@ -838,6 +844,29 @@ int episode_graph_half(const r3dfs_episode_cfg_t* cfg, const EpisodeDims& d, int
                                  sr));
   return episode_query_part(cfg, d, E, w, d.ep_rows, query_y, logits, loss, pred, diag, st, sr,
                             latency);
+}
+
+// input stage of a whole episode: the clouds -> point-major, episode-major order [queries |
+// supports] (F's row layout), then the features of every cloud (models/mpti.py:433-437), written
+// straight into the node matrix
+static int episode_input(const r3dfs_episode_cfg_t* cfg, const EpisodeDims& d,
+                         const r3dfs_weights_t* hw, int E, const EpisodeWs& w,
+                         const float* support_x, int64_t s_e, int64_t s_cloud, int64_t s_c,
+                         int64_t s_n, const float* query_x, int64_t q_e, int64_t q_cloud,
+                         int64_t q_c, int64_t q_n, cudaStream_t st, const StageRec* sr) {
+  const int N = cfg->n_points, in_dim = hw->in_dim;
+  if (sr) sr->mark(R3DFS_ST_BEGIN, st);
+  const int64_t tq = (int64_t)E * cfg->n_query * N * in_dim;
+  gather_clouds_kernel<<<nblk(tq), 256, 0, st>>>(query_x, cfg->n_query, in_dim, N, q_e, q_cloud,
+                                                 q_c, q_n, d.cpe, 0, w.xp, tq);
+  R3DFS_CHECK_LAUNCH();
+  const int64_t tsup = (int64_t)E * d.C * N * in_dim;
+  gather_clouds_kernel<<<nblk(tsup), 256, 0, st>>>(support_x, d.C, in_dim, N, s_e, s_cloud, s_c,
+                                                   s_n, d.cpe, cfg->n_query, w.xp, tsup);
+  R3DFS_CHECK_LAUNCH();
+  if (sr) sr->mark(R3DFS_ST_INPUT, st);
+  RowMap fmap{d.cpe, N, d.ep_rows, (int64_t)d.ppad};
+  return encoder_forward(hw, w.xp, (int64_t)E * d.cpe, N, w.enc, w.F, fmap, nullptr, st, sr);
 }
 
 size_t r3dfs_mpti_support_workspace(const r3dfs_episode_cfg_t* cfg, int n_sets) {
@@ -884,28 +913,14 @@ int r3dfs_mpti_forward(const r3dfs_episode_cfg_t* cfg, const r3dfs_weights_t* hw
   if ((int64_t)E * d.cpe > 65535) return R3DFS_E_UNSUPPORTED;
   if (ws_bytes < r3dfs_mpti_workspace(cfg, E)) return R3DFS_E_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
-  const int N = cfg->n_points, in_dim = hw->in_dim;
   WsBump ws(wsp, ws_bytes);
   EpisodeWs w;
-  carve_episode(ws, cfg, d, E, in_dim, hw->dgcnn_k, w);
+  carve_episode(ws, cfg, d, E, hw->in_dim, hw->dgcnn_k, w);
   if (!ws.ok()) return R3DFS_E_WORKSPACE;
-  const int64_t B = (int64_t)E * d.cpe;
-  StageRec srv{diag ? (cudaEvent_t*)diag->h_stage_events : nullptr};
-  const StageRec* sr = srv.ev ? &srv : nullptr;
-  if (sr) sr->mark(R3DFS_ST_BEGIN, st);
-  // clouds -> point-major, episode-major order [queries | supports] (matches F's row layout)
-  int64_t tq = (int64_t)E * cfg->n_query * N * in_dim;
-  gather_clouds_kernel<<<nblk(tq), 256, 0, st>>>(query_x, cfg->n_query, in_dim, N, q_e, q_cloud,
-                                                 q_c, q_n, d.cpe, 0, w.xp, tq);
-  R3DFS_CHECK_LAUNCH();
-  int64_t tsup = (int64_t)E * d.C * N * in_dim;
-  gather_clouds_kernel<<<nblk(tsup), 256, 0, st>>>(support_x, d.C, in_dim, N, s_e, s_cloud, s_c,
-                                                   s_n, d.cpe, cfg->n_query, w.xp, tsup);
-  R3DFS_CHECK_LAUNCH();
-  if (sr) sr->mark(R3DFS_ST_INPUT, st);
-  // features of every cloud (models/mpti.py:433-437), written straight into the node matrix
-  RowMap fmap{d.cpe, N, d.ep_rows, (int64_t)d.ppad};
-  R3DFS_TRY(encoder_forward(hw, w.xp, B, N, w.enc, w.F, fmap, nullptr, st, sr));
+  StageRec srv;
+  const StageRec* sr = stage_rec(diag, srv);
+  R3DFS_TRY(episode_input(cfg, d, hw, E, w, support_x, s_e, s_cloud, s_c, s_n, query_x, q_e,
+                          q_cloud, q_c, q_n, st, sr));
   return episode_graph_half(cfg, d, E, w, support_x, s_e, s_cloud, s_c, s_n, support_y, query_y,
                             logits, loss, pred, diag, st);
 }
@@ -923,22 +938,13 @@ int r3dfs_protonet_forward(const r3dfs_episode_cfg_t* cfg, const r3dfs_weights_t
   if (dist_method != 0 || (int64_t)E * d.cpe > 65535) return R3DFS_E_UNSUPPORTED;
   if (ws_bytes < r3dfs_mpti_workspace(cfg, E)) return R3DFS_E_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
-  const int N = cfg->n_points, in_dim = hw->in_dim, D = R3DFS_FEAT_DIM;
+  const int N = cfg->n_points, D = R3DFS_FEAT_DIM;
   WsBump ws(wsp, ws_bytes);
   EpisodeWs w;
-  carve_episode(ws, cfg, d, E, in_dim, hw->dgcnn_k, w);
+  carve_episode(ws, cfg, d, E, hw->in_dim, hw->dgcnn_k, w);
   if (!ws.ok()) return R3DFS_E_WORKSPACE;
-  const int64_t B = (int64_t)E * d.cpe;
-  int64_t tq = (int64_t)E * cfg->n_query * N * in_dim;
-  gather_clouds_kernel<<<nblk(tq), 256, 0, st>>>(query_x, cfg->n_query, in_dim, N, q_e, q_cloud,
-                                                 q_c, q_n, d.cpe, 0, w.xp, tq);
-  R3DFS_CHECK_LAUNCH();
-  int64_t tsup = (int64_t)E * d.C * N * in_dim;
-  gather_clouds_kernel<<<nblk(tsup), 256, 0, st>>>(support_x, d.C, in_dim, N, s_e, s_cloud, s_c,
-                                                   s_n, d.cpe, cfg->n_query, w.xp, tsup);
-  R3DFS_CHECK_LAUNCH();
-  RowMap fmap{d.cpe, N, d.ep_rows, (int64_t)d.ppad};
-  R3DFS_TRY(encoder_forward(hw, w.xp, B, N, w.enc, w.F, fmap, nullptr, st));
+  R3DFS_TRY(episode_input(cfg, d, hw, E, w, support_x, s_e, s_cloud, s_c, s_n, query_x, q_e,
+                          q_cloud, q_c, q_n, st, nullptr));
   const int32_t* keep = nullptr;
   if (cfg->mdns) {  // Mean_pl_support_y_multi_scale (models/protonet.py:491-536) = the MPTI kernels
     R3DFS_TRY(launch_mdns(support_x, s_e, s_cloud, s_c, s_n, support_y, w.F, d.ep_rows, d.nn, E,
@@ -1013,8 +1019,8 @@ int r3dfs_mpti_support(const r3dfs_episode_cfg_t* cfg, const r3dfs_weights_t* hw
   carve_support(ws, cfg, d, n_sets, in_dim, hw->dgcnn_k, w);
   if (!ws.ok()) return R3DFS_E_WORKSPACE;
   w.proto_cnt = proto_count;
-  StageRec srv{diag ? (cudaEvent_t*)diag->h_stage_events : nullptr};
-  const StageRec* sr = srv.ev ? &srv : nullptr;
+  StageRec srv;
+  const StageRec* sr = stage_rec(diag, srv);
   if (sr) sr->mark(R3DFS_ST_BEGIN, st);
   const int64_t proto_rows = (int64_t)d.S * d.slot;
   cudaError_t ce = cudaMemsetAsync(proto, 0, sizeof(float) * (size_t)n_sets * proto_rows * D, st);
@@ -1055,8 +1061,8 @@ int r3dfs_mpti_query(const r3dfs_episode_cfg_t* cfg, const r3dfs_weights_t* hw, 
   EpisodeWs w;
   carve_query(ws, &qc, d, E, in_dim, hw->dgcnn_k, w);
   if (!ws.ok()) return R3DFS_E_WORKSPACE;
-  StageRec srv{diag ? (cudaEvent_t*)diag->h_stage_events : nullptr};
-  const StageRec* sr = srv.ev ? &srv : nullptr;
+  StageRec srv;
+  const StageRec* sr = stage_rec(diag, srv);
   if (sr) sr->mark(R3DFS_ST_BEGIN, st);
   const int64_t tq = (int64_t)E * qc.n_query * N * in_dim;
   gather_clouds_kernel<<<nblk(tq), 256, 0, st>>>(query_x, qc.n_query, in_dim, N, q_e, q_cloud, q_c,

@@ -25,6 +25,42 @@ from .attention import SelfAttention
 from .dgcnn import DGCNN
 
 
+def _need_eval(m: nn.Module) -> None:
+    if m.training:
+        raise NotImplementedError("r3dfsseg_b200: stand-alone call in training mode; use "
+                                  "forward(..., train=True) for the training step or .eval()")
+
+
+def packed_weights(model: nn.Module) -> ops.PackedWeights:
+    """The model's weights as the kernels read them, packed lazily in eager mode and packed again
+    when the signature of its parameters and buffers changed: the storage and version counter of
+    each, which change with any in-place update (optimizer step, load_state_dict, BatchNorm
+    statistics).  model._packed_sig is the signature of the packed weights."""
+    if torch.compiler.is_compiling():
+        # tracing (torch.compile / export): the packed tensors are graph inputs, built beforehand
+        if model._packed is None:
+            raise RuntimeError("call model.pack_weights() once before tracing the module")
+        return model._packed
+    sig = tuple((t.data_ptr(), t._version) for t in model.state_dict(keep_vars=True).values())
+    if model._packed is None or sig != model._packed_sig:
+        model._packed = ops.PackedWeights(model)
+        model._packed_sig = sig
+    return model._packed
+
+
+def _check_scan(points, block_size, overlap, seed) -> None:
+    if not isinstance(points, torch.Tensor) or not points.is_cuda:
+        raise ValueError("points must be a CUDA tensor")
+    if points.dim() != 2 or points.shape[1] != 6 or points.shape[0] == 0:
+        raise ValueError(f"points must be (M, 6) with M > 0; got {tuple(points.shape)}")
+    if int(overlap) != overlap or not 1 <= overlap <= 4:
+        raise ValueError(f"overlap must be an integer in 1..4; got {overlap}")
+    if not float(block_size) > 0.0 or float(block_size) == float("inf"):
+        raise ValueError(f"block_size must be a positive number of metres; got {block_size}")
+    if int(seed) != seed or not 0 <= seed < 2 ** 32:
+        raise ValueError(f"seed must be a uint32; got {seed}")
+
+
 class BaseLearner(nn.Module):
     """Conv1d(bias) + BatchNorm1d stack, ReLU between layers (reference models/mpti.py:18-40)."""
 
@@ -38,9 +74,7 @@ class BaseLearner(nn.Module):
             width = out_dim
 
     def forward(self, x):
-        if self.training:
-            raise NotImplementedError("r3dfsseg_b200: stand-alone call in training mode; use "
-                                      "forward(..., train=True) for the training step or .eval()")
+        _need_eval(self)
         B, _, N = x.shape
         h = x.transpose(1, 2).reshape(B * N, -1)
         for i, seq in enumerate(self.convs):
@@ -106,22 +140,7 @@ class MPTI_SelfAtten(nn.Module):
         self._train_step = 0
 
     # ---------------------------------------------------------------------------------------
-    def _weights(self) -> ops.PackedWeights:
-        if torch.compiler.is_compiling():
-            # tracing (torch.compile / export): the packed tensors are graph inputs, built beforehand
-            if self._packed is None:
-                raise RuntimeError("call model.pack_weights() once before tracing the module")
-            return self._packed
-        sig = self._state_sig()
-        if self._packed is None or sig != self._packed_sig:
-            self._packed = ops.PackedWeights(self)
-            self._packed_sig = sig
-        return self._packed
-
-    def _state_sig(self) -> Tuple:
-        # storage and version counter of every parameter and buffer: changes with any in-place
-        # update (optimizer step, load_state_dict, BatchNorm statistics)
-        return tuple((t.data_ptr(), t._version) for t in self.state_dict(keep_vars=True).values())
+    _weights = packed_weights
 
     def pack_weights(self) -> ops.PackedWeights:
         """Folds the BatchNorm statistics into per-channel scale/shift and packs the 31 weight
@@ -136,9 +155,7 @@ class MPTI_SelfAtten(nn.Module):
 
     def getFeatures(self, x):
         """(B, C_in, N) -> (B, 192, N)   (reference models/mpti.py:579-589)"""
-        if self.training:
-            raise NotImplementedError("r3dfsseg_b200: stand-alone call in training mode; use "
-                                      "forward(..., train=True) for the training step or .eval()")
+        _need_eval(self)
         pw = self._weights()
         return ops.op.features(x, pw.tensors, self.in_channels, int(self.encoder.k)).transpose(1, 2)
 
@@ -150,9 +167,7 @@ class MPTI_SelfAtten(nn.Module):
         Returns dict(logits (E, n_query, N, n_way+1), loss (E), pred (E, n_query, N)).
         With `support_feat` (E, n_way*k_shot*N, 192) / `query_feat` (E, n_query*N, 192) given,
         the encoder is skipped and only the graph half runs on those features."""
-        if self.training:
-            raise NotImplementedError("r3dfsseg_b200: stand-alone call in training mode; use "
-                                      "forward(..., train=True) for the training step or .eval()")
+        _need_eval(self)
         if support_feat is None and stage_events is None and query_y is not None:
             # the registered op r3dfs::mpti_forward (traceable: torch.compile, fake tensors)
             pw = self._weights()
@@ -165,11 +180,13 @@ class MPTI_SelfAtten(nn.Module):
                 out["diag"] = {"proto_count": r[3], "clean_flag": r[4], "cg_iters": r[5],
                                "cg_resid": r[6]}
             return out
+        # eager only (ctypes structs): stage events, precomputed features, no query labels
         cfg = self._cfg(query_x.shape[1], mdns=bool(eval))
+        if support_feat is not None:
+            return ops.mpti_forward_features(cfg, support_x, support_y, support_feat, query_feat,
+                                             query_y, want_diag, workspace, stage_events)
         return ops.mpti_forward(self._weights(), cfg, support_x, support_y, query_x, query_y,
-                                want_diag=want_diag, workspace=workspace,
-                                support_feat=support_feat, query_feat=query_feat,
-                                stage_events=stage_events)
+                                want_diag, workspace, stage_events)
 
     # ---------------------------------------------------------------------------------------
     def encode_support(self, support_x, support_y, eval=True) -> SupportSet:
@@ -177,9 +194,7 @@ class MPTI_SelfAtten(nn.Module):
         support set: (n_way, k_shot, C, N) / (n_way, k_shot, N) for one set, or a leading S for
         S sets.  eval=True runs the noise suppression, exactly as forward(eval=True).  The result
         is handed to `segment` as often as wanted."""
-        if self.training:
-            raise NotImplementedError("r3dfsseg_b200: stand-alone call in training mode; use "
-                                      "forward(..., train=True) for the training step or .eval()")
+        _need_eval(self)
         if support_x.dim() == 4:
             support_x, support_y = support_x.unsqueeze(0), support_y.unsqueeze(0)
         if support_x.dim() != 5 or support_y.dim() != 4:
@@ -197,6 +212,34 @@ class MPTI_SelfAtten(nn.Module):
         return SupportSet(proto, count, clean, int(n_way), int(k_shot), int(N),
                           int(self.n_subprototypes), bool(eval), sig)
 
+    def _check_support(self, support: SupportSet) -> None:
+        _need_eval(self)
+        if (support.n_way, support.n_points, support.n_subprototypes) != \
+                (self.n_way, self.n_points, self.n_subprototypes):
+            raise ValueError(
+                f"support set built for n_way={support.n_way} n_points={support.n_points} "
+                f"n_subprototypes={support.n_subprototypes}; the model has n_way={self.n_way} "
+                f"n_points={self.n_points} n_subprototypes={self.n_subprototypes}")
+
+    def _support_weights(self, support: SupportSet) -> ops.PackedWeights:
+        """The packed weights, refused when they are not those `support` was encoded under."""
+        pw = self._weights()
+        if not torch.compiler.is_compiling() and self._packed_sig != support.weights_sig:
+            raise RuntimeError("the weights or BatchNorm statistics changed after the support set "
+                               "was encoded: its prototypes are stale, call encode_support again")
+        return pw
+
+    def _query(self, pw: ops.PackedWeights, support: SupportSet, query_x, query_y=None, sel=None):
+        """The registered op r3dfs::mpti_query (traceable) of E query episodes against `support`:
+        episode i against set i, against the one set (read in place), or against set sel[i]."""
+        proto, count = support.prototypes, support.proto_count
+        if sel is not None:
+            proto, count = proto.index_select(0, sel), count.index_select(0, sel)
+        return ops.op.mpti_query(pw.tensors, self.in_channels, int(self.encoder.k), proto, count,
+                                 query_x, query_y, sel is None and support.n_sets == 1,
+                                 support.k_shot, self.k_connect, float(self.sigma), self.lp_alpha,
+                                 self.cg_max_iter, self.cg_tol, None)
+
     def segment(self, support: SupportSet, query_x, query_y=None,
                 set_index: Optional[Sequence[int]] = None):
         """Query half of forward (models/mpti.py:436-437, 495-571) against an encoded support set.
@@ -205,38 +248,21 @@ class MPTI_SelfAtten(nn.Module):
         Returns dict(logits (E, n_query, N, n_way+1), loss (E), pred (E, n_query, N)), equal bit
         for bit to forward_episodes on the same supports.  A 3-D query_x (n_query, C, N) is one
         episode and returns what forward returns: (query_pred (n_query, n_way+1, N), loss)."""
-        if self.training:
-            raise NotImplementedError("r3dfsseg_b200: stand-alone call in training mode; use "
-                                      "forward(..., train=True) for the training step or .eval()")
-        if (support.n_way, support.n_points, support.n_subprototypes) != \
-                (self.n_way, self.n_points, self.n_subprototypes):
-            raise ValueError(
-                f"support set built for n_way={support.n_way} n_points={support.n_points} "
-                f"n_subprototypes={support.n_subprototypes}; the model has n_way={self.n_way} "
-                f"n_points={self.n_points} n_subprototypes={self.n_subprototypes}")
+        self._check_support(support)
         single = query_x.dim() == 3
         if single:
             query_x = query_x.unsqueeze(0)
             query_y = None if query_y is None else query_y.unsqueeze(0)
         E, S = query_x.shape[0], support.n_sets
-        proto, count, shared = support.prototypes, support.proto_count, False
+        sel = None
         if set_index is not None:
             idx = [int(i) for i in set_index]
             if len(idx) != E or any(i < 0 or i >= S for i in idx):
                 raise ValueError(f"set_index must hold {E} indices in [0, {S}); got {idx}")
-            sel = torch.tensor(idx, dtype=torch.int64, device=proto.device)
-            proto, count = proto.index_select(0, sel), count.index_select(0, sel)
-        elif S == 1:
-            shared = True
-        elif S != E:
+            sel = torch.tensor(idx, dtype=torch.int64, device=support.prototypes.device)
+        elif S != 1 and S != E:
             raise ValueError(f"{S} support sets for {E} query episodes: pass set_index")
-        pw = self._weights()
-        if not torch.compiler.is_compiling() and self._packed_sig != support.weights_sig:
-            raise RuntimeError("the weights or BatchNorm statistics changed after the support set "
-                               "was encoded: its prototypes are stale, call encode_support again")
-        r = ops.op.mpti_query(pw.tensors, self.in_channels, int(self.encoder.k), proto, count,
-                              query_x, query_y, shared, support.k_shot, self.k_connect,
-                              float(self.sigma), self.lp_alpha, self.cg_max_iter, self.cg_tol, None)
+        r = self._query(self._support_weights(support), support, query_x, query_y, sel)
         if single:
             return r[0][0].transpose(1, 2), r[1][0]
         return {"logits": r[0], "loss": r[1], "pred": r[2]}
@@ -255,33 +281,13 @@ class MPTI_SelfAtten(nn.Module):
         point, n_chunks).  Eager only: the chunk count depends on the data and is read back once.
         Results are reproducible for a given chunk_batch; another chunk_batch can change the
         logits in the last bits, as the query kernels round differently at another batch size."""
-        if self.training:
-            raise NotImplementedError("r3dfsseg_b200: stand-alone call in training mode; use "
-                                      "forward(..., train=True) for the training step or .eval()")
-        if (support.n_way, support.n_points, support.n_subprototypes) != \
-                (self.n_way, self.n_points, self.n_subprototypes):
-            raise ValueError(
-                f"support set built for n_way={support.n_way} n_points={support.n_points} "
-                f"n_subprototypes={support.n_subprototypes}; the model has n_way={self.n_way} "
-                f"n_points={self.n_points} n_subprototypes={self.n_subprototypes}")
+        self._check_support(support)
         if support.n_sets != 1:
             raise ValueError(f"a scene is segmented against one support set; got {support.n_sets}")
-        if not isinstance(points, torch.Tensor) or not points.is_cuda:
-            raise ValueError("points must be a CUDA tensor")
-        if points.dim() != 2 or points.shape[1] != 6 or points.shape[0] == 0:
-            raise ValueError(f"points must be (M, 6) with M > 0; got {tuple(points.shape)}")
-        if int(overlap) != overlap or not 1 <= overlap <= 4:
-            raise ValueError(f"overlap must be an integer in 1..4; got {overlap}")
-        if not float(block_size) > 0.0 or float(block_size) == float("inf"):
-            raise ValueError(f"block_size must be a positive number of metres; got {block_size}")
-        if int(seed) != seed or not 0 <= seed < 2 ** 32:
-            raise ValueError(f"seed must be a uint32; got {seed}")
+        _check_scan(points, block_size, overlap, seed)
         if int(chunk_batch) < 1 or chunk_batch > 65535:
             raise ValueError(f"chunk_batch must be in 1..65535; got {chunk_batch}")
-        pw = self._weights()
-        if self._packed_sig != support.weights_sig:
-            raise RuntimeError("the weights or BatchNorm statistics changed after the support set "
-                               "was encoded: its prototypes are stale, call encode_support again")
+        pw = self._support_weights(support)
         N, nc = self.n_points, self.n_classes
         plan = ops.scene_plan(points, N, float(block_size), int(overlap), int(seed))
         E = int(plan.n_chunks.item())
@@ -293,11 +299,7 @@ class MPTI_SelfAtten(nn.Module):
         logits = torch.empty((E, N, nc), dtype=torch.float32, device=points.device)
         B = int(chunk_batch)
         for b0 in range(0, E, B):
-            r = ops.op.mpti_query(pw.tensors, self.in_channels, int(self.encoder.k),
-                                  support.prototypes, support.proto_count, query_x[b0:b0 + B], None,
-                                  True, support.k_shot, self.k_connect, float(self.sigma),
-                                  self.lp_alpha, self.cg_max_iter, self.cg_tol, None)
-            logits[b0:b0 + B] = r[0][:, 0]
+            logits[b0:b0 + B] = self._query(pw, support, query_x[b0:b0 + B])[0][:, 0]
         out = ops.scene_merge(plan, logits, E)
         out["n_chunks"] = E
         return out
@@ -319,10 +321,7 @@ class MPTI_SelfAtten(nn.Module):
         ValueError when a class has fewer than k_shot eligible blocks.  Eager only: n_eligible is
         read back once."""
         k_shot = self.k_shot if k_shot is None else k_shot
-        if not isinstance(points, torch.Tensor) or not points.is_cuda:
-            raise ValueError("points must be a CUDA tensor")
-        if points.dim() != 2 or points.shape[1] != 6 or points.shape[0] == 0:
-            raise ValueError(f"points must be (M, 6) with M > 0; got {tuple(points.shape)}")
+        _check_scan(points, block_size, overlap, seed)
         if not isinstance(labels, torch.Tensor) or labels.device != points.device or \
                 labels.dtype not in (torch.int32, torch.int64) or \
                 tuple(labels.shape) != (points.shape[0],):
@@ -334,12 +333,6 @@ class MPTI_SelfAtten(nn.Module):
             raise ValueError(f"classes must be {self.n_way} distinct int32 class ids; got {classes}")
         if int(k_shot) != k_shot or not 1 <= k_shot <= 32:
             raise ValueError(f"k_shot must be an integer in 1..32; got {k_shot}")
-        if int(overlap) != overlap or not 1 <= overlap <= 4:
-            raise ValueError(f"overlap must be an integer in 1..4; got {overlap}")
-        if not float(block_size) > 0.0 or float(block_size) == float("inf"):
-            raise ValueError(f"block_size must be a positive number of metres; got {block_size}")
-        if int(seed) != seed or not 0 <= seed < 2 ** 32:
-            raise ValueError(f"seed must be a uint32; got {seed}")
         if int(min_points) != min_points or not 0 <= min_points < 2 ** 31:
             raise ValueError(f"min_points must be a non-negative int32; got {min_points}")
         if not 0.0 <= float(min_ratio) <= 1.0:

@@ -17,7 +17,7 @@ import torch.nn.functional as F
 from .. import ops
 from .attention import SelfAttention
 from .dgcnn import DGCNN
-from .mpti import BaseLearner
+from .mpti import BaseLearner, packed_weights
 
 
 class ProtoNet_Contrast(nn.Module):
@@ -43,12 +43,7 @@ class ProtoNet_Contrast(nn.Module):
         self._packed_sig = None
         self.clean_flag = None
 
-    def _weights(self) -> ops.PackedWeights:
-        sig = tuple((t.data_ptr(), t._version) for t in self.state_dict(keep_vars=True).values())
-        if self._packed is None or sig != self._packed_sig:
-            self._packed = ops.PackedWeights(self)
-            self._packed_sig = sig
-        return self._packed
+    _weights = packed_weights
 
     def getFeatures(self, x):
         """(B, C_in, N) -> (B, 192, N)   (reference models/protonet.py:860-876)"""

@@ -387,103 +387,128 @@ def make_cfg(n_way: int, k_shot: int, n_query: int, n_points: int, n_subprototyp
                       float(alpha), int(bool(mdns)), int(cg_max_iter), float(cg_tol))
 
 
-def _envelope_error(cfg: EpisodeCfg) -> "_lib.R3dfsError":
-    """What a workspace query of 0 means for an episode configuration."""
-    return _lib.R3dfsError(
-        "episode configuration outside what libr3dfs is built for: n_way 1..7, k_shot 1..32, "
-        "n_points >= 64, n_subprototypes 1..127, k_connect 1..1024 and < n_queries * n_points, "
-        "graph nodes = roundup64((n_way + 1) * (n_subprototypes + 1)) + n_queries * n_points <= 8192 "
-        "(the merged rows index columns with 16 bits and the CG kernels stage 8192 nodes); got "
-        f"n_way={cfg.n_way} k_shot={cfg.k_shot} n_query={cfg.n_query} n_points={cfg.n_points} "
-        f"n_subprototypes={cfg.n_subprototypes} k_connect={cfg.k_connect}")
-
-
-def _stage_event_array(stage_events: Optional[Sequence["torch.cuda.Event"]]):
-    """Raw cudaEvent_t handles of caller-owned torch events (created by a first record())."""
-    if stage_events is None:
-        return None
-    if len(stage_events) != len(_lib.STAGES):
-        raise ValueError(f"need {len(_lib.STAGES)} stage events")
-    return (C.c_void_p * len(stage_events))(*[int(e.cuda_event) for e in stage_events])
-
-
-def _mpti_forward_raw(pw: Optional[PackedWeights], cfg: EpisodeCfg, support_x: torch.Tensor,
-                 support_y: torch.Tensor, query_x: torch.Tensor, query_y: Optional[torch.Tensor],
-                 want_diag: bool = False, workspace: Optional[torch.Tensor] = None,
-                 support_feat: Optional[torch.Tensor] = None,
-                 query_feat: Optional[torch.Tensor] = None,
-                 stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
-    """E episodes in one call.
-    support_x (E, n_way, k_shot, C, N) any strides with uniform cloud stride; support_y
-    (E, n_way, k_shot, N) int32; query_x (E, n_query, C, N); query_y (E, n_query, N) int64.
-    Returns dict(logits (E, n_query, N, n_way+1), loss (E), pred (E, n_query, N) int32 [, diag])."""
-    dev = _need_cuda(support_x, support_y, query_x, query_y)
-    support_x, query_x = _f32(support_x), _f32(query_x)
-    E, n_way, k_shot, Cin, N = support_x.shape
-    nq = query_x.shape[1]
-    if (n_way, k_shot, nq, N) != (cfg.n_way, cfg.k_shot, cfg.n_query, cfg.n_points):
-        raise ValueError("episode tensors do not match the episode configuration")
+def _support_in(cfg: EpisodeCfg, support_x: torch.Tensor, support_y: torch.Tensor,
+                n_query: Optional[int] = None):
+    """Support clouds (S, n_way, k_shot, C, N) as fp32 with the uniform cloud stride the C ABI
+    takes, masks as int32.  Checked against cfg, with n_query for whole episodes."""
+    support_x = _f32(support_x)
+    _, n_way, k_shot, _, N = support_x.shape
+    if (n_way, k_shot, N) != (cfg.n_way, cfg.k_shot, cfg.n_points) or \
+            n_query not in (None, cfg.n_query):
+        raise ValueError(("support" if n_query is None else "episode") +
+                         " tensors do not match the episode configuration")
     if support_x.stride(1) != k_shot * support_x.stride(2):
         support_x = support_x.contiguous()
-    support_y = support_y.to(torch.int32).contiguous()
-    if query_y is not None:
-        query_y = query_y.to(torch.int64).contiguous()
-    nc = n_way + 1
-    logits = torch.empty((E, nq, N, nc), dtype=torch.float32, device=dev)
-    loss = torch.zeros((E,), dtype=torch.float32, device=dev)
-    pred = torch.empty((E, nq, N), dtype=torch.int32, device=dev)
-    L = _lib.lib()
-    need = L.r3dfs_mpti_workspace(C.byref(cfg), E)
+    return support_x, support_y.to(torch.int32).contiguous()
+
+
+def _support_args(support_x: torch.Tensor):
+    """Pointer and (episode, cloud, channel, point) strides of `_support_in`'s clouds."""
+    return (_p(support_x), support_x.stride(0), *support_x.stride()[2:])
+
+
+def _episode_out(E: int, n_query: int, N: int, nc: int, dev: torch.device):
+    return {"logits": torch.empty((E, n_query, N, nc), dtype=torch.float32, device=dev),
+            "loss": torch.zeros((E,), dtype=torch.float32, device=dev),
+            "pred": torch.empty((E, n_query, N), dtype=torch.int32, device=dev)}
+
+
+def _episode_ws(need: int, cfg: EpisodeCfg, dev: torch.device,
+                workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """`workspace` when it holds `need` bytes, else a new one.  A workspace query of 0 means the
+    configuration is outside what the library is built for."""
     if need == 0:
-        raise _envelope_error(cfg)
-    ws = workspace if workspace is not None and workspace.numel() >= need else _ws(need, dev)
-    diag = None
-    dstruct = None
-    ev_arr = _stage_event_array(stage_events)
-    if want_diag or ev_arr is not None:
-        dstruct = EpisodeDiag(None, None, None, None, None)
+        raise _lib.R3dfsError(
+            "episode configuration outside what libr3dfs is built for: n_way 1..7, k_shot 1..32, "
+            "n_points >= 64, n_subprototypes 1..127, k_connect 1..1024 and < n_queries * n_points, "
+            "graph nodes = roundup64((n_way + 1) * (n_subprototypes + 1)) + n_queries * n_points "
+            "<= 8192 (the merged rows index columns with 16 bits and the CG kernels stage 8192 "
+            f"nodes); got n_way={cfg.n_way} k_shot={cfg.k_shot} n_query={cfg.n_query} "
+            f"n_points={cfg.n_points} n_subprototypes={cfg.n_subprototypes} "
+            f"k_connect={cfg.k_connect}")
+    return workspace if workspace is not None and workspace.numel() >= need else _ws(need, dev)
+
+
+def _diag_bufs(cfg: EpisodeCfg, E: int, dev: torch.device, clean_flag: bool = True):
+    d = {"proto_count": torch.zeros((E, cfg.n_way + 1), dtype=torch.int32, device=dev),
+         "cg_iters": torch.zeros((E,), dtype=torch.int32, device=dev),
+         "cg_resid": torch.zeros((E,), dtype=torch.float32, device=dev)}
+    if clean_flag:
+        d["clean_flag"] = torch.ones((E, cfg.n_way, cfg.k_shot), dtype=torch.float32, device=dev)
+    return d
+
+
+def _diag_ref(bufs: dict, stage_events: Optional[Sequence["torch.cuda.Event"]]):
+    """Reference to an r3dfs_episode_diag_t over the device buffers in `bufs` (by field name) and
+    the raw cudaEvent_t handles of caller-owned torch events (created by a first record()), or
+    None when there is neither."""
+    if not bufs and stage_events is None:
+        return None
+    d = EpisodeDiag(*[bufs[f].data_ptr() if f in bufs else None
+                      for f in ("proto_count", "clean_flag", "cg_iters", "cg_resid")], None)
+    if stage_events is not None:
+        if len(stage_events) != len(_lib.STAGES):
+            raise ValueError(f"need {len(_lib.STAGES)} stage events")
+        ev = (C.c_void_p * len(stage_events))(*[int(e.cuda_event) for e in stage_events])
+        d.h_stage_events = C.cast(ev, C.POINTER(C.c_void_p))   # the struct keeps `ev` alive
+    return C.byref(d)
+
+
+def mpti_forward(pw: PackedWeights, cfg: EpisodeCfg, support_x: torch.Tensor,
+                 support_y: torch.Tensor, query_x: torch.Tensor, query_y: Optional[torch.Tensor],
+                 want_diag: bool = False, workspace: Optional[torch.Tensor] = None,
+                 stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
+    """E episodes in one call (r3dfs_mpti_forward).
+    support_x (E, n_way, k_shot, C, N) any strides with uniform cloud stride; support_y
+    (E, n_way, k_shot, N) int32; query_x (E, n_query, C, N); query_y (E, n_query, N) int64.
+    Returns dict(logits (E, n_query, N, n_way+1), loss (E), pred (E, n_query, N) int32 [, diag]).
+    Eager; module code calls the registered op `r3dfs::mpti_forward`."""
+    dev = _need_cuda(support_x, support_y, query_x, query_y)
+    support_x, support_y = _support_in(cfg, support_x, support_y, query_x.shape[1])
+    query_x = _f32(query_x)
+    query_y = None if query_y is None else query_y.to(torch.int64).contiguous()
+    E = support_x.shape[0]
+    out = _episode_out(E, cfg.n_query, cfg.n_points, cfg.n_way + 1, dev)
+    L = _lib.lib()
+    ws = _episode_ws(L.r3dfs_mpti_workspace(C.byref(cfg), E), cfg, dev, workspace)
     if want_diag:
-        diag = {
-            "proto_count": torch.zeros((E, nc), dtype=torch.int32, device=dev),
-            "clean_flag": torch.ones((E, n_way, k_shot), dtype=torch.float32, device=dev),
-            "cg_iters": torch.zeros((E,), dtype=torch.int32, device=dev),
-            "cg_resid": torch.zeros((E,), dtype=torch.float32, device=dev),
-        }
-        dstruct.proto_count = diag["proto_count"].data_ptr()
-        dstruct.clean_flag = diag["clean_flag"].data_ptr()
-        dstruct.cg_iters = diag["cg_iters"].data_ptr()
-        dstruct.cg_resid = diag["cg_resid"].data_ptr()
-    if ev_arr is not None:
-        dstruct.h_stage_events = C.cast(ev_arr, C.POINTER(C.c_void_p))
-    if support_feat is not None:
-        # precomputed features (point-major (E, rows, 192)): graph half only
-        support_feat = _f32(support_feat).contiguous()
-        query_feat = _f32(query_feat).contiguous()
-        assert support_feat.shape == (E, n_way * k_shot * N, 192)
-        assert query_feat.shape == (E, nq * N, 192)
-        with torch.cuda.device(dev):
-            check(L.r3dfs_mpti_forward_features(
-                C.byref(cfg), E, _p(support_x), support_x.stride(0), support_x.stride(2),
-                support_x.stride(3), support_x.stride(4), _p(support_y), _p(support_feat),
-                _p(query_feat), _p(query_y), _p(logits), _p(loss), _p(pred),
-                C.byref(dstruct) if dstruct is not None else None, _p(ws), ws.numel(), _stream()),
-                "r3dfs_mpti_forward_features")
-        out = {"logits": logits, "loss": loss, "pred": pred}
-        if diag is not None:
-            out["diag"] = diag
-        return out
+        out["diag"] = _diag_bufs(cfg, E, dev)
     with torch.cuda.device(dev):
         check(L.r3dfs_mpti_forward(
-            C.byref(cfg), C.byref(pw.struct), E,
-            _p(support_x), support_x.stride(0), support_x.stride(2), support_x.stride(3),
-            support_x.stride(4), _p(support_y),
-            _p(query_x), query_x.stride(0), query_x.stride(1), query_x.stride(2), query_x.stride(3),
-            _p(query_y), _p(logits), _p(loss), _p(pred),
-            C.byref(dstruct) if dstruct is not None else None, _p(ws), ws.numel(), _stream()),
-            "r3dfs_mpti_forward")
-    out = {"logits": logits, "loss": loss, "pred": pred}
-    if diag is not None:
-        out["diag"] = diag
+            C.byref(cfg), C.byref(pw.struct), E, *_support_args(support_x), _p(support_y),
+            _p(query_x), *query_x.stride(), _p(query_y), _p(out["logits"]), _p(out["loss"]),
+            _p(out["pred"]), _diag_ref(out.get("diag", {}), stage_events), _p(ws), ws.numel(),
+            _stream()), "r3dfs_mpti_forward")
+    return out
+
+
+def mpti_forward_features(cfg: EpisodeCfg, support_x: torch.Tensor, support_y: torch.Tensor,
+                          support_feat: torch.Tensor, query_feat: torch.Tensor,
+                          query_y: Optional[torch.Tensor], want_diag: bool = False,
+                          workspace: Optional[torch.Tensor] = None,
+                          stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
+    """The graph half of E episodes on precomputed point-major features
+    (r3dfs_mpti_forward_features): support_feat (E, n_way*k_shot*N, 192), query_feat
+    (E, n_query*N, 192); the other tensors and the result as `mpti_forward`."""
+    dev = _need_cuda(support_x, support_y, support_feat, query_feat, query_y)
+    N = cfg.n_points
+    support_x, support_y = _support_in(cfg, support_x, support_y, query_feat.shape[1] // N)
+    support_feat, query_feat = _f32(support_feat).contiguous(), _f32(query_feat).contiguous()
+    query_y = None if query_y is None else query_y.to(torch.int64).contiguous()
+    E = support_x.shape[0]
+    assert support_feat.shape == (E, cfg.n_way * cfg.k_shot * N, 192)
+    assert query_feat.shape == (E, cfg.n_query * N, 192)
+    out = _episode_out(E, cfg.n_query, N, cfg.n_way + 1, dev)
+    L = _lib.lib()
+    ws = _episode_ws(L.r3dfs_mpti_workspace(C.byref(cfg), E), cfg, dev, workspace)
+    if want_diag:
+        out["diag"] = _diag_bufs(cfg, E, dev)
+    with torch.cuda.device(dev):
+        check(L.r3dfs_mpti_forward_features(
+            C.byref(cfg), E, *_support_args(support_x), _p(support_y), _p(support_feat),
+            _p(query_feat), _p(query_y), _p(out["logits"]), _p(out["loss"]), _p(out["pred"]),
+            _diag_ref(out.get("diag", {}), stage_events), _p(ws), ws.numel(), _stream()),
+            "r3dfs_mpti_forward_features")
     return out
 
 
@@ -500,88 +525,60 @@ def protonet_forward(pw: PackedWeights, cfg: EpisodeCfg, support_x: torch.Tensor
         raise NotImplementedError(
             "Error! Distance computation method (%s) is unknown!" % dist_method)
     dev = _need_cuda(support_x, support_y, query_x, query_y)
-    support_x, query_x = _f32(support_x), _f32(query_x)
-    E, n_way, k_shot, Cin, N = support_x.shape
-    nq = query_x.shape[1]
-    if (n_way, k_shot, nq, N) != (cfg.n_way, cfg.k_shot, cfg.n_query, cfg.n_points):
-        raise ValueError("episode tensors do not match the episode configuration")
-    if support_x.stride(1) != k_shot * support_x.stride(2):
-        support_x = support_x.contiguous()
-    support_y = support_y.to(torch.int32).contiguous()
-    if query_y is not None:
-        query_y = query_y.to(torch.int64).contiguous()
-    nc = n_way + 1
-    logits = torch.empty((E, nq, N, nc), dtype=torch.float32, device=dev)
-    loss = torch.zeros((E,), dtype=torch.float32, device=dev)
-    pred = torch.empty((E, nq, N), dtype=torch.int32, device=dev)
-    clean = torch.ones((E, n_way, k_shot), dtype=torch.float32, device=dev)
+    support_x, support_y = _support_in(cfg, support_x, support_y, query_x.shape[1])
+    query_x = _f32(query_x)
+    query_y = None if query_y is None else query_y.to(torch.int64).contiguous()
+    E = support_x.shape[0]
+    out = _episode_out(E, cfg.n_query, cfg.n_points, cfg.n_way + 1, dev)
+    out["clean_flag"] = torch.ones((E, cfg.n_way, cfg.k_shot), dtype=torch.float32, device=dev)
     L = _lib.lib()
-    need = L.r3dfs_mpti_workspace(C.byref(cfg), E)
-    if need == 0:
-        raise _envelope_error(cfg)
-    ws = workspace if workspace is not None and workspace.numel() >= need else _ws(need, dev)
+    ws = _episode_ws(L.r3dfs_mpti_workspace(C.byref(cfg), E), cfg, dev, workspace)
     with torch.cuda.device(dev):
         check(L.r3dfs_protonet_forward(
-            C.byref(cfg), C.byref(pw.struct), E,
-            _p(support_x), support_x.stride(0), support_x.stride(2), support_x.stride(3),
-            support_x.stride(4), _p(support_y),
-            _p(query_x), query_x.stride(0), query_x.stride(1), query_x.stride(2), query_x.stride(3),
-            _p(query_y), 0, _p(logits), _p(loss), _p(pred), _p(clean), _p(ws), ws.numel(),
-            _stream()), "r3dfs_protonet_forward")
-    return {"logits": logits, "loss": loss, "pred": pred, "clean_flag": clean}
+            C.byref(cfg), C.byref(pw.struct), E, *_support_args(support_x), _p(support_y),
+            _p(query_x), *query_x.stride(), _p(query_y), 0, _p(out["logits"]), _p(out["loss"]),
+            _p(out["pred"]), _p(out["clean_flag"]), _p(ws), ws.numel(), _stream()),
+            "r3dfs_protonet_forward")
+    return out
 
 
-def _mpti_support_raw(pw: PackedWeights, cfg: EpisodeCfg, support_x: torch.Tensor,
-                      support_y: torch.Tensor, want_diag: bool = False,
-                      stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
-    """The support half of S episodes in one call (r3dfs_mpti_support).
+def mpti_support(pw: PackedWeights, cfg: EpisodeCfg, support_x: torch.Tensor,
+                 support_y: torch.Tensor, want_diag: bool = False,
+                 stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
+    """The support half of S episodes in one call (r3dfs_mpti_support), encoded once.
     support_x (S, n_way, k_shot, C, N) any strides with uniform cloud stride, support_y
     (S, n_way, k_shot, N).  Returns (proto (S, n_way+1, n_subprototypes+1, 192), proto_count
-    (S, n_way+1) int32, clean_flag (S, n_way, k_shot) or None without want_diag)."""
+    (S, n_way+1) int32, clean_flag (S, n_way, k_shot) or None without want_diag).
+    Eager; module code calls the registered op `r3dfs::mpti_support`."""
     dev = _need_cuda(support_x, support_y)
-    support_x = _f32(support_x)
-    S, n_way, k_shot, Cin, N = support_x.shape
-    if (n_way, k_shot, N) != (cfg.n_way, cfg.k_shot, cfg.n_points):
-        raise ValueError("support tensors do not match the episode configuration")
-    if support_x.stride(1) != k_shot * support_x.stride(2):
-        support_x = support_x.contiguous()
-    support_y = support_y.to(torch.int32).contiguous()
-    nc = n_way + 1
+    support_x, support_y = _support_in(cfg, support_x, support_y)
+    S, nc = support_x.shape[0], cfg.n_way + 1
     proto = torch.empty((S, nc, cfg.n_subprototypes + 1, 192), dtype=torch.float32, device=dev)
     count = torch.empty((S, nc), dtype=torch.int32, device=dev)
-    clean = torch.ones((S, n_way, k_shot), dtype=torch.float32, device=dev) if want_diag else None
+    clean = torch.ones((S, cfg.n_way, cfg.k_shot), dtype=torch.float32,
+                       device=dev) if want_diag else None
     L = _lib.lib()
-    need = L.r3dfs_mpti_support_workspace(C.byref(cfg), S)
-    if need == 0:
-        raise _envelope_error(cfg)
-    ws = _ws(need, dev)
-    ev_arr = _stage_event_array(stage_events)
-    dstruct = None
-    if want_diag or ev_arr is not None:
-        dstruct = EpisodeDiag(None, None if clean is None else clean.data_ptr(), None, None, None)
-        if ev_arr is not None:
-            dstruct.h_stage_events = C.cast(ev_arr, C.POINTER(C.c_void_p))
+    ws = _episode_ws(L.r3dfs_mpti_support_workspace(C.byref(cfg), S), cfg, dev)
+    diag = {} if clean is None else {"clean_flag": clean}
     with torch.cuda.device(dev):
         check(L.r3dfs_mpti_support(
-            C.byref(cfg), C.byref(pw.struct), S,
-            _p(support_x), support_x.stride(0), support_x.stride(2), support_x.stride(3),
-            support_x.stride(4), _p(support_y), _p(proto), _p(count),
-            C.byref(dstruct) if dstruct is not None else None, _p(ws), ws.numel(), _stream()),
+            C.byref(cfg), C.byref(pw.struct), S, *_support_args(support_x), _p(support_y),
+            _p(proto), _p(count), _diag_ref(diag, stage_events), _p(ws), ws.numel(), _stream()),
             "r3dfs_mpti_support")
     return proto, count, clean
 
 
-def _mpti_query_raw(pw: PackedWeights, cfg: EpisodeCfg, proto: torch.Tensor,
-                    proto_count: torch.Tensor, query_x: torch.Tensor,
-                    query_y: Optional[torch.Tensor] = None, shared: bool = False,
-                    want_diag: bool = False, workspace: Optional[torch.Tensor] = None,
-                    stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
+def mpti_query(pw: PackedWeights, cfg: EpisodeCfg, proto: torch.Tensor, proto_count: torch.Tensor,
+               query_x: torch.Tensor, query_y: Optional[torch.Tensor] = None, shared: bool = False,
+               want_diag: bool = False, workspace: Optional[torch.Tensor] = None,
+               stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
     """The query half of E episodes in one call (r3dfs_mpti_query) against the prototypes of
     `mpti_support`.  proto (S, n_way+1, n_subprototypes+1, 192), proto_count (S, n_way+1):
     S == E (episode i uses set i), or S == 1 with shared=True (every episode uses set 0, read in
     place).  query_x (E, n_query, C, N) any strides, query_y (E, n_query, N) or None.
     Returns dict(logits (E, n_query, N, n_way+1), loss (E), pred (E, n_query, N) int32 [, diag
-    (proto_count, cg_iters, cg_resid)])."""
+    (proto_count, cg_iters, cg_resid)]).  Eager; module code calls the registered op
+    `r3dfs::mpti_query`."""
     dev = _need_cuda(proto, proto_count, query_x, query_y)
     query_x = _f32(query_x)
     E, nq, Cin, N = query_x.shape
@@ -596,39 +593,18 @@ def _mpti_query_raw(pw: PackedWeights, cfg: EpisodeCfg, proto: torch.Tensor,
     if S != (1 if shared else E):
         raise ValueError(f"{S} prototype sets for {E} episodes (shared={shared})")
     p_e, c_e = (0, 0) if shared else (nc * slot * 192, nc)
-    if query_y is not None:
-        query_y = query_y.to(torch.int64).contiguous()
-    logits = torch.empty((E, nq, N, nc), dtype=torch.float32, device=dev)
-    loss = torch.zeros((E,), dtype=torch.float32, device=dev)
-    pred = torch.empty((E, nq, N), dtype=torch.int32, device=dev)
+    query_y = None if query_y is None else query_y.to(torch.int64).contiguous()
+    out = _episode_out(E, nq, N, nc, dev)
     L = _lib.lib()
-    need = L.r3dfs_mpti_query_workspace(C.byref(cfg), E)
-    if need == 0:
-        raise _envelope_error(cfg)
-    ws = workspace if workspace is not None and workspace.numel() >= need else _ws(need, dev)
-    ev_arr = _stage_event_array(stage_events)
-    diag = dstruct = None
-    if want_diag or ev_arr is not None:
-        dstruct = EpisodeDiag(None, None, None, None, None)
+    ws = _episode_ws(L.r3dfs_mpti_query_workspace(C.byref(cfg), E), cfg, dev, workspace)
     if want_diag:
-        diag = {"proto_count": torch.zeros((E, nc), dtype=torch.int32, device=dev),
-                "cg_iters": torch.zeros((E,), dtype=torch.int32, device=dev),
-                "cg_resid": torch.zeros((E,), dtype=torch.float32, device=dev)}
-        dstruct.proto_count = diag["proto_count"].data_ptr()
-        dstruct.cg_iters = diag["cg_iters"].data_ptr()
-        dstruct.cg_resid = diag["cg_resid"].data_ptr()
-    if ev_arr is not None:
-        dstruct.h_stage_events = C.cast(ev_arr, C.POINTER(C.c_void_p))
+        out["diag"] = _diag_bufs(cfg, E, dev, clean_flag=False)
     with torch.cuda.device(dev):
         check(L.r3dfs_mpti_query(
             C.byref(cfg), C.byref(pw.struct), E, _p(proto), p_e, _p(proto_count), c_e,
-            _p(query_x), query_x.stride(0), query_x.stride(1), query_x.stride(2), query_x.stride(3),
-            _p(query_y), _p(logits), _p(loss), _p(pred),
-            C.byref(dstruct) if dstruct is not None else None, _p(ws), ws.numel(), _stream()),
-            "r3dfs_mpti_query")
-    out = {"logits": logits, "loss": loss, "pred": pred}
-    if diag is not None:
-        out["diag"] = diag
+            _p(query_x), *query_x.stride(), _p(query_y), _p(out["logits"]), _p(out["loss"]),
+            _p(out["pred"]), _diag_ref(out.get("diag", {}), stage_events), _p(ws), ws.numel(),
+            _stream()), "r3dfs_mpti_query")
     return out
 
 
@@ -948,8 +924,8 @@ def _mpti_forward_op(weights: Sequence[torch.Tensor], in_dim: int, dgcnn_k: int,
     E, n_way, k_shot, _, N = support_x.shape
     cfg = make_cfg(n_way, k_shot, query_x.shape[1], N, n_subprototypes, k_connect, sigma, alpha,
                    mdns, cg_max_iter, cg_tol)
-    out = _mpti_forward_raw(_WeightsView(weights, in_dim, dgcnn_k), cfg, support_x, support_y,
-                            query_x, query_y, want_diag=True, workspace=workspace)
+    out = mpti_forward(_WeightsView(weights, in_dim, dgcnn_k), cfg, support_x, support_y, query_x,
+                       query_y, want_diag=True, workspace=workspace)
     d = out["diag"]
     return (out["logits"], out["loss"], out["pred"], d["proto_count"], d["clean_flag"],
             d["cg_iters"], d["cg_resid"])
@@ -975,8 +951,8 @@ def _mpti_support_op(weights: Sequence[torch.Tensor], in_dim: int, dgcnn_k: int,
     clean_flag (S, n_way, k_shot)).  n_query / k_connect only enter the envelope check."""
     S, n_way, k_shot, _, N = support_x.shape
     cfg = make_cfg(n_way, k_shot, n_query, N, n_subprototypes, k_connect, mdns=mdns)
-    return _mpti_support_raw(_WeightsView(weights, in_dim, dgcnn_k), cfg, support_x, support_y,
-                             want_diag=True)
+    return mpti_support(_WeightsView(weights, in_dim, dgcnn_k), cfg, support_x, support_y,
+                        want_diag=True)
 
 
 @_mpti_support_op.register_fake
@@ -1001,8 +977,8 @@ def _mpti_query_op(weights: Sequence[torch.Tensor], in_dim: int, dgcnn_k: int, p
     E, nq, _, N = query_x.shape
     n_way, n_sub = proto.shape[1] - 1, proto.shape[2] - 1
     cfg = make_cfg(n_way, k_shot, nq, N, n_sub, k_connect, sigma, alpha, False, cg_max_iter, cg_tol)
-    out = _mpti_query_raw(_WeightsView(weights, in_dim, dgcnn_k), cfg, proto, proto_count, query_x,
-                          query_y, shared, want_diag=True, workspace=workspace)
+    out = mpti_query(_WeightsView(weights, in_dim, dgcnn_k), cfg, proto, proto_count, query_x,
+                     query_y, shared, want_diag=True, workspace=workspace)
     d = out["diag"]
     return out["logits"], out["loss"], out["pred"], d["cg_iters"], d["cg_resid"]
 
@@ -1017,56 +993,3 @@ def _(weights, in_dim, dgcnn_k, proto, proto_count, query_x, query_y, shared, k_
 
 # the registered ops, for module code (traceable by torch.compile / fake tensors)
 op = torch.ops.r3dfs
-
-
-def mpti_forward(pw: Optional[PackedWeights], cfg: EpisodeCfg, support_x: torch.Tensor,
-                 support_y: torch.Tensor, query_x: torch.Tensor, query_y: Optional[torch.Tensor],
-                 want_diag: bool = False, workspace: Optional[torch.Tensor] = None,
-                 support_feat: Optional[torch.Tensor] = None,
-                 query_feat: Optional[torch.Tensor] = None,
-                 stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
-    """E episodes in one call (see _mpti_forward_raw).  The plain case goes through the registered
-    op `r3dfs::mpti_forward`; stage events and precomputed features are eager-only diagnostics."""
-    if stage_events is not None or support_feat is not None or query_y is None or pw is None:
-        return _mpti_forward_raw(pw, cfg, support_x, support_y, query_x, query_y, want_diag,
-                                 workspace, support_feat, query_feat, stage_events)
-    r = op.mpti_forward(pw.tensors, pw.struct.in_dim, pw.struct.dgcnn_k, support_x, support_y,
-                        query_x, query_y, cfg.n_subprototypes, cfg.k_connect, cfg.sigma, cfg.alpha,
-                        bool(cfg.mdns), cfg.cg_max_iter, cfg.cg_tol, workspace)
-    out = {"logits": r[0], "loss": r[1], "pred": r[2]}
-    if want_diag:
-        out["diag"] = {"proto_count": r[3], "clean_flag": r[4], "cg_iters": r[5], "cg_resid": r[6]}
-    return out
-
-
-def mpti_support(pw: PackedWeights, cfg: EpisodeCfg, support_x: torch.Tensor,
-                 support_y: torch.Tensor, want_diag: bool = False,
-                 stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
-    """Support half of S episodes, encoded once (see _mpti_support_raw): -> (proto, proto_count,
-    clean_flag or None).  The plain case goes through the registered op `r3dfs::mpti_support`."""
-    if stage_events is not None:
-        return _mpti_support_raw(pw, cfg, support_x, support_y, want_diag, stage_events)
-    proto, count, clean = op.mpti_support(pw.tensors, pw.struct.in_dim, pw.struct.dgcnn_k,
-                                          support_x, support_y, cfg.n_query, cfg.n_subprototypes,
-                                          cfg.k_connect, bool(cfg.mdns))
-    return proto, count, clean if want_diag else None
-
-
-def mpti_query(pw: PackedWeights, cfg: EpisodeCfg, proto: torch.Tensor, proto_count: torch.Tensor,
-               query_x: torch.Tensor, query_y: Optional[torch.Tensor] = None, shared: bool = False,
-               want_diag: bool = False, workspace: Optional[torch.Tensor] = None,
-               stage_events: Optional[Sequence["torch.cuda.Event"]] = None):
-    """Query half of E episodes against given prototypes (see _mpti_query_raw); returns the dict
-    of `mpti_forward`.  The plain case goes through the registered op `r3dfs::mpti_query`."""
-    if stage_events is not None:
-        return _mpti_query_raw(pw, cfg, proto, proto_count, query_x, query_y, shared, want_diag,
-                               workspace, stage_events)
-    if (proto.shape[1], proto.shape[2]) != (cfg.n_way + 1, cfg.n_subprototypes + 1):
-        raise ValueError("prototypes do not match the episode configuration")
-    r = op.mpti_query(pw.tensors, pw.struct.in_dim, pw.struct.dgcnn_k, proto, proto_count, query_x,
-                      query_y, bool(shared), cfg.k_shot, cfg.k_connect, cfg.sigma, cfg.alpha,
-                      cfg.cg_max_iter, cfg.cg_tol, workspace)
-    out = {"logits": r[0], "loss": r[1], "pred": r[2]}
-    if want_diag:
-        out["diag"] = {"cg_iters": r[3], "cg_resid": r[4]}
-    return out

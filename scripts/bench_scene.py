@@ -52,11 +52,7 @@ def run_phases(model, support, pts, overlap, chunk_batch, seed=0):
     qx = chunk_x.view(E, 1, N_PTS, 9).transpose(2, 3)
     logits = torch.empty((E, N_PTS, N_WAY + 1), dtype=torch.float32, device=pts.device)
     for b0 in range(0, E, chunk_batch):
-        r = ops.op.mpti_query(pw.tensors, model.in_channels, int(model.encoder.k),
-                              support.prototypes, support.proto_count, qx[b0:b0 + chunk_batch],
-                              None, True, support.k_shot, model.k_connect, float(model.sigma),
-                              model.lp_alpha, model.cg_max_iter, model.cg_tol, None)
-        logits[b0:b0 + chunk_batch] = r[0][:, 0]
+        logits[b0:b0 + chunk_batch] = model._query(pw, support, qx[b0:b0 + chunk_batch])[0][:, 0]
     ev[3].record()
     out = ops.scene_merge(plan, logits, E)
     ev[4].record()
