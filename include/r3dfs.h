@@ -458,6 +458,93 @@ int r3dfs_scene_support(const float* points, int64_t M, int64_t s_m, int64_t s_c
                         int32_t* shot_block, int32_t* n_eligible, const void* plan_ws,
                         size_t plan_ws_bytes, void* ws, size_t ws_bytes, r3dfs_stream_t stream);
 
+/* Few-shot episodes from labelled scans (the reference's NoiseInMetaTest.generate_one_episode,
+ * dataloaders/loader.py:648-890, over its class2scans lists).
+ *
+ * Dataset index.  A dataset is a list of labelled scans concatenated into one points and one labels
+ * array; scan i starts at point point_base_i.  Every scan is planned by r3dfs_scene_plan on its own
+ * slice (one block_size, overlap and seed for all) and appended by r3dfs_scene_index, which reads
+ * the plan workspace (the workspace may be freed afterwards).  Global blocks are numbered in scan
+ * order, then by ascending block id within the scan:
+ *   block_off (n_blocks + 1) int64: first membership of each block in `member`;
+ *   block_scan, block_id (n_blocks) int32: its scan and its block id in that scan;
+ *   member (n_members) int32: the GLOBAL point of every member, in the plan's rank order k(i);
+ *   count (n_blocks, n_cls) int32: members whose label is h_classes[k] (1..64 distinct ids; other
+ *     labels count for no class).
+ * r3dfs_scene_index appends one scan at (n_blocks, n_members), the sizes so far, and writes the
+ * scan's block and membership counts to HOST h_sizes[0..1] (it synchronises the stream once).  When
+ * the arrays' capacities (block_cap blocks, member_cap members) are too small it returns
+ * R3DFS_E_WORKSPACE after writing h_sizes, with nothing written: grow them and call again.  A plan
+ * that found no valid grid gives h_sizes = -1 and R3DFS_E_BADARG.  Limits: the plan's, point_base + M
+ * < 2^31 and total memberships < 2^31 (R3DFS_E_UNSUPPORTED).
+ * r3dfs_scene_index_classes, once after the last scan: block b is eligible for class k iff
+ *   count(b, k) > max(floor(n_b * min_ratio), min_points), the product in fp64 (the rule of
+ *   r3dfs_scene_support).  elig_off (n_cls + 1) and elig_block (room for n_blocks * n_cls) hold
+ *   every class's eligible global blocks in ascending order (the reference's class2scans);
+ *   h_elig_off (HOST, n_cls + 1) receives a copy (one stream synchronisation).  ws:
+ *   r3dfs_scene_index_workspace bytes; n_blocks * n_cls < 2^31 - 1.
+ *
+ * Episodes.  r3dfs_scene_episodes builds E episodes of n_way ways, k_shot shots and n_queries query
+ * blocks per way.  Host inputs: h_elig_off (from r3dfs_scene_index_classes), h_classes (the index's
+ * n_cls ids), h_way_class (E, n_way) class ids, h_n_noise (E) noisy shots per way, noise_type
+ * (0 none, 1 ood, 2 sym, 3 pair) and h_pair (n_cls) = pair[h_classes[k]] as class ids (pair only;
+ * may map a class to itself).  Episode e has index g = first + e * step (uint32).  Every key is
+ * integer hashing with lowbias32 (see "Segmenting a whole scan"), H(a, b) = lowbias32(a ^
+ * lowbias32(b)) on uint32:
+ *   K_e = H(lowbias32(seed), g);  way w: K_w = H(K_e, w + 1);  k_clean = k_shot - n_noise.
+ *   Clean shots and queries.  The way's class list is ranked by lowbias32(b ^ K_w) over the global
+ *     block index b (a bijection: no ties); the first k_clean blocks are the clean shots, the next
+ *     n_queries the way's query blocks (distinct from its shots; blocks may repeat across ways).
+ *   Noise range R.  ood: the index's classes with at least one eligible block that are not among
+ *     the episode's ways, in index order; sym: the other ways' classes in way order; pair:
+ *     [pair[c]].  Noisy shot j (0 <= j < n_noise) takes class R[(H(K_w, 64 + j) * |R|) >> 32]
+ *     (64-bit product), except when k_clean - 1 == 1 for ood and sym, the reference's single-use
+ *     rule: then it takes R[pi[min(j, |R| - 1)]], where pi lists 0..|R|-1 by ascending
+ *     lowbias32(r ^ H(K_w, 33)).  Its block is the smallest lowbias32(b ^ H(K_w, 128 + j)) of
+ *     that class's eligible list.
+ *   Shuffle.  Shot t of the way (t < k_clean: clean shot t; else noisy shot t - k_clean) goes to
+ *     slot rank_t, its rank among t = 0..k_shot-1 under lowbias32(t ^ H(K_w, 34)).
+ *   Clouds.  Slot s of a block's cloud holds member rank s mod min(n_b, N), normalised as a chunk
+ *     cloud (the shot clouds of r3dfs_scene_support).
+ * Outputs (device): support_x (E, n_way, k_shot, N, 9) and query_x (E, n_way * n_queries, N, 9)
+ *   point-major, query clouds way-major; support_y (E, n_way, k_shot, N) int32 = label == the
+ *   shot's class; gt_support_y = support_y on clean shots, 0 on noisy ones; support_flag
+ *   (E, n_way, k_shot) int32 class id of every shot; query_y (E, n_way * n_queries, N) int64 = w + 1
+ *   where label == class of way w, else 0; shot_block (E, n_way, k_shot), query_block
+ *   (E, n_way * n_queries) int32 global blocks; support_src / query_src int32 global point of
+ *   every slot.  Every output is a function of (seed, g) and the index alone.
+ * Deterministic, no atomics, no host synchronisation; the host arrays are copied into the
+ * workspace (r3dfs_scene_episodes_workspace bytes).  Limits (R3DFS_E_UNSUPPORTED): 1 <= n_way <= 7,
+ * 1 <= k_shot <= 32, n_queries >= 1, k_clean + n_queries <= 32, E * n_way * n_queries <= 65535,
+ * 1 <= n_cls <= 64, 64 <= N <= 65536.  R3DFS_E_BADARG: an unknown or repeated class, a way class
+ * with fewer than k_clean + n_queries eligible blocks, n_noise outside 0..k_shot or non-zero
+ * without noise, an empty noise range (or a pair class without eligible blocks) where n_noise > 0,
+ * first < 0, step < 1 or g past 2^32 - 1.  Every check happens before anything is launched. */
+int r3dfs_scene_index(const int32_t* labels, int64_t M, int overlap, const int32_t* h_classes,
+                      int n_cls, int32_t scan, int64_t point_base, int64_t n_blocks,
+                      int64_t n_members, int64_t block_cap, int64_t member_cap, int64_t* block_off,
+                      int32_t* block_scan, int32_t* block_id, int32_t* member, int32_t* count,
+                      int64_t* h_sizes, const void* plan_ws, size_t plan_ws_bytes,
+                      r3dfs_stream_t stream);
+size_t r3dfs_scene_index_workspace(int64_t n_blocks, int n_cls); /* 0 outside the limits */
+int r3dfs_scene_index_classes(const int64_t* block_off, const int32_t* count, int64_t n_blocks,
+                              int n_cls, int min_points, double min_ratio, int32_t* elig_off,
+                              int32_t* elig_block, int32_t* h_elig_off, void* ws, size_t ws_bytes,
+                              r3dfs_stream_t stream);
+size_t r3dfs_scene_episodes_workspace(int n_episodes, int n_way, int k_shot, int n_queries,
+                                      int n_cls); /* 0 outside the limits; host only */
+int r3dfs_scene_episodes(const float* points, int64_t s_m, int64_t s_c, const int32_t* labels,
+                         const int64_t* block_off, const int32_t* member, const int32_t* elig_off,
+                         const int32_t* elig_block, const int32_t* h_elig_off,
+                         const int32_t* h_classes, int n_cls, const int32_t* h_way_class,
+                         const int32_t* h_n_noise, int noise_type, const int32_t* h_pair,
+                         int n_episodes, int n_way, int k_shot, int n_queries, int n_points,
+                         uint32_t seed, int64_t first, int64_t step, float* support_x,
+                         int32_t* support_y, int32_t* gt_support_y, int32_t* support_flag,
+                         float* query_x, int64_t* query_y, int32_t* shot_block,
+                         int32_t* query_block, int32_t* support_src, int32_t* query_src, void* ws,
+                         size_t ws_bytes, r3dfs_stream_t stream);
+
 /* ProtoNet + MDNS (reference models/protonet.py:357-945 ProtoNet_Contrast.forward, train=False):
  * same encoder and noise suppression as MPTI, then masked average pooling of the support
  * features (:878-890), one prototype per way from the kept shots + one background prototype

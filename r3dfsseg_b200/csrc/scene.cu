@@ -6,6 +6,10 @@
 // shots out of a labelled scan: per-block class counts, a seeded choice of blocks per class, and
 // shot clouds built by the chunk clouds' code.
 //
+// r3dfs_scene_index / r3dfs_scene_index_classes / r3dfs_scene_episodes ("Few-shot episodes from
+// labelled scans") append planned scans to a dataset index (global blocks, members, class counts,
+// per-class eligible lists) and sample few-shot episodes from it with the same shot clouds.
+//
 // r3dfs_scene_plan builds every index the other calls need and leaves it in the workspace:
 //   bbox -> grid -> per-point membership counts -> scan -> one record (block << 32 | key, position)
 //   per membership -> LSD radix sort -> block segments -> chunk counts -> scan -> (chunk, slot) of
@@ -14,6 +18,7 @@
 // (__fsub_rn / __fdiv_rn), so that the numpy oracle of the tests reproduces it bit for bit, and no
 // step uses a float atomic.
 #include <algorithm>
+#include <vector>
 
 #include "common.cuh"
 
@@ -457,16 +462,32 @@ __global__ void scene_member_kernel(int64_t n, int N, SceneHdr* __restrict__ hp,
 }
 
 // ---- chunk clouds ------------------------------------------------------------------------------
-// A cloud of N slots over `count` members of one block: slot q holds the member of sorted record
-// first + (q mod count) * stride + offset, normalised over those members.  One CTA of 256 threads.
+// Member q of a plan block: sorted record first + q * stride + offset.
+struct PlanMembers {
+  const int32_t* __restrict__ vals;
+  const int32_t* __restrict__ mem_point;
+  int32_t first, stride, offset;
+  __device__ __forceinline__ int32_t operator()(int32_t q) const {
+    return mem_point[vals[first + (int64_t)q * stride + offset]];
+  }
+};
+
+// Member q of a dataset-index block: its q-th member in rank order.
+struct IndexMembers {
+  const int32_t* __restrict__ member;
+  int64_t first;
+  __device__ __forceinline__ int32_t operator()(int32_t q) const { return member[first + q]; }
+};
+
+// A cloud of N slots over `count` members of one block: slot q holds member q mod count,
+// normalised over those members.  One CTA of 256 threads.
+template <class Members>
 __device__ __forceinline__ void scene_cloud(const float* __restrict__ pts, int64_t s_m, int64_t s_c,
-                                            int N, const int32_t* __restrict__ vals,
-                                            const int32_t* __restrict__ mem_point, int32_t first,
-                                            int32_t stride, int32_t offset, int32_t count,
+                                            int N, const Members at, int32_t count,
                                             float* __restrict__ out, int32_t* __restrict__ src) {
   float mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
   for (int q = threadIdx.x; q < count; q += blockDim.x) {
-    const int64_t i = mem_point[vals[first + (int64_t)q * stride + offset]];
+    const int64_t i = at(q);
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
       const float v = pts[i * s_m + k * s_c];
@@ -502,7 +523,7 @@ __device__ __forceinline__ void scene_cloud(const float* __restrict__ pts, int64
   }
   __syncthreads();
   for (int q = threadIdx.x; q < N; q += blockDim.x) {
-    const int32_t i = mem_point[vals[first + (int64_t)(q % count) * stride + offset]];
+    const int32_t i = at(q % count);
     const float* pt = pts + (int64_t)i * s_m;
     float* o = out + (int64_t)q * 9;
 #pragma unroll
@@ -543,7 +564,7 @@ __global__ __launch_bounds__(256) void scene_chunk_kernel(
   const int32_t s = chunk_seg[c], c0 = chunk_off[s], cb = chunk_off[s + 1] - c0;
   const int32_t j = (int32_t)c - c0, p0 = seg_start[s], nb = seg_start[s + 1] - p0;
   const int32_t cnt = (nb - j + cb - 1) / cb;
-  scene_cloud(pts, s_m, s_c, N, vals, mem_point, p0, cb, j, cnt, out, src);
+  scene_cloud(pts, s_m, s_c, N, PlanMembers{vals, mem_point, p0, cb, j}, cnt, out, src);
 }
 
 // ---- merge ---------------------------------------------------------------------------------------
@@ -764,9 +785,296 @@ __global__ __launch_bounds__(256) void scene_support_cloud_kernel(
     return;
   }
   const int32_t p0 = seg_start[s], nb = seg_start[s + 1] - p0;
-  scene_cloud(pts, s_m, s_c, N, vals, mem_point, p0, 1, 0, min(nb, N), out, src);
+  scene_cloud(pts, s_m, s_c, N, PlanMembers{vals, mem_point, p0, 1, 0}, min(nb, N), out, src);
   const int32_t cls = sel.cls[g / k_shot];
   for (int q = threadIdx.x; q < N; q += blockDim.x) y[q] = labels[src[q]] == cls ? 1 : 0;
+}
+
+// ---- dataset index ----------------------------------------------------------------------------
+constexpr int MAX_IDX_CLS = 64, IDX_T = 256, IDX_WARPS = IDX_T / 32;
+
+struct IndexCls {
+  int32_t id[MAX_IDX_CLS];  // class ids, ascending
+  int32_t at[MAX_IDX_CLS];  // index of id[k] in the caller's class list
+  int32_t n;
+};
+
+// block table and members of one planned scan, appended at (b0, m0)
+__global__ void index_blocks_kernel(const SceneHdr* __restrict__ hp,
+                                    const uint64_t* __restrict__ keys,
+                                    const int32_t* __restrict__ seg_start, int32_t scan, int64_t b0,
+                                    int64_t m0, int64_t* __restrict__ block_off,
+                                    int32_t* __restrict__ block_scan,
+                                    int32_t* __restrict__ block_id) {
+  const int32_t s = blockIdx.x * blockDim.x + threadIdx.x, n_seg = hp->n_seg;
+  if (s > n_seg) return;
+  block_off[b0 + s] = m0 + seg_start[s];
+  if (s == n_seg) return;
+  block_scan[b0 + s] = scan;
+  block_id[b0 + s] = (int32_t)(keys[seg_start[s]] >> 32);
+}
+
+__global__ void index_members_kernel(int64_t T, const int32_t* __restrict__ vals,
+                                     const int32_t* __restrict__ mem_point, int64_t m0,
+                                     int32_t point_base, int32_t* __restrict__ member) {
+  const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (p < T) member[m0 + p] = point_base + mem_point[vals[p]];
+}
+
+// One warp per block: class counts of its members.  Lanes holding the same class are counted by
+// their lowest lane (__match_any_sync), so no two lanes write one counter.
+__global__ __launch_bounds__(IDX_T) void index_count_kernel(
+    const SceneHdr* __restrict__ hp, const int32_t* __restrict__ vals,
+    const int32_t* __restrict__ mem_point, const int32_t* __restrict__ seg_start,
+    const int32_t* __restrict__ labels, const __grid_constant__ IndexCls cls, int64_t b0,
+    int32_t* __restrict__ count) {
+  __shared__ int s_cnt[IDX_WARPS][MAX_IDX_CLS];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int32_t s = blockIdx.x * IDX_WARPS + wid;
+  if (s >= hp->n_seg) return;
+  for (int k = lane; k < MAX_IDX_CLS; k += 32) s_cnt[wid][k] = 0;
+  __syncwarp();
+  const int32_t p0 = seg_start[s], nb = seg_start[s + 1] - p0;
+  for (int32_t base = 0; base < nb; base += 32) {
+    int k = -1;
+    if (base + lane < nb) {
+      const int32_t l = labels[mem_point[vals[p0 + base + lane]]];
+      int lo = 0, hi = cls.n;  // first id >= l
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (cls.id[mid] < l) lo = mid + 1; else hi = mid;
+      }
+      if (lo < cls.n && cls.id[lo] == l) k = cls.at[lo];
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, k);
+    if (k >= 0 && lane == __ffs(peers) - 1) s_cnt[wid][k] += __popc(peers);
+    __syncwarp();
+  }
+  for (int k = lane; k < cls.n; k += 32) count[(b0 + s) * cls.n + k] = s_cnt[wid][k];
+}
+
+// flag[c * n_blocks + b] = block b is eligible for class c; flag[n_cls * n_blocks] = 0
+__global__ void index_flag_kernel(const int64_t* __restrict__ block_off,
+                                  const int32_t* __restrict__ count, int64_t n_blocks, int n_cls,
+                                  int min_points, double min_ratio, int32_t* __restrict__ flag) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, n = n_blocks * n_cls;
+  if (i > n) return;
+  if (i == n) {
+    flag[i] = 0;
+    return;
+  }
+  const int64_t c = i / n_blocks, b = i - c * n_blocks;
+  const int64_t nb = block_off[b + 1] - block_off[b];
+  // max(floor(n_b * min_ratio), min_points), the rule of scene_support_count_kernel
+  const double thr = fmax(floor((double)nb * min_ratio), (double)min_points);
+  flag[i] = (double)count[b * n_cls + c] > thr ? 1 : 0;
+}
+
+// after the exclusive scan: entry i is eligible iff pos[i + 1] > pos[i]
+__global__ void index_lists_kernel(const int32_t* __restrict__ pos, int64_t n_blocks, int n_cls,
+                                   int32_t* __restrict__ elig_off,
+                                   int32_t* __restrict__ elig_block) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, n = n_blocks * n_cls;
+  if (i > n) return;
+  if (i % n_blocks == 0) elig_off[i / n_blocks] = pos[i];
+  if (i < n && pos[i + 1] > pos[i]) elig_block[pos[i]] = (int32_t)(i % n_blocks);
+}
+
+// ---- episodes ---------------------------------------------------------------------------------
+enum { NOISE_NONE = 0, NOISE_OOD = 1, NOISE_SYM = 2, NOISE_PAIR = 3 };
+constexpr int EP_T = 256, EP_WARPS = EP_T / 32;
+
+struct EpisodeArgs {
+  uint32_t seed_hash;  // lowbias32(seed)
+  int64_t first, step;
+  int n_way, k_shot, n_queries, n_cls, noise_type;
+};
+
+// the host arrays, copied into the workspace as one block of int32
+struct EpisodeHost {
+  int32_t* way;      // (E, n_way) class index of every way
+  int32_t* n_noise;  // (E)
+  int32_t* cls;      // (n_cls) class ids
+  int32_t* pair;     // (n_cls) class index of pair[c]
+};
+
+struct EpisodeWs {
+  int32_t* host;   // the EpisodeHost block
+  int32_t* noisy;  // (E, n_way, k_shot) 1 = noisy shot
+};
+
+__host__ __device__ inline size_t ep_host_ints(int E, int n_way, int n_cls) {
+  return (size_t)E * n_way + E + 2 * (size_t)n_cls;
+}
+
+__host__ __device__ inline EpisodeHost ep_host_view(int32_t* p, int E, int n_way, int n_cls) {
+  EpisodeHost h;
+  h.way = p;
+  h.n_noise = h.way + (size_t)E * n_way;
+  h.cls = h.n_noise + E;
+  h.pair = h.cls + n_cls;
+  return h;
+}
+
+void carve_episodes(WsBump& ws, int E, int n_way, int k_shot, int n_cls, EpisodeWs& w) {
+  w.host = ws.take<int32_t>(ep_host_ints(E, n_way, n_cls));
+  w.noisy = ws.take<int32_t>((size_t)E * n_way * k_shot);
+}
+
+__host__ __device__ inline uint32_t hkey(uint32_t a, uint32_t b) {
+  return lowbias32(a ^ lowbias32(b));
+}
+
+// One CTA per (episode, way): the way's clean shots and query blocks (the smallest keys of its
+// class's eligible list), the noise class and block of every noisy shot, and the keyed shuffle.
+__global__ __launch_bounds__(EP_T) void episode_select_kernel(
+    const int32_t* __restrict__ elig_off, const int32_t* __restrict__ elig_block,
+    const EpisodeArgs a, const int32_t* __restrict__ hbuf, int E, int32_t* __restrict__ noisy,
+    int32_t* __restrict__ shot_block, int32_t* __restrict__ support_flag,
+    int32_t* __restrict__ query_block) {
+  __shared__ uint64_t s_top[EP_WARPS][32];
+  __shared__ int32_t s_range[MAX_IDX_CLS], s_perm[MAX_IDX_CLS], s_ncls[MAX_SHOT],
+      s_nblk[MAX_SHOT], s_n_range;
+  __shared__ uint32_t s_okey[MAX_SHOT];
+  const EpisodeHost h = ep_host_view(const_cast<int32_t*>(hbuf), E, a.n_way, a.n_cls);
+  const int e = blockIdx.x / a.n_way, w = blockIdx.x % a.n_way;
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int n_noise = h.n_noise[e], k_clean = a.k_shot - n_noise;
+  const int c = h.way[e * a.n_way + w];
+  const uint32_t ke = hkey(a.seed_hash, (uint32_t)(a.first + (int64_t)e * a.step));
+  const uint32_t kw = hkey(ke, (uint32_t)w + 1u);
+
+  // clean shots and queries: the k_clean + n_queries smallest lowbias32(b ^ kw)
+  const int32_t l0 = elig_off[c], ln = elig_off[c + 1] - l0;
+  uint64_t top = TOP_EMPTY;
+  for (int32_t base = wid * 32; base < ln; base += EP_T) {
+    const int32_t q = base + lane;
+    const uint64_t v = q < ln ? ((uint64_t)lowbias32((uint32_t)elig_block[l0 + q] ^ kw) << 32) |
+                                    (uint32_t)elig_block[l0 + q]
+                              : TOP_EMPTY;
+    const uint64_t thr = __shfl_sync(0xffffffffu, top, 31);
+    for (unsigned m = __ballot_sync(0xffffffffu, v < thr); m; m &= m - 1)
+      top = top_insert(top, __shfl_sync(0xffffffffu, v, __ffs(m) - 1));
+  }
+  s_top[wid][lane] = top;
+
+  // noise range: ood = the index's classes with an eligible block that no way holds, ascending;
+  // sym = the other ways' classes in way order; pair = pair[c]
+  if (threadIdx.x == 0) {
+    int n = 0;
+    if (a.noise_type == NOISE_OOD) {
+      for (int k = 0; k < a.n_cls; ++k) {
+        bool used = elig_off[k + 1] == elig_off[k];
+        for (int v = 0; v < a.n_way; ++v) used |= h.way[e * a.n_way + v] == k;
+        if (!used) s_range[n++] = k;
+      }
+    } else if (a.noise_type == NOISE_SYM) {
+      for (int v = 0; v < a.n_way; ++v)
+        if (v != w) s_range[n++] = h.way[e * a.n_way + v];
+    } else if (a.noise_type == NOISE_PAIR) {
+      s_range[n++] = h.pair[c];
+    }
+    s_n_range = n;
+  }
+  __syncthreads();
+  const int nr = s_n_range;
+  const bool single_use = k_clean - 1 == 1 && (a.noise_type == NOISE_OOD || a.noise_type == NOISE_SYM);
+  if (single_use && threadIdx.x < nr) {  // pi: the range ranked by lowbias32(r ^ hkey(kw, 33))
+    const uint32_t kp = hkey(kw, 33u), mine = lowbias32((uint32_t)threadIdx.x ^ kp);
+    int rank = 0;
+    for (int r = 0; r < nr; ++r) rank += lowbias32((uint32_t)r ^ kp) < mine ? 1 : 0;
+    s_perm[rank] = threadIdx.x;
+  }
+  if (wid == 0) {
+    for (int o = 1; o < EP_WARPS; ++o) top_merge(s_top[0], s_top[o], s_top[0]);
+  }
+  __syncthreads();
+  if (threadIdx.x < n_noise) {
+    const int j = threadIdx.x;
+    s_ncls[j] = single_use ? s_range[s_perm[min(j, nr - 1)]]
+                           : s_range[((uint64_t)hkey(kw, 64u + j) * (uint32_t)nr) >> 32];
+  }
+  __syncthreads();
+  // noisy shot j: the smallest lowbias32(b ^ hkey(kw, 128 + j)) of its class's eligible list
+  for (int j = wid; j < n_noise; j += EP_WARPS) {
+    const int32_t o = elig_off[s_ncls[j]], n = elig_off[s_ncls[j] + 1] - o;
+    const uint32_t kj = hkey(kw, 128u + j);
+    uint64_t best = TOP_EMPTY;
+    for (int32_t q = lane; q < n; q += 32) {
+      const uint32_t b = (uint32_t)elig_block[o + q];
+      const uint64_t v = ((uint64_t)lowbias32(b ^ kj) << 32) | b;
+      best = v < best ? v : best;
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) {
+      const uint64_t u = __shfl_xor_sync(0xffffffffu, best, d);
+      best = u < best ? u : best;
+    }
+    if (lane == 0) s_nblk[j] = (int32_t)(uint32_t)best;
+  }
+  const uint32_t ks = hkey(kw, 34u);
+  if (threadIdx.x < a.k_shot) s_okey[threadIdx.x] = lowbias32((uint32_t)threadIdx.x ^ ks);
+  __syncthreads();
+  // shot t before the shuffle: clean shot t (t < k_clean) or noisy shot t - k_clean; it goes to
+  // the slot of its rank under lowbias32(t ^ hkey(kw, 34))
+  const int64_t ew = (int64_t)e * a.n_way + w;
+  if (threadIdx.x < a.k_shot) {
+    const int t = threadIdx.x;
+    int slot = 0;
+    for (int u = 0; u < a.k_shot; ++u) slot += s_okey[u] < s_okey[t] ? 1 : 0;
+    const bool nz = t >= k_clean;
+    const int32_t b = nz ? s_nblk[t - k_clean] : (int32_t)(uint32_t)s_top[0][t];
+    const int32_t k = nz ? s_ncls[t - k_clean] : c;
+    shot_block[ew * a.k_shot + slot] = b;
+    support_flag[ew * a.k_shot + slot] = h.cls[k];
+    noisy[ew * a.k_shot + slot] = nz ? 1 : 0;
+  }
+  if (threadIdx.x < a.n_queries)
+    query_block[ew * a.n_queries + threadIdx.x] = (int32_t)(uint32_t)s_top[0][k_clean + threadIdx.x];
+}
+
+// One CTA per cloud: the support shots of every (episode, way), then the query clouds.  Slot s of
+// a block's cloud holds member rank s mod min(n_b, N), normalised as a chunk cloud.
+__global__ __launch_bounds__(256) void episode_cloud_kernel(
+    const float* __restrict__ pts, int64_t s_m, int64_t s_c, int N,
+    const int32_t* __restrict__ labels, const int64_t* __restrict__ block_off,
+    const int32_t* __restrict__ member, const EpisodeArgs a, const int32_t* __restrict__ hbuf,
+    int E, const int32_t* __restrict__ noisy, const int32_t* __restrict__ shot_block,
+    const int32_t* __restrict__ support_flag, const int32_t* __restrict__ query_block,
+    float* __restrict__ support_x, int32_t* __restrict__ support_y,
+    int32_t* __restrict__ gt_support_y, int32_t* __restrict__ support_src,
+    float* __restrict__ query_x, int64_t* __restrict__ query_y, int32_t* __restrict__ query_src) {
+  const int64_t g = blockIdx.x, n_shots = (int64_t)E * a.n_way * a.k_shot;
+  const bool shot = g < n_shots;
+  const int64_t i = shot ? g : g - n_shots;
+  const int32_t b = shot ? shot_block[i] : query_block[i];
+  const int64_t m0 = block_off[b];
+  const int32_t nb = (int32_t)(block_off[b + 1] - m0);
+  float* out = (shot ? support_x : query_x) + i * N * 9;
+  int32_t* src = (shot ? support_src : query_src) + i * N;
+  scene_cloud(pts, s_m, s_c, N, IndexMembers{member, m0}, min(nb, N), out, src);
+  if (shot) {
+    const int32_t cls = support_flag[i], nz = noisy[i];
+    for (int q = threadIdx.x; q < N; q += blockDim.x) {
+      const int32_t y = labels[src[q]] == cls ? 1 : 0;
+      support_y[i * N + q] = y;
+      gt_support_y[i * N + q] = nz ? 0 : y;
+    }
+  } else {
+    const EpisodeHost h = ep_host_view(const_cast<int32_t*>(hbuf), E, a.n_way, a.n_cls);
+    const int64_t e = i / ((int64_t)a.n_way * a.n_queries);
+    int32_t wc[MAX_WAY];
+#pragma unroll
+    for (int v = 0; v < MAX_WAY; ++v) wc[v] = v < a.n_way ? h.cls[h.way[e * a.n_way + v]] : 0;
+    for (int q = threadIdx.x; q < N; q += blockDim.x) {
+      const int32_t l = labels[src[q]];
+      int64_t y = 0;
+#pragma unroll
+      for (int v = MAX_WAY - 1; v >= 0; --v)
+        if (v < a.n_way && l == wc[v]) y = v + 1;
+      query_y[i * N + q] = y;
+    }
+  }
 }
 
 int scene_common_checks(int64_t M, int overlap, int n_points) {
@@ -918,6 +1226,194 @@ int r3dfs_scene_support(const float* points, int64_t M, int64_t s_m, int64_t s_c
   scene_support_cloud_kernel<<<n_way * k_shot, 256, 0, st>>>(
       points, s_m, s_c, n_points, labels, sel, k_shot, p.vals[0], p.mem_point, p.seg_start,
       w.shot_seg, support_x, support_y, support_src);
+  R3DFS_CHECK_LAUNCH();
+  return 0;
+}
+
+int r3dfs_scene_index(const int32_t* labels, int64_t M, int overlap, const int32_t* h_classes,
+                      int n_cls, int32_t scan, int64_t point_base, int64_t n_blocks,
+                      int64_t n_members, int64_t block_cap, int64_t member_cap, int64_t* block_off,
+                      int32_t* block_scan, int32_t* block_id, int32_t* member, int32_t* count,
+                      int64_t* h_sizes, const void* plan_ws, size_t plan_ws_bytes,
+                      r3dfs_stream_t stream) {
+  if (!labels || !h_classes || !block_off || !block_scan || !block_id || !member || !count ||
+      !h_sizes || !plan_ws || scan < 0 || point_base < 0 || n_blocks < 0 || n_members < 0)
+    return R3DFS_E_BADARG;
+  R3DFS_TRY(scene_common_checks(M, overlap, 64));
+  if (n_cls < 1 || n_cls > MAX_IDX_CLS) return R3DFS_E_UNSUPPORTED;
+  if (point_base + M > INT32_MAX) return R3DFS_E_UNSUPPORTED;
+  IndexCls cls{};
+  cls.n = n_cls;
+  for (int k = 0; k < n_cls; ++k) {
+    for (int v = 0; v < k; ++v)
+      if (h_classes[v] == h_classes[k]) return R3DFS_E_BADARG;
+    cls.at[k] = k;
+  }
+  std::sort(cls.at, cls.at + n_cls, [&](int32_t x, int32_t y) { return h_classes[x] < h_classes[y]; });
+  for (int k = 0; k < n_cls; ++k) cls.id[k] = h_classes[cls.at[k]];
+  if (plan_ws_bytes < r3dfs_scene_workspace(M, overlap)) return R3DFS_E_WORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  WsBump pws(const_cast<void*>(plan_ws), plan_ws_bytes);
+  SceneWs p;
+  carve_scene(pws, M, overlap, p);
+  // the one host synchronisation per scan: the plan's block and membership counts
+  SceneHdr hdr;
+  cudaError_t e = cudaMemcpyAsync(&hdr, p.hdr, sizeof(hdr), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return (int)e;
+  if (hdr.err) {
+    h_sizes[0] = h_sizes[1] = -1;
+    return R3DFS_E_BADARG;
+  }
+  h_sizes[0] = hdr.n_seg;
+  h_sizes[1] = hdr.T;
+  if (n_members + hdr.T >= ((int64_t)1 << 31)) return R3DFS_E_UNSUPPORTED;
+  if (n_blocks + hdr.n_seg > block_cap || n_members + hdr.T > member_cap) return R3DFS_E_WORKSPACE;
+  index_blocks_kernel<<<nblk(hdr.n_seg + 1), 256, 0, st>>>(p.hdr, p.keys[0], p.seg_start, scan,
+                                                           n_blocks, n_members, block_off,
+                                                           block_scan, block_id);
+  R3DFS_CHECK_LAUNCH();
+  if (hdr.T > 0) {
+    index_members_kernel<<<nblk(hdr.T), 256, 0, st>>>(hdr.T, p.vals[0], p.mem_point, n_members,
+                                                      (int32_t)point_base, member);
+    R3DFS_CHECK_LAUNCH();
+  }
+  if (hdr.n_seg > 0) {
+    index_count_kernel<<<nblk(hdr.n_seg, IDX_WARPS), IDX_T, 0, st>>>(
+        p.hdr, p.vals[0], p.mem_point, p.seg_start, labels, cls, n_blocks, count);
+    R3DFS_CHECK_LAUNCH();
+  }
+  return 0;
+}
+
+size_t r3dfs_scene_index_workspace(int64_t n_blocks, int n_cls) {
+  if (n_blocks < 1 || n_cls < 1 || n_cls > MAX_IDX_CLS ||
+      n_blocks * n_cls >= ((int64_t)1 << 31) - 1)
+    return 0;
+  const int64_t n = n_blocks * n_cls + 1;
+  WsBump ws(nullptr, 0);
+  ws.take<int32_t>(n);
+  ws.take<int32_t>(scan_tiles(n) + 1);
+  ws.take<int32_t>(1);
+  return align_up(ws.off, 256);
+}
+
+int r3dfs_scene_index_classes(const int64_t* block_off, const int32_t* count, int64_t n_blocks,
+                              int n_cls, int min_points, double min_ratio, int32_t* elig_off,
+                              int32_t* elig_block, int32_t* h_elig_off, void* wsp, size_t ws_bytes,
+                              r3dfs_stream_t stream) {
+  if (!block_off || !count || !elig_off || !elig_block || !h_elig_off || !wsp)
+    return R3DFS_E_BADARG;
+  if (min_points < 0 || !(min_ratio >= 0.0 && min_ratio <= 1.0)) return R3DFS_E_BADARG;
+  const size_t need = r3dfs_scene_index_workspace(n_blocks, n_cls);
+  if (need == 0) return n_blocks < 1 ? R3DFS_E_BADARG : R3DFS_E_UNSUPPORTED;
+  if (ws_bytes < need) return R3DFS_E_WORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t n = n_blocks * n_cls + 1;
+  WsBump ws(wsp, ws_bytes);
+  int32_t* pos = ws.take<int32_t>(n);
+  int32_t* bsum = ws.take<int32_t>(scan_tiles(n) + 1);
+  int32_t* total = ws.take<int32_t>(1);
+  index_flag_kernel<<<nblk(n), 256, 0, st>>>(block_off, count, n_blocks, n_cls, min_points,
+                                             min_ratio, pos);
+  R3DFS_CHECK_LAUNCH();
+  R3DFS_TRY(scan_excl(pos, n, bsum, total, st));
+  index_lists_kernel<<<nblk(n), 256, 0, st>>>(pos, n_blocks, n_cls, elig_off, elig_block);
+  R3DFS_CHECK_LAUNCH();
+  cudaError_t e = cudaMemcpyAsync(h_elig_off, elig_off, sizeof(int32_t) * (n_cls + 1),
+                                  cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  return e == cudaSuccess ? 0 : (int)e;
+}
+
+size_t r3dfs_scene_episodes_workspace(int n_episodes, int n_way, int k_shot, int n_queries,
+                                      int n_cls) {
+  if (n_episodes < 1 || n_way < 1 || n_way > MAX_WAY || k_shot < 1 || k_shot > MAX_SHOT ||
+      n_queries < 1 || n_queries > MAX_SHOT || n_cls < 1 || n_cls > MAX_IDX_CLS ||
+      (int64_t)n_episodes * n_way * n_queries > 65535)
+    return 0;
+  WsBump ws(nullptr, 0);
+  EpisodeWs w;
+  carve_episodes(ws, n_episodes, n_way, k_shot, n_cls, w);
+  return align_up(ws.off, 256);
+}
+
+int r3dfs_scene_episodes(const float* points, int64_t s_m, int64_t s_c, const int32_t* labels,
+                         const int64_t* block_off, const int32_t* member, const int32_t* elig_off,
+                         const int32_t* elig_block, const int32_t* h_elig_off,
+                         const int32_t* h_classes, int n_cls, const int32_t* h_way_class,
+                         const int32_t* h_n_noise, int noise_type, const int32_t* h_pair,
+                         int n_episodes, int n_way, int k_shot, int n_queries, int n_points,
+                         uint32_t seed, int64_t first, int64_t step, float* support_x,
+                         int32_t* support_y, int32_t* gt_support_y, int32_t* support_flag,
+                         float* query_x, int64_t* query_y, int32_t* shot_block,
+                         int32_t* query_block, int32_t* support_src, int32_t* query_src,
+                         void* wsp, size_t ws_bytes, r3dfs_stream_t stream) {
+  if (!points || !labels || !block_off || !member || !elig_off || !elig_block || !h_elig_off ||
+      !h_classes || !h_way_class || !h_n_noise || !support_x || !support_y || !gt_support_y ||
+      !support_flag || !query_x || !query_y || !shot_block || !query_block || !support_src ||
+      !query_src || !wsp)
+    return R3DFS_E_BADARG;
+  const size_t need = r3dfs_scene_episodes_workspace(n_episodes, n_way, k_shot, n_queries, n_cls);
+  if (need == 0 || n_points < 64 || n_points > 65536) return R3DFS_E_UNSUPPORTED;
+  if (noise_type < NOISE_NONE || noise_type > NOISE_PAIR || (noise_type == NOISE_PAIR && !h_pair))
+    return R3DFS_E_BADARG;
+  if (first < 0 || step < 1 || first + (int64_t)(n_episodes - 1) * step > (int64_t)UINT32_MAX)
+    return R3DFS_E_BADARG;
+  const int E = n_episodes;
+  std::vector<int32_t> hb(ep_host_ints(E, n_way, n_cls));
+  EpisodeHost h = ep_host_view(hb.data(), E, n_way, n_cls);
+  auto index_of = [&](int32_t id) {
+    for (int k = 0; k < n_cls; ++k)
+      if (h_classes[k] == id) return k;
+    return -1;
+  };
+  auto n_elig = [&](int k) { return h_elig_off[k + 1] - h_elig_off[k]; };
+  for (int k = 0; k < n_cls; ++k) {
+    if (index_of(h_classes[k]) != k) return R3DFS_E_BADARG;  // duplicate class id
+    h.cls[k] = h_classes[k];
+    h.pair[k] = k;
+    if (noise_type == NOISE_PAIR && (h.pair[k] = index_of(h_pair[k])) < 0) return R3DFS_E_BADARG;
+  }
+  for (int e = 0; e < E; ++e) {
+    const int nn = h_n_noise[e];
+    if (nn < 0 || nn > k_shot || (noise_type == NOISE_NONE && nn > 0)) return R3DFS_E_BADARG;
+    if (k_shot - nn + n_queries > MAX_SHOT) return R3DFS_E_UNSUPPORTED;
+    h.n_noise[e] = nn;
+    int n_ood = 0;
+    int32_t* way = h.way + (size_t)e * n_way;
+    for (int w = 0; w < n_way; ++w) {
+      way[w] = index_of(h_way_class[(size_t)e * n_way + w]);
+      if (way[w] < 0 || n_elig(way[w]) < k_shot - nn + n_queries) return R3DFS_E_BADARG;
+      for (int v = 0; v < w; ++v)
+        if (way[v] == way[w]) return R3DFS_E_BADARG;
+    }
+    for (int k = 0; k < n_cls; ++k)
+      n_ood += n_elig(k) > 0 && std::find(way, way + n_way, k) == way + n_way ? 1 : 0;
+    if (nn == 0) continue;
+    if ((noise_type == NOISE_OOD && n_ood == 0) || (noise_type == NOISE_SYM && n_way < 2))
+      return R3DFS_E_BADARG;
+    if (noise_type == NOISE_PAIR)
+      for (int w = 0; w < n_way; ++w)
+        if (n_elig(h.pair[way[w]]) < 1) return R3DFS_E_BADARG;
+  }
+  if (ws_bytes < need) return R3DFS_E_WORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  WsBump ws(wsp, ws_bytes);
+  EpisodeWs w;
+  carve_episodes(ws, E, n_way, k_shot, n_cls, w);
+  cudaError_t ce = cudaMemcpyAsync(w.host, hb.data(), sizeof(int32_t) * hb.size(),
+                                   cudaMemcpyHostToDevice, st);
+  if (ce != cudaSuccess) return (int)ce;
+  const EpisodeArgs a{lowbias32(seed), first, step, n_way, k_shot, n_queries, n_cls, noise_type};
+  episode_select_kernel<<<E * n_way, EP_T, 0, st>>>(elig_off, elig_block, a, w.host, E, w.noisy,
+                                                    shot_block, support_flag, query_block);
+  R3DFS_CHECK_LAUNCH();
+  const int64_t n_clouds = (int64_t)E * n_way * (k_shot + n_queries);
+  episode_cloud_kernel<<<(unsigned)n_clouds, 256, 0, st>>>(
+      points, s_m, s_c, n_points, labels, block_off, member, a, w.host, E, w.noisy, shot_block,
+      support_flag, query_block, support_x, support_y, gt_support_y, support_src, query_x, query_y,
+      query_src);
   R3DFS_CHECK_LAUNCH();
   return 0;
 }

@@ -266,6 +266,63 @@ class EpisodeEvaluator:
             logger.cprint("mean IoU: %f\n" % res["mean_iou"])
         return res
 
+    def run_scenes(self, ds, way_classes, k_shot: int, n_queries: int = 1,
+                   noise_type: Optional[str] = None, noise_ratio=0.0, rank: int = 0,
+                   world: int = 1, pair_dict=None, first: int = 0, logger=None,
+                   log_every: int = 50) -> Dict[str, object]:
+        """`run` over episodes sampled on the device from a `SceneEpisodes` dataset: episode i has
+        way classes way_classes[i] (e.g. ds.test_classes(n_way)) and index first + i, and belongs
+        to rank i % world.  Each batch of this rank's episodes is sampled, run through
+        forward_episodes and counted without leaving the device; the run ends with the same
+        all-reduce as `run` and returns the same dict."""
+        from . import _lib, ops
+        wc = np.asarray(way_classes, dtype=np.int64)
+        if wc.ndim == 1:
+            wc = wc[None]
+        mine = shard_indices(len(wc), rank, world)
+        n_slots = len(self.test_classes) + 1
+        dev = self.device
+        counters = torch.zeros((3, n_slots), dtype=torch.int64, device=dev)
+        loss_sum = torch.zeros((), dtype=torch.float64, device=dev)
+        cg_bad = torch.zeros((), dtype=torch.float64, device=dev)
+        slots = torch.tensor([class_slots(wc[i], self.test_classes) for i in mine],
+                             dtype=torch.int32).reshape(len(mine), wc.shape[1]).to(dev)
+        ws, done = None, 0
+        for s in range(0, len(mine), self.batch):
+            idx = mine[s:s + self.batch]
+            b = ds.sample(wc[idx], k_shot, n_queries, first=first + idx[0], noise_type=noise_type,
+                          noise_ratio=noise_ratio, pair_dict=pair_dict, step=world)
+            if ws is None:
+                cfg = self.model._cfg(int(b["query_x"].shape[1]), mdns=bool(self.eval_mdns))
+                ws = torch.empty(_lib.lib().r3dfs_mpti_workspace(cfg, self.batch),
+                                 dtype=torch.uint8, device=dev)
+            out = self.model.forward_episodes(b["support_x"], b["support_y"], b["query_x"],
+                                              b["query_y"], eval=self.eval_mdns, workspace=ws,
+                                              want_diag=True)
+            ops.confusion_accumulate(out["pred"], b["query_y"], slots[s:s + len(idx)], counters)
+            loss_sum += out["loss"].double().sum()
+            cg_bad += (out["diag"]["cg_iters"] >= int(self.model.cg_max_iter)).sum().double()
+            if logger is not None and (done + len(idx)) // log_every > done // log_every:
+                from datetime import datetime
+                logger.cprint("[Eval] Iter: %d | Loss: %.4f | %s" % (
+                    done + len(idx), float(out["loss"][-1]), str(datetime.now())))
+            done += len(idx)
+        n = torch.tensor(float(done), dtype=torch.float64, device=dev)
+        all_reduce_eval_state(counters, loss_sum, n)
+        res = iou_from_counters(counters)
+        res.update(counters=counters.cpu(), mean_loss=float(loss_sum / n), n_episodes=int(n),
+                   cg_not_converged=int(cg_bad))
+        if res["cg_not_converged"]:
+            import warnings
+            warnings.warn("%d label-propagation solve(s) on this rank stopped at cg_max_iter=%d "
+                          "before reaching cg_tol=%g" % (res["cg_not_converged"],
+                                                         self.model.cg_max_iter, self.model.cg_tol))
+        if logger is not None and rank == 0:
+            for c in range(n_slots):
+                logger.cprint("class %d: iou %f" % (c, res["iou"][c]))
+            logger.cprint("mean IoU: %f\n" % res["mean_iou"])
+        return res
+
 
 class _EpisodeList:
     """Adapter: Episode-like objects (support_x, support_y, query_x, query_y, sampled_classes) as an

@@ -723,6 +723,152 @@ def scene_support(plan: ScenePlan, labels: torch.Tensor, classes: Sequence[int],
     return out
 
 
+@dataclass
+class SceneIndex:
+    """A dataset of labelled scans indexed by r3dfs_scene_index: the global block table
+    (block_off (n_blocks+1) int64, block_scan / block_id (n_blocks) int32), every block's members
+    as global points in rank order (member int32), class counts (count (n_blocks, n_cls) int32) and
+    the eligible blocks of every class in ascending order (elig_block from elig_off[k] to
+    elig_off[k+1], the reference's class2scans).  h_elig_off is the host copy of elig_off."""
+    classes: List[int]
+    block_off: torch.Tensor
+    block_scan: torch.Tensor
+    block_id: torch.Tensor
+    member: torch.Tensor
+    count: torch.Tensor
+    elig_off: torch.Tensor
+    elig_block: torch.Tensor
+    h_elig_off: List[int]
+
+    @property
+    def n_blocks(self) -> int:
+        return int(self.block_scan.shape[0])
+
+
+def _grown(t: torch.Tensor, used: int, need: int) -> torch.Tensor:
+    if t.shape[0] >= need:
+        return t
+    g = torch.empty((max(need, 2 * t.shape[0]),) + tuple(t.shape[1:]), dtype=t.dtype,
+                    device=t.device)
+    g[:used] = t[:used]
+    return g
+
+
+def scene_index(plans: Sequence[ScenePlan], labels: Sequence[torch.Tensor], point_base: Sequence[int],
+                classes: Sequence[int], min_points: int = 100,
+                min_ratio: float = 0.05) -> SceneIndex:
+    """Dataset index over planned scans (r3dfs_scene_index per scan, then
+    r3dfs_scene_index_classes).  plans[i] was made by scene_plan on scan i's slice of the dataset's
+    points, which starts at point point_base[i]; labels[i] is that scan's (M_i,) int32 labels.
+    Reads back each scan's sizes and the class lists' offsets (one synchronisation each)."""
+    dev = _need_cuda(*labels)
+    n_cls = len(classes)
+    h_cls = (C.c_int32 * n_cls)(*[int(c) for c in classes])
+    L = _lib.lib()
+    n_blocks = n_members = 0
+    cap_m = sum(int(p.points.shape[0]) for p in plans)
+    off = torch.empty((1025,), dtype=torch.int64, device=dev)
+    bscan = torch.empty((1024,), dtype=torch.int32, device=dev)
+    bid = torch.empty((1024,), dtype=torch.int32, device=dev)
+    count = torch.empty((1024, n_cls), dtype=torch.int32, device=dev)
+    member = torch.empty((cap_m,), dtype=torch.int32, device=dev)
+    sizes = (C.c_int64 * 2)()
+    for i, (plan, lab) in enumerate(zip(plans, labels)):
+        M = int(plan.points.shape[0])
+        while True:
+            sizes[0] = sizes[1] = -2
+            with torch.cuda.device(dev):
+                rc = L.r3dfs_scene_index(
+                    _p(lab), M, plan.overlap, h_cls, n_cls, i, int(point_base[i]), n_blocks,
+                    n_members, bscan.shape[0], member.shape[0], _p(off), _p(bscan), _p(bid),
+                    _p(member), _p(count), sizes, _p(plan.workspace), plan.workspace.numel(),
+                    _stream())
+            if rc != -3 or sizes[0] < 0:
+                break
+            nb = n_blocks + int(sizes[0])
+            off = _grown(off, n_blocks + 1, nb + 1)
+            bscan, bid, count = (_grown(t, n_blocks, nb) for t in (bscan, bid, count))
+            member = _grown(member, n_members, n_members + int(sizes[1]))
+        if rc == -1 and sizes[0] == -1:
+            raise ValueError(f"scan {i} holds a non-finite x or y coordinate, or spans 2^31 blocks "
+                             "or more")
+        check(rc, "r3dfs_scene_index")
+        n_blocks += int(sizes[0])
+        n_members += int(sizes[1])
+    if n_blocks == 0:
+        raise ValueError("the scans hold no blocks")
+    count = count[:n_blocks]
+    need = L.r3dfs_scene_index_workspace(n_blocks, n_cls)
+    if need == 0:
+        raise _lib.R3dfsError(f"{n_blocks} blocks x {n_cls} classes is outside what libr3dfs is "
+                              "built for: 1..64 classes and n_blocks * n_classes < 2^31 - 1")
+    ws = _ws(need, dev)
+    elig_off = torch.empty((n_cls + 1,), dtype=torch.int32, device=dev)
+    elig_block = torch.empty((n_blocks * n_cls,), dtype=torch.int32, device=dev)
+    h_off = (C.c_int32 * (n_cls + 1))()
+    with torch.cuda.device(dev):
+        check(L.r3dfs_scene_index_classes(_p(off), _p(count), n_blocks, n_cls, int(min_points),
+                                          float(min_ratio), _p(elig_off), _p(elig_block), h_off,
+                                          _p(ws), ws.numel(), _stream()),
+              "r3dfs_scene_index_classes")
+    h_off = list(h_off)
+    return SceneIndex([int(c) for c in classes], off[:n_blocks + 1], bscan[:n_blocks],
+                      bid[:n_blocks], member[:n_members], count, elig_off,
+                      elig_block[:h_off[-1]], h_off)
+
+
+NOISE_CODES = {None: 0, "ood": 1, "sym": 2, "pair": 3}
+
+
+def scene_episodes(index: SceneIndex, points: torch.Tensor, labels: torch.Tensor, way_classes,
+                   n_noise: Sequence[int], noise_type: Optional[str], pair: Optional[Sequence[int]],
+                   k_shot: int, n_queries: int, n_points: int, seed: int = 0, first: int = 0,
+                   step: int = 1):
+    """E episodes sampled from a dataset index (r3dfs_scene_episodes): episode e has index
+    first + e * step.  points (M, 6) and labels (M,) int32 are the dataset's; way_classes (E, n_way)
+    class ids; n_noise (E) noisy shots per way; pair (n_cls) = pair[c] for the index's classes in
+    order (pair noise only).  Enqueued only.  Returns dict(support_x (E, n_way, k_shot, N, 9),
+    support_y / gt_support_y / support_src (E, n_way, k_shot, N) int32, support_flag / shot_block
+    (E, n_way, k_shot) int32, query_x (E, n_way*n_queries, N, 9), query_y int64 / query_src int32
+    (E, n_way*n_queries, N), query_block (E, n_way*n_queries) int32)."""
+    dev = _need_cuda(points, labels)
+    E, n_way = len(way_classes), len(way_classes[0])
+    n_cls, N = len(index.classes), int(n_points)
+    L = _lib.lib()
+    need = L.r3dfs_scene_episodes_workspace(E, n_way, int(k_shot), int(n_queries), n_cls)
+    if need == 0:
+        raise _lib.R3dfsError(f"{E} episodes of {n_way} ways x {k_shot} shots x {n_queries} "
+                              "queries is outside what libr3dfs is built for: 1..7 ways, 1..32 "
+                              "shots, E * n_way * n_queries <= 65535")
+    ws = _ws(need, dev)
+    nq = n_way * int(n_queries)
+    i32 = dict(dtype=torch.int32, device=dev)
+    out = {"support_x": torch.empty((E, n_way, k_shot, N, 9), dtype=torch.float32, device=dev),
+           "support_y": torch.empty((E, n_way, k_shot, N), **i32),
+           "gt_support_y": torch.empty((E, n_way, k_shot, N), **i32),
+           "support_flag": torch.empty((E, n_way, k_shot), **i32),
+           "query_x": torch.empty((E, nq, N, 9), dtype=torch.float32, device=dev),
+           "query_y": torch.empty((E, nq, N), dtype=torch.int64, device=dev),
+           "shot_block": torch.empty((E, n_way, k_shot), **i32),
+           "query_block": torch.empty((E, nq), **i32),
+           "support_src": torch.empty((E, n_way, k_shot, N), **i32),
+           "query_src": torch.empty((E, nq, N), **i32)}
+    ints = lambda v: (C.c_int32 * max(1, len(v)))(*[int(x) for x in v])  # noqa: E731
+    h_way = ints([c for row in way_classes for c in row])
+    h_pair = None if pair is None else ints(pair)
+    with torch.cuda.device(dev):
+        check(L.r3dfs_scene_episodes(
+            _p(points), points.stride(0), points.stride(1), _p(labels), _p(index.block_off),
+            _p(index.member), _p(index.elig_off), _p(index.elig_block), ints(index.h_elig_off),
+            ints(index.classes), n_cls, h_way, ints(n_noise), NOISE_CODES[noise_type], h_pair, E,
+            n_way, int(k_shot), int(n_queries), N, int(seed), int(first), int(step),
+            *(_p(out[k]) for k in ("support_x", "support_y", "gt_support_y", "support_flag",
+                                   "query_x", "query_y", "shot_block", "query_block",
+                                   "support_src", "query_src")),
+            _p(ws), ws.numel(), _stream()), "r3dfs_scene_episodes")
+    return out
+
+
 def confusion_accumulate(pred: torch.Tensor, gt: torch.Tensor, class_slot: torch.Tensor,
                          counters: torch.Tensor) -> None:
     """evaluate_metric counters (eval_noise.py:35-62), accumulated in place into the (3, n_slots)
