@@ -9,7 +9,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # R3DFS_LIB selects another build of the SAME library (the measurement build libr3dfs_ab.so, which
-# has the A/B switches of DESIGN.md §3.1 compiled in); it is read here, never by the library.
+# has the A/B switches of DESIGN.md §6 compiled in); it is read here, never by the library.
 LIB_PATH = os.environ.get("R3DFS_LIB") or os.path.join(_HERE, "libr3dfs.so")
 AB_LIB_PATH = os.path.join(_HERE, "libr3dfs_ab.so")
 

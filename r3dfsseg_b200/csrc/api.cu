@@ -91,44 +91,19 @@ __global__ void i32_to_i64_kernel(const int32_t* __restrict__ a, int64_t* __rest
 
 thread_local long long r3dfs_launches = 0;
 
-bool simt_gemm_forced() {
-  static const bool v = [] {
-    const char* e = R3DFS_GETENV("R3DFS_SIMT_GEMM");
-    return e && e[0] == '1';
-  }();
-  return v;
-}
-
 int launch_knn_auto(const float* x, int ld, int C, const float* xx, int64_t B, int N, int k,
                     int32_t* idx32, int64_t* idx64, int impl, cudaStream_t st, void* split_ws,
                     size_t split_bytes) {
   if (impl == 2)
     return launch_knn_tc(x, ld, C, xx, B, N, k, idx32, idx64, st, split_ws, split_bytes);
-  if (impl == 0 && !simt_gemm_forced() && C <= 64)
+  if (impl == 0 && C <= 64)
     return launch_knn_tc(x, ld, C, xx, B, N, k, idx32, idx64, st, split_ws, split_bytes);
   return launch_knn(x, ld, C, xx, B, N, k, idx32, idx64, st);
-}
-
-int launch_edge_mlp_auto(const float* PQ, const int32_t* idx, const float* w2, const float* s2,
-                         const float* t2, int64_t B, int N, int k, float* Y, int ldy, RowMap map,
-                         cudaStream_t st) {
-  if (simt_gemm_forced())
-    return launch_edge_mlp(PQ, idx, w2, s2, t2, B, N, k, Y, ldy, map, nullptr, st);
-  return launch_edge_mlp_tc(PQ, idx, w2, s2, t2, B, N, k, Y, ldy, map, st);
-}
-
-int launch_attention_auto(const float* qkv, int ld, int64_t B, int N, float* Y, int ldy,
-                          RowMap map, cudaStream_t st, float* kmax_ws, void* split_ws,
-                          size_t split_bytes) {
-  if (simt_gemm_forced()) return launch_attention(qkv, ld, B, N, Y, ldy, map, st);
-  return launch_attention_tc(qkv, ld, B, N, Y, ldy, map, st, kmax_ws, split_ws, split_bytes);
 }
 
 int launch_linear_auto(const float* X, int ldx, const float* W, const float* s, const float* t,
                        int act, int64_t M, int K, int Nout, float* Y, int ldy, RowMap map,
                        cudaStream_t st) {
-  if (simt_gemm_forced())
-    return launch_linear(X, ldx, W, s, t, act, M, K, Nout, Y, ldy, map, st);
   // TMA-fed kernel when the operands meet TMA's alignment rules, register-fed kernel otherwise
   const int rc = launch_linear_tma(X, ldx, W, s, t, act, M, K, Nout, Y, ldy, map, st);
   if (rc != R3DFS_E_UNSUPPORTED) return rc;
@@ -188,8 +163,8 @@ int encoder_forward(const r3dfs_weights_t* w, const float* xp, int64_t B, int N,
     R3DFS_TRY(launch_linear_auto(in, ld, e.wpq, e.spq, e.tpq, ACT_NONE, M, C, 128, e.PQ, 128,
                             identity_map(), st));
     if (sr) sr->mark(R3DFS_ST_PQ0 + 3 * i, st);
-    R3DFS_TRY(launch_edge_mlp_auto(e.PQ, e.idx, w->ec_w2[i], w->ec_s2[i], w->ec_t2[i], B, N, k,
-                                   e.ecat + 64 * i, 192, identity_map(), st));
+    R3DFS_TRY(launch_edge_mlp_tc(e.PQ, e.idx, w->ec_w2[i], w->ec_s2[i], w->ec_t2[i], B, N, k,
+                                 e.ecat + 64 * i, 192, identity_map(), st));
     if (sr) sr->mark(R3DFS_ST_EDGE0 + 3 * i, st);
   }
   // level-1 feature = first EdgeConv output (models/dgcnn.py:127, models/mpti.py:586-589)
@@ -214,8 +189,8 @@ int encoder_forward(const r3dfs_weights_t* w, const float* xp, int64_t B, int N,
                           192, identity_map(), st));
   if (sr) sr->mark(R3DFS_ST_QKV, st);
   // xx: free scratch for the key-norm maxima; h512 (idle after the MLP) holds the pre-split K / V^T
-  R3DFS_TRY(launch_attention_auto(e.qkv, 192, B, N, F + 64, 192, map, st, e.xx, e.h512,
-                                  sizeof(float) * (size_t)M * 512));
+  R3DFS_TRY(launch_attention_tc(e.qkv, 192, B, N, F + 64, 192, map, st, e.xx, e.h512,
+                                sizeof(float) * (size_t)M * 512));
   if (sr) sr->mark(R3DFS_ST_ATT, st);
   return 0;
 }
@@ -352,7 +327,7 @@ int r3dfs_edgeconv(const float* x, int64_t B, int64_t C, int64_t N, int64_t sb, 
   R3DFS_TRY(launch_fold_edge_w1(w1, s1, t1, (int)C, wpq, spq, tpq, st));
   R3DFS_TRY(launch_linear_auto(xp, (int)C, wpq, spq, tpq, ACT_NONE, M, (int)C, 128, PQ, 128,
                                identity_map(), st));
-  return launch_edge_mlp_auto(PQ, idx, w2, s2, t2, B, (int)N, k, y, 64, identity_map(), st);
+  return launch_edge_mlp_tc(PQ, idx, w2, s2, t2, B, (int)N, k, y, 64, identity_map(), st);
 }
 
 // ---- attention ----------------------------------------------------------------------------------
@@ -375,8 +350,8 @@ int r3dfs_attention(const float* x, int64_t B, int64_t N, int64_t Cin, const flo
   if (!ws.ok()) return R3DFS_E_WORKSPACE;
   R3DFS_TRY(launch_linear_auto(x, (int)Cin, wqkv, nullptr, nullptr, ACT_NONE, B * N, (int)Cin, 192,
                                qkv, 192, identity_map(), st));
-  return launch_attention_auto(qkv, 192, B, (int)N, y, 64, identity_map(), st, kmax, split,
-                               split_bytes);
+  return launch_attention_tc(qkv, 192, B, (int)N, y, 64, identity_map(), st, kmax, split,
+                             split_bytes);
 }
 
 // ---- getFeatures --------------------------------------------------------------------------------

@@ -11,7 +11,7 @@
 
 extern thread_local long long r3dfs_launches;  // diagnostic: kernels launched by this thread
 
-// A/B switches (alternative kernels kept for re-measuring the claims of DESIGN.md §3.1) exist only
+// A/B switches (predecessor kernels that tests pin the current ones to, DESIGN.md §6) exist only
 // in the measurement build `libr3dfs_ab.so` (make ab: -DR3DFS_AB_SWITCHES); the shipped library
 // reads no environment variable and keeps no configuration state.
 #ifdef R3DFS_AB_SWITCHES
@@ -116,7 +116,7 @@ int launch_knn_tc(const float* x, int ld, int C, const float* xx, int64_t B, int
                   size_t split_bytes = 0);
 // scratch the TMA-fed kNN kernel wants for the pre-split candidate tiles (0: shape not served)
 size_t knn_split_bytes(int C, int64_t B, int N, int k);
-// impl 0: tensor cores when the shape allows (and R3DFS_SIMT_GEMM is unset), 1: CUDA cores, 2: tensor cores
+// impl 0: tensor cores when C <= 64, CUDA cores otherwise; 1: CUDA cores; 2: tensor cores
 int launch_knn_auto(const float* x, int ld, int C, const float* xx, int64_t B, int N, int k,
                     int32_t* idx32, int64_t* idx64, int impl, cudaStream_t st,
                     void* split_ws = nullptr, size_t split_bytes = 0);
@@ -128,7 +128,7 @@ int launch_linear_tc(const float* X, int ldx, const float* W, const float* s, co
 int launch_linear_tma(const float* X, int ldx, const float* W, const float* s, const float* t,
                       int act, int64_t M, int K, int Nout, float* Y, int ldy, RowMap map,
                       cudaStream_t st);
-// tensor-core path unless R3DFS_SIMT_GEMM=1 is set in the environment (A/B measurements)
+// TMA-fed tensor-core kernel, or the register-fed one when TMA cannot address the operands
 int launch_linear_auto(const float* X, int ldx, const float* W, const float* s, const float* t,
                        int act, int64_t M, int K, int Nout, float* Y, int ldy, RowMap map,
                        cudaStream_t st);
@@ -139,25 +139,13 @@ int launch_gram_dist_tc(const float* F, int64_t graph_rows, int64_t row_off, int
 int launch_edge_mlp_tc(const float* PQ, const int32_t* idx, const float* w2, const float* s2,
                        const float* t2, int64_t B, int N, int k, float* Y, int ldy, RowMap map,
                        cudaStream_t st);
-int launch_edge_mlp_auto(const float* PQ, const int32_t* idx, const float* w2, const float* s2,
-                         const float* t2, int64_t B, int N, int k, float* Y, int ldy, RowMap map,
-                         cudaStream_t st);
-bool simt_gemm_forced();
-int launch_edge_mlp(const float* PQ, const int32_t* idx, const float* w2, const float* s2,
-                    const float* t2, int64_t B, int N, int k, float* Y, int ldy, RowMap map,
-                    float* w2t_scratch, cudaStream_t st);
 int launch_edge_feature(const float* x, int64_t B, int64_t C, int64_t N, int64_t sb, int64_t sc,
                         int64_t sn, const int64_t* idx, int K, float* out, cudaStream_t st,
                         void* ws = nullptr, size_t ws_bytes = 0);
 size_t edge_feature_scratch_bytes(int64_t B, int64_t C, int64_t N);
-int launch_attention(const float* qkv, int ld, int64_t B, int N, float* Y, int ldy, RowMap map,
-                     cudaStream_t st);
 int launch_attention_tc(const float* qkv, int ld, int64_t B, int N, float* Y, int ldy, RowMap map,
                         cudaStream_t st, float* kmax_ws = nullptr, void* split_ws = nullptr,
                         size_t split_bytes = 0);
-int launch_attention_auto(const float* qkv, int ld, int64_t B, int N, float* Y, int ldy,
-                          RowMap map, cudaStream_t st, float* kmax_ws = nullptr,
-                          void* split_ws = nullptr, size_t split_bytes = 0);
 // scratch for the pre-split K / V^T tiles of the TMA-fed attention kernel
 size_t attention_split_bytes(int64_t B, int N);
 int launch_fold_edge_w1(const float* w1, const float* s1, const float* t1, int C, float* wpq,

@@ -350,128 +350,6 @@ int launch_fold_edge_w1(const float* w1, const float* s1, const float* t1, int C
 }
 
 // --------------------------------------------------------------------------------------------
-// EdgeConv tail: for point i and neighbour j:  h1 = LReLU(P_j + Q_i);  h2 = LReLU(s2 * (W2 h1) + t2);
-// y_i = max_j h2      (reference models/dgcnn.py:56-57 second conv/BN/LReLU, :118 max over k).
-// 64 points per CTA; 8 threads share a pair of points, each thread owns 8 output channels.
-// --------------------------------------------------------------------------------------------
-#define EDGE_PTS 64
-#define EDGE_WSTRIDE 68
-
-__global__ __launch_bounds__(256) void edge_mlp_kernel(const float* __restrict__ PQ,
-                                                       const int32_t* __restrict__ idx,
-                                                       const float* __restrict__ w2,
-                                                       const float* __restrict__ s2,
-                                                       const float* __restrict__ t2, int N, int k,
-                                                       float* __restrict__ Y, int ldy, RowMap map) {
-  __shared__ __align__(16) float W2t[64 * EDGE_WSTRIDE];  // [kk][c]
-  __shared__ __align__(16) float H1[EDGE_PTS * 64];       // [point][kk]
-  const int tid = threadIdx.x;
-  const int b = blockIdx.y;
-  const int p0 = blockIdx.x * EDGE_PTS;
-  const int64_t base = (int64_t)b * N;
-  for (int e = tid; e < 64 * 64; e += 256) {
-    int c = e >> 6, kk = e & 63;
-    W2t[kk * EDGE_WSTRIDE + c] = w2[e];
-  }
-  const int oct = tid >> 3, g = tid & 7;
-  const int pa = p0 + 2 * oct, pb = pa + 1;
-  const bool va = pa < N, vb = pb < N;
-  float qa[8], qb[8], sc[8], sh[8], mxa[8], mxb[8];
-  {
-    const float4* qpa = reinterpret_cast<const float4*>(PQ + (base + (va ? pa : 0)) * 128 + 64 + 8 * g);
-    const float4* qpb = reinterpret_cast<const float4*>(PQ + (base + (vb ? pb : 0)) * 128 + 64 + 8 * g);
-    float4 a0 = qpa[0], a1 = qpa[1], b0 = qpb[0], b1 = qpb[1];
-    qa[0] = a0.x; qa[1] = a0.y; qa[2] = a0.z; qa[3] = a0.w; qa[4] = a1.x; qa[5] = a1.y; qa[6] = a1.z; qa[7] = a1.w;
-    qb[0] = b0.x; qb[1] = b0.y; qb[2] = b0.z; qb[3] = b0.w; qb[4] = b1.x; qb[5] = b1.y; qb[6] = b1.z; qb[7] = b1.w;
-  }
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    sc[c] = s2[8 * g + c];
-    sh[c] = t2[8 * g + c];
-    mxa[c] = -INFINITY;
-    mxb[c] = -INFINITY;
-  }
-  __syncthreads();
-  float* ha = H1 + (2 * oct) * 64;
-  float* hb = ha + 64;
-  for (int j = 0; j < k; ++j) {
-    const int na = va ? idx[(base + pa) * k + j] : 0;
-    const int nb = vb ? idx[(base + pb) * k + j] : 0;
-    const float4* ppa = reinterpret_cast<const float4*>(PQ + (base + na) * 128 + 8 * g);
-    const float4* ppb = reinterpret_cast<const float4*>(PQ + (base + nb) * 128 + 8 * g);
-    float4 a0 = ppa[0], a1 = ppa[1], b0 = ppb[0], b1 = ppb[1];
-    float hva[8] = {a0.x + qa[0], a0.y + qa[1], a0.z + qa[2], a0.w + qa[3],
-                    a1.x + qa[4], a1.y + qa[5], a1.z + qa[6], a1.w + qa[7]};
-    float hvb[8] = {b0.x + qb[0], b0.y + qb[1], b0.z + qb[2], b0.w + qb[3],
-                    b1.x + qb[4], b1.y + qb[5], b1.z + qb[6], b1.w + qb[7]};
-#pragma unroll
-    for (int c = 0; c < 8; ++c) {
-      hva[c] = hva[c] > 0.f ? hva[c] : 0.2f * hva[c];
-      hvb[c] = hvb[c] > 0.f ? hvb[c] : 0.2f * hvb[c];
-    }
-    __syncwarp();  // previous iteration's readers of ha/hb are done
-    *reinterpret_cast<float4*>(ha + 8 * g) = make_float4(hva[0], hva[1], hva[2], hva[3]);
-    *reinterpret_cast<float4*>(ha + 8 * g + 4) = make_float4(hva[4], hva[5], hva[6], hva[7]);
-    *reinterpret_cast<float4*>(hb + 8 * g) = make_float4(hvb[0], hvb[1], hvb[2], hvb[3]);
-    *reinterpret_cast<float4*>(hb + 8 * g + 4) = make_float4(hvb[4], hvb[5], hvb[6], hvb[7]);
-    __syncwarp();
-    float aa[8], ab[8];
-#pragma unroll
-    for (int c = 0; c < 8; ++c) {
-      aa[c] = 0.f;
-      ab[c] = 0.f;
-    }
-#pragma unroll 4
-    for (int kk = 0; kk < 64; kk += 4) {
-      float4 xa = *reinterpret_cast<const float4*>(ha + kk);
-      float4 xb = *reinterpret_cast<const float4*>(hb + kk);
-      float xav[4] = {xa.x, xa.y, xa.z, xa.w};
-      float xbv[4] = {xb.x, xb.y, xb.z, xb.w};
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const float* wr = W2t + (kk + u) * EDGE_WSTRIDE + 8 * g;
-        float4 w0 = *reinterpret_cast<const float4*>(wr);
-        float4 w1 = *reinterpret_cast<const float4*>(wr + 4);
-        float wv[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
-#pragma unroll
-        for (int c = 0; c < 8; ++c) {
-          aa[c] = fmaf(wv[c], xav[u], aa[c]);
-          ab[c] = fmaf(wv[c], xbv[u], ab[c]);
-        }
-      }
-    }
-#pragma unroll
-    for (int c = 0; c < 8; ++c) {
-      float ya = fmaf(sc[c], aa[c], sh[c]);
-      float yb = fmaf(sc[c], ab[c], sh[c]);
-      ya = ya > 0.f ? ya : 0.2f * ya;
-      yb = yb > 0.f ? yb : 0.2f * yb;
-      mxa[c] = fmaxf(mxa[c], ya);
-      mxb[c] = fmaxf(mxb[c], yb);
-    }
-  }
-  if (va) {
-    float* y = Y + map(base + pa) * (int64_t)ldy + 8 * g;
-    *reinterpret_cast<float4*>(y) = make_float4(mxa[0], mxa[1], mxa[2], mxa[3]);
-    *reinterpret_cast<float4*>(y + 4) = make_float4(mxa[4], mxa[5], mxa[6], mxa[7]);
-  }
-  if (vb) {
-    float* y = Y + map(base + pb) * (int64_t)ldy + 8 * g;
-    *reinterpret_cast<float4*>(y) = make_float4(mxb[0], mxb[1], mxb[2], mxb[3]);
-    *reinterpret_cast<float4*>(y + 4) = make_float4(mxb[4], mxb[5], mxb[6], mxb[7]);
-  }
-}
-
-int launch_edge_mlp(const float* PQ, const int32_t* idx, const float* w2, const float* s2,
-                    const float* t2, int64_t B, int N, int k, float* Y, int ldy, RowMap map,
-                    float* /*unused*/, cudaStream_t st) {
-  dim3 grid((N + EDGE_PTS - 1) / EDGE_PTS, (unsigned)B);
-  edge_mlp_kernel<<<grid, 256, 0, st>>>(PQ, idx, w2, s2, t2, N, k, Y, ldy, map);
-  R3DFS_CHECK_LAUNCH();
-  return 0;
-}
-
-// --------------------------------------------------------------------------------------------
 // get_edge_feature (reference models/dgcnn.py:26-42), materialising: out (B, 2C, N, K) =
 // cat(x_j - x_i, x_i).  Pure HBM write stream (the output is 2K x the input).  One thread owns 4
 // consecutive (n, j) positions and walks over the channels: the neighbour indices are read once,
@@ -674,140 +552,6 @@ int launch_edge_feature(const float* x, int64_t B, int64_t C, int64_t N, int64_t
   int64_t quads = (N * K + 3) / 4;
   dim3 grid((unsigned)((quads + 255) / 256), (unsigned)B);
   edge_feature_kernel<<<grid, 256, 0, st>>>(x, (int)C, N, sb, sc, sn, idx, K, out, quads);
-  R3DFS_CHECK_LAUNCH();
-  return 0;
-}
-
-// --------------------------------------------------------------------------------------------
-// SelfAttention, eval (reference models/attention.py:39-48): softmax((q/8)^T k) v, single head,
-// d = 64, streamed over key tiles with a running (max, sum) so the (N, N) map never exists.
-// qkv: rows of [q(64) | k(64) | v(64)] (ld floats apart).  64 queries per CTA.
-// --------------------------------------------------------------------------------------------
-#define ATT_BQ 64
-#define ATT_BK 64
-
-__global__ __launch_bounds__(256) void attention_kernel(const float* __restrict__ qkv, int ld,
-                                                        int N, float* __restrict__ Y, int ldy,
-                                                        RowMap map) {
-  extern __shared__ __align__(16) float smem[];
-  float* Qs = smem;               // [64 d][64 q]  swizzled, pre-divided by 8
-  float* Ks = Qs + 64 * 64;       // [64 d][64 key] swizzled
-  float* Vs = Ks + 64 * 64;       // [64 key][64 d]
-  float* Ps = Vs + 64 * 64;       // [64 key][64 q] swizzled
-  const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
-  const int b = blockIdx.y;
-  const int q0 = blockIdx.x * ATT_BQ;
-  const int64_t base = (int64_t)b * N;
-
-  load_tile_T<64, 64>(Qs, qkv, ld, base + q0, base + N, 0, 64);
-  __syncthreads();
-  for (int e = tid; e < 64 * 64; e += 256) Qs[e] = Qs[e] / 8.f;
-
-  float m_run[4], l_run[4], o[4][4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    m_run[i] = -INFINITY;
-    l_run[i] = 0.f;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) o[i][j] = 0.f;
-  }
-
-  for (int c0 = 0; c0 < N; c0 += ATT_BK) {
-    __syncthreads();
-    load_tile_T<64, 64>(Ks, qkv + 64, ld, base + c0, base + N, 0, 64);
-    for (int e = tid; e < 64 * 16; e += 256) {
-      int r = e >> 4, c4 = e & 15;
-      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (c0 + r < N)
-        v = *reinterpret_cast<const float4*>(qkv + (base + c0 + r) * (int64_t)ld + 128 + 4 * c4);
-      *reinterpret_cast<float4*>(Vs + r * 64 + 4 * c4) = v;
-    }
-    __syncthreads();
-    float sacc[4][4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) sacc[i][j] = 0.f;
-#pragma unroll 8
-    for (int kk = 0; kk < 64; ++kk) {
-      const int sw = (kk & 7) << 2;
-      float4 a = *reinterpret_cast<const float4*>(&Qs[kk * 64 + ((4 * ty) ^ sw)]);
-      float4 c = *reinterpret_cast<const float4*>(&Ks[kk * 64 + ((4 * tx) ^ sw)]);
-      float av[4] = {a.x, a.y, a.z, a.w};
-      float cv[4] = {c.x, c.y, c.z, c.w};
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) sacc[i][j] = fmaf(av[i], cv[j], sacc[i][j]);
-    }
-    // running softmax over this key tile
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      float mx = -INFINITY;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        if (c0 + 4 * tx + j >= N) sacc[i][j] = -INFINITY;
-        mx = fmaxf(mx, sacc[i][j]);
-      }
-#pragma unroll
-      for (int off = 8; off > 0; off >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, off));
-      const float m_new = fmaxf(m_run[i], mx);
-      const float corr = expf(m_run[i] - m_new);  // exp(-inf) = 0 on the first tile
-      float ps = 0.f;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        float p = expf(sacc[i][j] - m_new);
-        sacc[i][j] = p;
-        ps += p;
-      }
-#pragma unroll
-      for (int off = 8; off > 0; off >>= 1) ps += __shfl_xor_sync(0xffffffffu, ps, off);
-      l_run[i] = l_run[i] * corr + ps;
-      m_run[i] = m_new;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) o[i][j] *= corr;
-    }
-    // P -> smem [key][q] swizzled
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int key = 4 * tx + j;
-      const int sw = (key & 7) << 2;
-      *reinterpret_cast<float4*>(&Ps[key * 64 + ((4 * ty) ^ sw)]) =
-          make_float4(sacc[0][j], sacc[1][j], sacc[2][j], sacc[3][j]);
-    }
-    __syncthreads();
-#pragma unroll 8
-    for (int key = 0; key < 64; ++key) {
-      const int sw = (key & 7) << 2;
-      float4 a = *reinterpret_cast<const float4*>(&Ps[key * 64 + ((4 * ty) ^ sw)]);
-      float4 v = *reinterpret_cast<const float4*>(&Vs[key * 64 + 4 * tx]);
-      float av[4] = {a.x, a.y, a.z, a.w};
-      float vv[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) o[i][j] = fmaf(av[i], vv[j], o[i][j]);
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int q = q0 + 4 * ty + i;
-    if (q >= N) continue;
-    const float inv = 1.f / l_run[i];
-    float* y = Y + map(base + q) * (int64_t)ldy + 4 * tx;
-    *reinterpret_cast<float4*>(y) =
-        make_float4(o[i][0] * inv, o[i][1] * inv, o[i][2] * inv, o[i][3] * inv);
-  }
-}
-
-int launch_attention(const float* qkv, int ld, int64_t B, int N, float* Y, int ldy, RowMap map,
-                     cudaStream_t st) {
-  const size_t smem = sizeof(float) * 4 * 64 * 64;
-  cudaError_t e = cudaFuncSetAttribute(attention_kernel,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  dim3 grid((N + ATT_BQ - 1) / ATT_BQ, (unsigned)B);
-  attention_kernel<<<grid, 256, smem, st>>>(qkv, ld, N, Y, ldy, map);
   R3DFS_CHECK_LAUNCH();
   return 0;
 }

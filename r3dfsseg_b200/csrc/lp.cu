@@ -2,103 +2,10 @@
 // in sparse form, plus the query loss / prediction / confusion counters.
 #include <cooperative_groups.h>
 
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "lp.cuh"
 
 namespace cg = cooperative_groups;
-
-// --------------------------------------------------------------------------------------------
-// Squared-L2 matrix of one graph's nodes, Gram form (what faiss.IndexFlatL2 ranks by,
-// models/mpti.py:733-735):  D2[i][j] = |f_i|^2 + |f_j|^2 - 2 f_i.f_j .   128 x 64 tiles.
-// --------------------------------------------------------------------------------------------
-#define GD_BM 128
-#define GD_BN 64
-#define GD_BK 16
-
-template <int ROWS, int KC>
-__device__ __forceinline__ void lp_load_tile_T(float* __restrict__ dst,
-                                               const float* __restrict__ src, int ld, int64_t row0,
-                                               int64_t rows_end, int k0, int k_end) {
-  constexpr int KG = KC / 8;
-  constexpr int PAIRS = (ROWS / 4) * KG;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int nw = blockDim.x >> 5;
-  const int r_lo = lane & 3, k_lo = lane >> 2;
-  for (int p = w; p < PAIRS; p += nw) {
-    int kg = p % KG, rg = p / KG;
-    int row = 4 * rg + r_lo, kk = 8 * kg + k_lo;
-    int64_t gr = row0 + row;
-    int gk = k0 + kk;
-    float v = 0.f;
-    if (gr < rows_end && gk < k_end) v = src[gr * (int64_t)ld + gk];
-    dst[kk * ROWS + (row ^ (k_lo << 2))] = v;
-  }
-}
-
-__global__ __launch_bounds__(256) void gram_dist_kernel(const float* __restrict__ F,
-                                                        int64_t graph_rows, int64_t row_off,
-                                                        int nn, int D,
-                                                        const float* __restrict__ norms,
-                                                        float* __restrict__ D2) {
-  __shared__ __align__(16) float As[GD_BK * GD_BM];
-  __shared__ __align__(16) float Bs[GD_BK * GD_BN];
-  const int g = blockIdx.z;
-  const float* Fg = F + ((int64_t)g * graph_rows + row_off) * D;
-  const float* ng = norms + (int64_t)g * nn;
-  float* Dg = D2 + (int64_t)g * nn * nn;
-  const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
-  const int m0 = blockIdx.x * GD_BM, n0 = blockIdx.y * GD_BN;
-  float acc[8][4];
-#pragma unroll
-  for (int i = 0; i < 8; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-  for (int k0 = 0; k0 < D; k0 += GD_BK) {
-    __syncthreads();
-    lp_load_tile_T<GD_BM, GD_BK>(As, Fg, D, m0, nn, k0, D);
-    lp_load_tile_T<GD_BN, GD_BK>(Bs, Fg, D, n0, nn, k0, D);
-    __syncthreads();
-    const int kend = min(GD_BK, D - k0);
-#pragma unroll 4
-    for (int kk = 0; kk < kend; ++kk) {
-      const int sw = (kk & 7) << 2;
-      float4 a0 = *reinterpret_cast<const float4*>(&As[kk * GD_BM + ((8 * ty) ^ sw)]);
-      float4 a1 = *reinterpret_cast<const float4*>(&As[kk * GD_BM + ((8 * ty + 4) ^ sw)]);
-      float4 bb = *reinterpret_cast<const float4*>(&Bs[kk * GD_BN + ((4 * tx) ^ sw)]);
-      float av[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-      float bv[4] = {bb.x, bb.y, bb.z, bb.w};
-#pragma unroll
-      for (int i = 0; i < 8; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(av[i], bv[j], acc[i][j]);
-    }
-  }
-  const int n = n0 + 4 * tx;
-  if (n >= nn) return;
-  float nj[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) nj[j] = (n + j < nn) ? ng[n + j] : 0.f;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const int m = m0 + 8 * ty + i;
-    if (m >= nn) continue;
-    const float ni = ng[m];
-    float4 o;
-    o.x = (ni + nj[0]) - 2.f * acc[i][0];
-    o.y = (ni + nj[1]) - 2.f * acc[i][1];
-    o.z = (ni + nj[2]) - 2.f * acc[i][2];
-    o.w = (ni + nj[3]) - 2.f * acc[i][3];
-    if (n + 3 < nn && (nn & 3) == 0) {
-      *reinterpret_cast<float4*>(Dg + (int64_t)m * nn + n) = o;
-    } else {
-      float ov[4] = {o.x, o.y, o.z, o.w};
-      for (int j = 0; j < 4; ++j)
-        if (n + j < nn) Dg[(int64_t)m * nn + n + j] = ov[j];
-    }
-  }
-}
 
 // --------------------------------------------------------------------------------------------
 // Per-row selection of the k nearest other valid nodes: 4-pass 8-bit radix select on the row's
@@ -2018,16 +1925,12 @@ static int launch_cg_group(int G, cudaStream_t st, const int32_t* rowptr, const 
     cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
   }
   if (!coop || n_sm < 8) return -1000;
-  static const int gs_env = [] {
-    const char* e = R3DFS_GETENV("R3DFS_CG_GROUP");
-    return e ? atoi(e) : 0;
-  }();
   // CTAs per graph: as few as keep (almost) the whole matrix in shared memory, so that as many
   // graphs as possible are in flight; never more groups than graphs
   // measured on the single graph of a training step (4416 nodes): 74 CTAs beat 37, 110 and 148 —
   // more CTAs shorten the row slices but every CTA restages the whole of P and joins every barrier
-  int n_groups = gs_env > 0 ? min(32, max(1, n_sm / gs_env)) : min(G, 4);
-  int GS = min(GCG_MAX_GS, gs_env > 0 ? gs_env : min(74, n_sm / n_groups));
+  const int n_groups = min(G, 4);
+  const int GS = min(GCG_MAX_GS, min(74, n_sm / n_groups));
   const int rows_max = (nn + GS - 1) / GS;
   const size_t fixed = sizeof(float) * ((size_t)nn * NCV + 3 * (size_t)rows_max * NCV) +
                        sizeof(int) * (size_t)rows_max;
@@ -2126,20 +2029,15 @@ int launch_affinity(const float* F, int64_t graph_rows, int64_t row_off, const u
                     float* sim, cudaStream_t st, const StageRec* sr) {
   if (D % 4 != 0 || D > 32 * LP_MAX_F4 || k > 1024 || nn > 65535) return R3DFS_E_UNSUPPORTED;
   R3DFS_TRY(launch_row_norms_batched(F + row_off * D, graph_rows * D, G, nn, D, D, norms, st));
-  if (simt_gemm_forced()) {
-    dim3 gd((nn + GD_BM - 1) / GD_BM, (nn + GD_BN - 1) / GD_BN, G);
-    gram_dist_kernel<<<gd, 256, 0, st>>>(F, graph_rows, row_off, nn, D, norms, D2);
-    R3DFS_CHECK_LAUNCH();
-  } else {
-    // TMEM-operand kernel (linear_ts_kernel<128, true>); the register-fed one when TMA cannot
-    // address the feature matrix, or under R3DFS_DIST_TC=1 in the measurement build
-    static const bool dist_tc = R3DFS_GETENV("R3DFS_DIST_TC") != nullptr;
-    int rc = dist_tc ? R3DFS_E_UNSUPPORTED
-                     : launch_gram_dist_ts(F, graph_rows, row_off, G, nn, D, norms, D2, st);
-    if (rc == R3DFS_E_UNSUPPORTED)
-      rc = launch_gram_dist_tc(F, graph_rows, row_off, G, nn, D, norms, D2, st);
-    R3DFS_TRY(rc);
-  }
+  // Squared-L2 matrix in Gram form (what faiss.IndexFlatL2 ranks by, models/mpti.py:733-735):
+  // the TMEM-operand kernel (linear_ts_kernel<128, true>); the register-fed one when TMA cannot
+  // address the feature matrix, or under R3DFS_DIST_TC=1 in the measurement build
+  static const bool dist_tc = R3DFS_GETENV("R3DFS_DIST_TC") != nullptr;
+  int rc = dist_tc ? R3DFS_E_UNSUPPORTED
+                   : launch_gram_dist_ts(F, graph_rows, row_off, G, nn, D, norms, D2, st);
+  if (rc == R3DFS_E_UNSUPPORTED)
+    rc = launch_gram_dist_tc(F, graph_rows, row_off, G, nn, D, norms, D2, st);
+  R3DFS_TRY(rc);
   if (sr) sr->mark(R3DFS_ST_DIST, st);
   static const bool sel_block = R3DFS_GETENV("R3DFS_SELECT_BLOCK") != nullptr;
   if (nn <= 32 * 80 && !sel_block) {
@@ -2151,15 +2049,11 @@ int launch_affinity(const float* F, int64_t graph_rows, int64_t row_off, const u
     R3DFS_CHECK_LAUNCH();
   } else if (nn <= 31 * SEL_THREADS && !sel_block) {
     const size_t smem = sizeof(unsigned) * (size_t)nn;  // <= 31 KB
-    static const bool sel_256 = R3DFS_GETENV("R3DFS_SELECT_256") != nullptr;  // A/B: 256-thread CTAs only
-    static const bool sel_512 = R3DFS_GETENV("R3DFS_SELECT_512") != nullptr;  // A/B: 512-thread CTAs always
-    if (nn <= 19 * SEL_THREADS && !sel_512)
+    if (nn <= 19 * SEL_THREADS)
       knn_select_reg_kernel<20><<<dim3(nn, G), SEL_THREADS, smem, st>>>(D2, valid, nn, k, nbr);
-    else if (!sel_256)  // 512 threads keep 20 keys per thread and 1024 threads per SM in flight
-      knn_select_reg_kernel<20, 512><<<dim3(nn, G), 512, smem, st>>>(D2, valid, nn, k, nbr);  // (32 keys
-                                                            // per thread on 256 threads: half the occupancy)
-    else
-      knn_select_reg_kernel<32><<<dim3(nn, G), SEL_THREADS, smem, st>>>(D2, valid, nn, k, nbr);
+    else  // 512 threads keep 20 keys per thread and 1024 threads per SM in flight (32 keys per
+          // thread on 256 threads: half the occupancy)
+      knn_select_reg_kernel<20, 512><<<dim3(nn, G), 512, smem, st>>>(D2, valid, nn, k, nbr);
     R3DFS_CHECK_LAUNCH();
   } else {
     size_t smem = sizeof(unsigned) * (size_t)nn;
@@ -2190,8 +2084,7 @@ int launch_lp_solve(const int32_t* rowptr, const int32_t* rowlen, const uint16_t
   const size_t smem_cg = sizeof(float) * (size_t)nn * ncv;
   if (smem_cg > 200 * 1024) return R3DFS_E_UNSUPPORTED;
   int rc = -1000;
-  static const bool no_group = R3DFS_GETENV("R3DFS_CG_NOGROUP") != nullptr;
-  if (latency && !no_group) {  // matrix resident in shared memory, groups of CTAs (cooperative launch)
+  if (latency) {  // matrix resident in shared memory, groups of CTAs (cooperative launch)
     const size_t scratch_floats = (size_t)G * nn * ncv;
     rc = ncv == 4 ? launch_cg_group<4>(G, st, rowptr, rowlen, mcol, mval, valid, nn, k, Y, nc, alpha,
                                        tol, max_iter, Z, P, AP, scratch_floats, iters_out, resid_out)
@@ -2200,11 +2093,6 @@ int launch_lp_solve(const int32_t* rowptr, const int32_t* rowlen, const uint16_t
     if (rc == 0) return 0;
     if (rc != -1000) return rc;
   }
-  static const int cl_first = [] {  // A/B switch: R3DFS_CG_CLUSTER = 16 | 8 | 4 | 2
-    const char* e = R3DFS_GETENV("R3DFS_CG_CLUSTER");
-    const int v = e ? atoi(e) : 0;
-    return (v == 16 || v == 8 || v == 4 || v == 2) ? v : 0;
-  }();
   // One CTA per SM (the kernel keeps a queue of matrix rounds in 128 registers per thread), so a
   // batch of graphs gets as many CTAs per graph as keep ALL graphs in flight in one wave (25 graphs
   // on 148 SMs: clusters of 5); a handful of graphs gets 16.  A warp keeps the metadata of at most
@@ -2214,8 +2102,7 @@ int launch_lp_solve(const int32_t* rowptr, const int32_t* rowlen, const uint16_t
   cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
   const int rows_cta_max = CGC_MAXT * CG_MAXPASS;
   const int cl_need = (nn + rows_cta_max - 1) / rows_cta_max;
-  int cl_start = cl_first ? cl_first : (G <= 4 ? 16 : max(1, min(8, n_sm / G)));
-  cl_start = max(cl_start, cl_need);
+  const int cl_start = max(G <= 4 ? 16 : max(1, min(8, n_sm / G)), cl_need);
   for (int CL = cl_start; CL >= cl_need && CL >= 1 && rc == -1000;
        CL = (CL & (CL - 1)) ? (1 << (31 - __builtin_clz(CL))) : CL >> 1) {
     if (ncv == 4)

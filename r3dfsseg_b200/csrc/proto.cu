@@ -165,15 +165,7 @@ __global__ __launch_bounds__(FPS_THREADS) void fps_kernel(const float* __restric
 // flight), so a set's sweep time is its bytes over (CTAs x that rate): with a batch of episodes
 // 8-CTA clusters already fill every SM twice over and HBM is the limit, but the handful of sets of
 // a single episode (the training step) leaves most SMs idle — those get 16-CTA clusters.
-static int fps_cluster_size(int n_sets) {
-  static const int forced = [] {  // A/B switch: R3DFS_FPS_CLUSTER = 1..16
-    const char* e = R3DFS_GETENV("R3DFS_FPS_CLUSTER");
-    const int v = e ? atoi(e) : 0;
-    return (v >= 1 && v <= FPS_MAX_CL) ? v : 0;
-  }();
-  if (forced) return forced;
-  return n_sets <= 16 ? 16 : 8;
-}
+static int fps_cluster_size(int n_sets) { return n_sets <= 16 ? 16 : 8; }
 
 // The streaming kernel above (every pick re-reads the set): few picks (the fps_k = 4 prototypes of
 // the way-contrast loss), feature widths other than 192, callers without a spill area.
@@ -231,19 +223,15 @@ int launch_fps_ex(const float* feat, int D, const int32_t* set_off, const int32_
                   int n_sets, int n_cap, int m_max, int k_for_count, int32_t* idx_out,
                   int32_t* cnt_out, cudaStream_t st, uint8_t* spill, int sets_per_group,
                   int impl) {
-  static const bool force_stream = R3DFS_GETENV("R3DFS_FPS_STREAM") != nullptr;  // A/B
   const bool q8_ok = spill != nullptr && D == 192;
   if (impl == R3DFS_FPS_Q8 && !q8_ok) return R3DFS_E_UNSUPPORTED;
-  if (impl == R3DFS_FPS_STREAM || !q8_ok || (impl == R3DFS_FPS_AUTO && (m_max < 16 || force_stream)))
+  if (impl == R3DFS_FPS_STREAM || !q8_ok || (impl == R3DFS_FPS_AUTO && m_max < 16))
     return launch_fps_stream(feat, D, set_off, set_n, n_sets, n_cap, m_max, k_for_count, idx_out,
                              cnt_out, st);
   if (sets_per_group > 1 && n_sets % sets_per_group == 0) {
     const int groups = n_sets / sets_per_group, per = sets_per_group - 1;
-    static const int bg_cl = [] {  // A/B switch: R3DFS_FPS_BG_CL = CTAs per background set (0: fit the set)
-      const char* e = R3DFS_GETENV("R3DFS_FPS_BG_CL");
-      return e ? atoi(e) : 0;
-    }();
-    R3DFS_TRY(launch_fps_q8(feat, set_off, set_n, groups, 0, 1, sets_per_group, n_cap, bg_cl, m_max,
+    // background sets: cl = 0, the smallest cluster whose shared memory holds the set
+    R3DFS_TRY(launch_fps_q8(feat, set_off, set_n, groups, 0, 1, sets_per_group, n_cap, 0, m_max,
                             k_for_count, spill, idx_out, cnt_out, st));
     // foreground sets: as many CTAs per set as keep all of them in ONE wave (rows beyond the
     // cluster's shared memory are swept from the spill area, still as bytes)
@@ -303,82 +291,6 @@ __global__ void seeds_unique_kernel(const int32_t* __restrict__ picks,
   }
   __syncthreads();
   for (int i = cnt + tid; i < m_max; i += 128) out[i] = -1;
-}
-
-// --------------------------------------------------------------------------------------------
-// Hard assignment (models/mpti.py:618-622): argmin_j || f - seed_j + 1e-6 ||_2, torch<=1.8
-// pairwise_distance semantics (eps added to the difference, inside the norm), first minimum.
-// Seeds staged in shared memory; 8 lanes per point.
-// --------------------------------------------------------------------------------------------
-#define ASSIGN_THREADS 256
-#define ASSIGN_PTS_PER_CTA 256
-
-__global__ __launch_bounds__(ASSIGN_THREADS) void assign_kernel(
-    const float* __restrict__ feat, int D, const int32_t* __restrict__ set_off,
-    const int32_t* __restrict__ set_n, const int32_t* __restrict__ seeds,
-    const int32_t* __restrict__ proto_cnt, int m_max, int k, int32_t* __restrict__ assign) {
-  extern __shared__ __align__(16) float sseed[];  // [m][D]
-  const int set = blockIdx.y;
-  const int n = set_n[set];
-  const int p_begin = blockIdx.x * ASSIGN_PTS_PER_CTA;
-  if (p_begin >= n) return;
-  const int64_t row0 = set_off[set];
-  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
-  const int sub = lane & 7, grp = lane >> 3;
-  const int p_end = min(n, p_begin + ASSIGN_PTS_PER_CTA);
-  if (n <= k) {  // identity
-    for (int p = p_begin + tid; p < p_end; p += ASSIGN_THREADS) assign[row0 + p] = p;
-    return;
-  }
-  const int m = proto_cnt[set];
-  const int D4 = D >> 2;
-  for (int e = tid; e < m * D4; e += ASSIGN_THREADS) {
-    int j = e / D4, c4 = e % D4;
-    int sidx = seeds[(int64_t)set * m_max + j];
-    reinterpret_cast<float4*>(sseed)[e] =
-        reinterpret_cast<const float4*>(feat + (row0 + sidx) * (int64_t)D)[c4];
-  }
-  __syncthreads();
-  for (int pb = p_begin + w * 4; pb < p_end; pb += (ASSIGN_THREADS / 32) * 4) {
-    const int p = pb + grp;
-    const bool valid = p < p_end;
-    float4 xf[FPS_MAX_F4];
-    const float4* xrow =
-        reinterpret_cast<const float4*>(feat + (row0 + (valid ? p : p_begin)) * (int64_t)D);
-#pragma unroll
-    for (int u = 0; u < FPS_MAX_F4; ++u) {
-      int c4 = sub + 8 * u;
-      xf[u] = (c4 < D4) ? xrow[c4] : make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-    float best = INFINITY;
-    int bj = 0;
-    for (int j = 0; j < m; ++j) {
-      const float4* sr = reinterpret_cast<const float4*>(sseed + (int64_t)j * D);
-      float acc = 0.f;
-#pragma unroll
-      for (int u = 0; u < FPS_MAX_F4; ++u) {
-        int c4 = sub + 8 * u;
-        if (c4 < D4) {
-          float4 s4 = sr[c4];
-          float d0 = __fadd_rn(xf[u].x - s4.x, 1e-6f), d1 = __fadd_rn(xf[u].y - s4.y, 1e-6f),
-                d2 = __fadd_rn(xf[u].z - s4.z, 1e-6f), d3 = __fadd_rn(xf[u].w - s4.w, 1e-6f);
-          acc = fmaf(d0, d0, acc);
-          acc = fmaf(d1, d1, acc);
-          acc = fmaf(d2, d2, acc);
-          acc = fmaf(d3, d3, acc);
-        }
-      }
-      acc += __shfl_xor_sync(0xffffffffu, acc, 1);
-      acc += __shfl_xor_sync(0xffffffffu, acc, 2);
-      acc += __shfl_xor_sync(0xffffffffu, acc, 4);
-      float dn = sqrtf(acc);
-      if (dn < best) {
-        best = dn;
-        bj = j;
-      }
-    }
-    if (valid && sub == 0) assign[row0 + p] = bj;
-  }
 }
 
 // --------------------------------------------------------------------------------------------
@@ -466,23 +378,13 @@ int launch_multi_prototypes(const float* feat, int D, const int32_t* set_off,
   if (sr) sr->mark(R3DFS_ST_FPS, st);
   seeds_unique_kernel<<<n_sets, 128, 0, st>>>(picks, pick_cnt, set_n, m_max, k, seeds, proto_cnt);
   R3DFS_CHECK_LAUNCH();
-  cudaError_t e = cudaSuccess;
-  if (simt_gemm_forced()) {  // FP32 CUDA-core evaluation of every (point, seed) pair
-    size_t smem = sizeof(float) * (size_t)m_max * D;
-    e = cudaFuncSetAttribute(assign_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    dim3 ga((n_cap + ASSIGN_PTS_PER_CTA - 1) / ASSIGN_PTS_PER_CTA, n_sets);
-    assign_kernel<<<ga, ASSIGN_THREADS, smem, st>>>(feat, D, set_off, set_n, seeds, proto_cnt,
-                                                    m_max, k, assign);
-    R3DFS_CHECK_LAUNCH();
-  } else {  // tensor-core filter + exact verify (tc_assign.cu)
-    R3DFS_TRY(launch_assign_tc(feat, D, set_off, set_n, seeds, proto_cnt, n_sets, n_cap, m_max, k,
-                               seed_stats, seed_stats + (size_t)n_sets * 128, assign, st));
-  }
+  // tensor-core filter + exact verify (tc_assign.cu)
+  R3DFS_TRY(launch_assign_tc(feat, D, set_off, set_n, seeds, proto_cnt, n_sets, n_cap, m_max, k,
+                             seed_stats, seed_stats + (size_t)n_sets * 128, assign, st));
   const int n_chunks = multi_prototypes_chunks(n_cap);
   const size_t smem_p = sizeof(float) * (size_t)m_max * D + sizeof(int) * (size_t)m_max;
-  e = cudaFuncSetAttribute(proto_partial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (int)smem_p);
+  cudaError_t e = cudaFuncSetAttribute(proto_partial_kernel,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_p);
   if (e != cudaSuccess) return (int)e;
   proto_partial_kernel<<<dim3(n_chunks, n_sets), MEAN_THREADS, smem_p, st>>>(
       feat, D, set_off, set_n, proto_cnt, assign, m_max, n_chunks, partial, pcount);

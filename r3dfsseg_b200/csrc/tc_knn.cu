@@ -1209,14 +1209,6 @@ static int launch_knn_tc_t(const float* x, int ld, int C, const float* xx, int64
   return 0;
 }
 
-static bool knn_single_pass_forced() {  // A/B switch: R3DFS_KNN_SINGLE_PASS=1
-  static const bool v = [] {
-    const char* e = R3DFS_GETENV("R3DFS_KNN_SINGLE_PASS");
-    return e && e[0] == '1';
-  }();
-  return v;
-}
-
 static bool knn_tc2_forced() {  // A/B switch: R3DFS_KNN_TC2=1 (register-fed two-pass kernel)
   static const bool v = [] {
     const char* e = R3DFS_GETENV("R3DFS_KNN_TC2");
@@ -1231,7 +1223,7 @@ int launch_knn_tc(const float* x, int ld, int C, const float* xx, int64_t B, int
                   size_t split_bytes) {
   if (k < 1 || k > 32 || C > 64 || N < k) return R3DFS_E_UNSUPPORTED;
   // TMA-fed kernel when the caller lends scratch for the pre-split tiles
-  if (split_ws && !knn_single_pass_forced() && !knn_tc2_forced()) {
+  if (split_ws && !knn_tc2_forced()) {
     const size_t need = knn_split_bytes(C, B, N, k);
     if (need && split_bytes >= need && (reinterpret_cast<uintptr_t>(split_ws) & 15) == 0) {
       if (C <= 16)
@@ -1240,8 +1232,8 @@ int launch_knn_tc(const float* x, int ld, int C, const float* xx, int64_t B, int
     }
   }
   // two-pass selection (measured per 300 clouds of 2048 points: C = 9: 2.03 vs 3.05 ms single
-  // pass, C = 64: 3.20 vs 3.43 ms); R3DFS_KNN_SINGLE_PASS=1 switches it off (A/B measurements).
-  if (k <= 20 && N >= 1024 && N <= 65535 && !knn_single_pass_forced()) {
+  // pass, C = 64: 3.20 vs 3.43 ms)
+  if (k <= 20 && N >= 1024 && N <= 65535) {
     if (C <= 16) return launch_knn_tc2_t<4>(x, ld, C, xx, B, N, k, idx32, idx64, st);
     return launch_knn_tc2_t<16>(x, ld, C, xx, B, N, k, idx32, idx64, st);
   }

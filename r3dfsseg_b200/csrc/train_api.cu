@@ -219,13 +219,12 @@ static int lin_bwd_x_tc(const TrainCtx& c, const float* dY, int ld_dy, const flo
 // dW (Nout x K) += dY^T X, reduced over M rows (split-K, fixed order)
 static int lin_bwd_w(const TrainCtx& c, const TrainWs& t, const float* dY, int ld_dy, const float* X,
                      int ldx, int64_t M, int K, int Nout, float* dW) {
-  if (!simt_gemm_forced()) {  // 3xTF32 tensor cores, split over the rows, fixed-order reduce
-    const int max_splits = (int)(SGEMM_PARTIAL_FLOATS / ((size_t)Nout * K));
-    if (max_splits >= 1) {
-      int splits = 1;
-      R3DFS_TRY(launch_gemm_tn_tc(dY, ld_dy, X, ldx, Nout, K, M, max_splits, t.partial, &splits, c.st));
-      return launch_sgemm_reduce(t.partial, Nout, K, splits, 1.f, 1.f, dW, K, c.st);
-    }
+  // 3xTF32 tensor cores, split over the rows, fixed-order reduce
+  const int max_splits = (int)(SGEMM_PARTIAL_FLOATS / ((size_t)Nout * K));
+  if (max_splits >= 1) {
+    int splits = 1;
+    R3DFS_TRY(launch_gemm_tn_tc(dY, ld_dy, X, ldx, Nout, K, M, max_splits, t.partial, &splits, c.st));
+    return launch_sgemm_reduce(t.partial, Nout, K, splits, 1.f, 1.f, dW, K, c.st);
   }
   const int splits = sgemm_splits(Nout, K, M, 1);
   if ((size_t)splits * Nout * K > SGEMM_PARTIAL_FLOATS) return R3DFS_E_WORKSPACE;

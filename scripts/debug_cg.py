@@ -11,5 +11,4 @@ for name in ("s3dis_2way_1shot", "s3dis_2way_5shot_mdns"):
     ep = make_episode(c["seed"], c["n_way"], c["k_shot"], dataset=c["dataset"], noise_ratio=c["noise_ratio"])
     pred, loss = m(ep.support_x.cuda(), ep.support_y.cuda(), ep.query_x.cuda(), ep.query_y.cuda(), gt_support_y=ep.gt_support_y.cuda(), eval=c["eval"])
     ref = c["query_pred"]
-    print(name, os.environ.get("R3DFS_CG_NOPACK"), os.environ.get("R3DFS_CG_NOSCHED"), os.environ.get("R3DFS_CG_CLUSTER"),
-          "err", float((pred.cpu() - ref).abs().max() / ref.abs().max()), "iters", int(m._last_diag["cg_iters"][0]), "resid", float(m._last_diag["cg_resid"][0]))
+    print(name, "err", float((pred.cpu() - ref).abs().max() / ref.abs().max()), "iters", int(m._last_diag["cg_iters"][0]), "resid", float(m._last_diag["cg_resid"][0]))
