@@ -478,7 +478,8 @@ size_t r3dfs_affinity_workspace(int n_graphs, int64_t n_max, int64_t D, int k) {
   (void)D;
   (void)k;
   return align_up(sizeof(float) * (size_t)n_graphs * n_max, 256) +
-         align_up(sizeof(float) * (size_t)n_graphs * n_max * n_max, 256) + 512;
+         align_up(sizeof(float) * (size_t)n_graphs * n_max * n_max, 256) +
+         align_up(sizeof(unsigned) * affinity_gmin_words(n_graphs, n_max), 256) + 512;
 }
 
 int r3dfs_affinity_knn(const float* node_feat, const uint8_t* valid, int n_graphs, int64_t n_max,
@@ -491,8 +492,9 @@ int r3dfs_affinity_knn(const float* node_feat, const uint8_t* valid, int n_graph
   WsBump ws(wsp, ws_bytes);
   float* norms = ws.take<float>((size_t)n_graphs * n_max);
   float* D2 = ws.take<float>((size_t)n_graphs * n_max * n_max);
+  unsigned* gmin = ws.take<unsigned>(affinity_gmin_words(n_graphs, n_max));
   return launch_affinity(node_feat, n_max, 0, valid, n_graphs, (int)n_max, (int)D, k, sigma, norms,
-                         D2, nbr, sim, (cudaStream_t)stream);
+                         D2, gmin, nbr, sim, (cudaStream_t)stream);
 }
 
 // scratch shared by the sort-free in-edge build (bit matrix + rank prefixes) and, after it, by the
@@ -656,6 +658,7 @@ static void carve_graph_bufs(WsBump& ws, const r3dfs_episode_cfg_t* c, const Epi
   w.norms = ws.take<float>(G * nn);
   // dense squared distances; afterwards scratch of the in-edge build and of the solver's packed rows
   w.D2 = ws.take<float>(episode_d2_floats(G, nn, k));
+  w.gmin = ws.take<unsigned>(affinity_gmin_words(G, nn));
   w.nbr = ws.take<int32_t>(G * nn * k);
   w.sim = ws.take<float>(G * nn * k);
   w.in_cnt = ws.take<int32_t>(G * (nn + 1));
@@ -780,7 +783,7 @@ static int episode_query_part(const r3dfs_episode_cfg_t* cfg, const EpisodeDims&
                                                          d.nc, w.valid, w.Y);
   R3DFS_CHECK_LAUNCH();
   R3DFS_TRY(launch_affinity(w.F, f_rows, 0, w.valid, E, d.nn, D, cfg->k_connect, cfg->sigma,
-                            w.norms, w.D2, w.nbr, w.sim, st, sr));
+                            w.norms, w.D2, w.gmin, w.nbr, w.sim, st, sr));
   R3DFS_TRY(launch_label_propagate(w.nbr, w.sim, w.valid, E, d.nn, cfg->k_connect, w.Y, d.nc,
                                    cfg->alpha, cfg->cg_tol, cfg->cg_max_iter, w.in_cnt, w.in_ptr,
                                    w.in_src, w.in_w, w.dinv, w.rowptr, w.rowlen, w.cursor, w.mcol,

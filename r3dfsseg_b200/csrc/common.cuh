@@ -97,6 +97,23 @@ __device__ __forceinline__ float apply_act(float v, int act) {
   return v;
 }
 
+// Affinity graph (lp.cu, and the distance GEMM's epilogue in tc_gemm_tma.cu): squared distances are
+// ranked by order-preserving integer keys.  0xffffffff is reserved for "not a real column" (the row's
+// own node, an invalid node), so a real distance whose key would be 0xffffffff is clamped.
+__device__ __forceinline__ unsigned f2key(float f) {
+  unsigned u = __float_as_uint(f);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ unsigned dist_key(float f) {
+  const unsigned kk = f2key(f);
+  return kk == 0xffffffffu ? 0xfffffffeu : kk;
+}
+// The distance GEMM can also write, per row, the smallest key of every group of AFF_GROUP
+// contiguous columns: the bound of the select (lp.cu).  Layout (graphs, nn, aff_gstride(nn)) u32,
+// rows padded to whole 32-column chunks (the GEMM stores a chunk's minima as one 16-byte vector).
+#define AFF_GROUP 8
+__host__ __device__ inline int aff_gstride(int nn) { return (nn + 31) / 32 * (32 / AFF_GROUP); }
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -132,8 +149,11 @@ int launch_linear_tma(const float* X, int ldx, const float* W, const float* s, c
 int launch_linear_auto(const float* X, int ldx, const float* W, const float* s, const float* t,
                        int act, int64_t M, int K, int Nout, float* Y, int ldy, RowMap map,
                        cudaStream_t st);
+// gmin (optional): the group minima of every row, with the row's own column and the columns of
+// invalid nodes (valid[g][j] == 0) counted as 0xffffffff
 int launch_gram_dist_ts(const float* F, int64_t graph_rows, int64_t row_off, int G, int nn, int D,
-                        const float* norms, float* D2, cudaStream_t st);
+                        const float* norms, float* D2, const uint8_t* valid, unsigned* gmin,
+                        cudaStream_t st);
 int launch_gram_dist_tc(const float* F, int64_t graph_rows, int64_t row_off, int G, int nn, int D,
                         const float* norms, float* D2, cudaStream_t st);
 int launch_edge_mlp_tc(const float* PQ, const int32_t* idx, const float* w2, const float* s2,

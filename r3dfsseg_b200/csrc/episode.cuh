@@ -36,6 +36,7 @@ struct EpisodeWs {
   int32_t* cell_cnt;
   uint8_t* valid;
   float *Y, *norms, *D2;
+  unsigned* gmin;  // group minima of the distance matrix (launch_affinity)
   int32_t* nbr;
   float* sim;
   int32_t *in_cnt, *in_ptr, *in_src;

@@ -12,11 +12,6 @@ namespace cg = cooperative_groups;
 // order-preserving integer keys in shared memory, then an ordered compaction (ties at the k-th
 // distance -> lowest index).  One CTA per row.
 // --------------------------------------------------------------------------------------------
-__device__ __forceinline__ unsigned f2key(float f) {
-  unsigned u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 #define SEL_THREADS 256
 
 __global__ __launch_bounds__(SEL_THREADS) void knn_select_kernel(const float* __restrict__ D2,
@@ -452,6 +447,230 @@ __global__ __launch_bounds__(NT, (KPT <= 20 ? 1024 : 512) / NT) void knn_select_
         ++pos;
       }
     }
+  }
+}
+
+// --------------------------------------------------------------------------------------------
+// Bounded selection: the same neighbour lists from the distance GEMM's group minima (AFF_GROUP
+// contiguous columns per group, tc_gemm_tma.cu) and one pass over the row.
+//
+// Why the bound holds: let tau be the k-th smallest group minimum.  The k groups with the smallest
+// minima each hold a distinct real column whose key is <= tau, so the k-th smallest real key T
+// satisfies T <= tau.  Every selected column has a key <= T <= tau, and so does every column whose
+// key equals T.  The candidates (real columns with key <= tau), kept in column order, therefore
+// hold all the columns the select can pick and every tie at T, in the order that sends ties to the
+// lowest index: the exact select on the candidates is the exact select on the row.
+//
+// One warp per row: tau by range narrowing over the ~nn / AFF_GROUP group minima; the row streamed
+// once in 16-byte loads, the candidates ballot-compacted into the warp's shared buffer; the exact
+// select (T, ties, ordered list) on the candidates.  A row without a bound (fewer than k groups hold
+// a real column) or with more than SELB_CAP candidates takes the same exact select on the whole row,
+// read again from global memory.  Needs nn % 4 == 0 and a 4-byte aligned `valid`.
+// --------------------------------------------------------------------------------------------
+#define SELB_WARPS 4
+#define SELB_CAP 1024  // candidates per row (see bounded_select_pays)
+#define SELB_LOADS 8    // 16-byte loads in flight per lane
+
+// the k-th smallest (k >= 1) of the keys key_at(0 .. n-1) that are not 0xffffffff, as T and the
+// number need_eq of keys equal to T among the k smallest; with fewer than k such keys, T = 0xffffffff
+// and need_eq = k - their count.  The range narrowing of knn_select_warp_kernel.  Whole warp.
+template <class KeyAt>
+__device__ __forceinline__ void warp_kth_key(int n, int k, KeyAt key_at, int* hist, int lane,
+                                             unsigned& T, int& need_eq) {
+  unsigned lo = 0xffffffffu, hi = 0u;
+  int n_real = 0;
+  for (int j = lane; j < n; j += 32) {
+    const unsigned kk = key_at(j);
+    const bool real = kk != 0xffffffffu;
+    lo = real ? min(lo, kk) : lo;
+    hi = real ? max(hi, kk) : hi;
+    n_real += real;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+    hi = max(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+    n_real += __shfl_xor_sync(0xffffffffu, n_real, o);
+  }
+  if (n_real < k) {
+    T = 0xffffffffu;
+    need_eq = k - n_real;
+    return;
+  }
+  int need = k;
+  while (true) {
+    const unsigned range = hi - lo;
+    if (range == 0) {
+      T = lo;
+      need_eq = need;
+      return;
+    }
+    const int sh = max(0, 24 - (int)__clz(range));
+#pragma unroll
+    for (int q = 0; q < 8; ++q) hist[lane + 32 * q] = 0;
+    __syncwarp();
+    for (int j = lane; j < n; j += 32) {
+      const unsigned kk = key_at(j);
+      if (kk >= lo && kk <= hi) atomicAdd(&hist[(kk - lo) >> sh], 1);
+    }
+    __syncwarp();
+    int h[8], local = 0;
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+      h[q] = hist[8 * lane + q];
+      local += h[q];
+    }
+    int incl = local;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int a = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += a;
+    }
+    const int excl = incl - local;
+    const bool mine = excl < need && need <= incl;
+    int b = 0, cum = 0, hb = 0;
+    if (mine) {
+      cum = excl;
+      b = 8 * lane;
+#pragma unroll
+      for (int q = 0; q < 8; ++q) {
+        hb = h[q];
+        if (cum + h[q] >= need) break;
+        cum += h[q];
+        ++b;
+      }
+    }
+    const int src = __ffs(__ballot_sync(0xffffffffu, mine)) - 1;
+    b = __shfl_sync(0xffffffffu, b, src);
+    cum = __shfl_sync(0xffffffffu, cum, src);
+    hb = __shfl_sync(0xffffffffu, hb, src);
+    __syncwarp();
+    need -= cum;
+    const unsigned nlo = lo + ((unsigned)b << sh);
+    const unsigned nhi = min(hi, nlo + ((1u << sh) - 1u));
+    if (hb == need) {
+      T = nhi + 1u;
+      need_eq = 0;
+      return;
+    }
+    if (sh == 0) {
+      T = nlo;
+      need_eq = need;
+      return;
+    }
+    lo = nlo;
+    hi = nhi;
+  }
+}
+
+// out[0 .. k-1] = col_at(j) of the keys < T and of the first need_eq keys == T, in the order of j
+template <class KeyAt, class ColAt>
+__device__ __forceinline__ void warp_emit_selected(int n, int k, KeyAt key_at, ColAt col_at,
+                                                   unsigned T, int need_eq, int lane, int32_t* out) {
+  const unsigned lt_mask = (1u << lane) - 1u;
+  int pos = 0, eq_seen = 0;
+  for (int j0 = 0; j0 < n && pos < k; j0 += 32) {
+    const int j = j0 + lane;
+    const unsigned kk = j < n ? key_at(j) : 0u;
+    const bool is_eq = j < n && kk == T;
+    const unsigned eqb = __ballot_sync(0xffffffffu, is_eq);
+    bool sel = j < n && kk < T;
+    if (is_eq) sel = eq_seen + __popc(eqb & lt_mask) < need_eq;
+    const unsigned sb = __ballot_sync(0xffffffffu, sel);
+    if (sel) {
+      const int p = pos + __popc(sb & lt_mask);
+      if (p < k) out[p] = col_at(j);
+    }
+    pos += __popc(sb);
+    eq_seen += __popc(eqb);
+  }
+}
+
+__global__ __launch_bounds__(SELB_WARPS * 32) void knn_select_bounded_kernel(
+    const float* __restrict__ D2, const uint8_t* __restrict__ valid,
+    const unsigned* __restrict__ gmin, int nn, int k, int32_t* __restrict__ nbr) {
+  __shared__ unsigned s_key[SELB_WARPS][SELB_CAP];
+  __shared__ uint16_t s_col[SELB_WARPS][SELB_CAP];
+  __shared__ int s_hist[SELB_WARPS][256];
+  const int g = blockIdx.y, lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int i = blockIdx.x * SELB_WARPS + w;  // no block barrier below: a warp may leave
+  if (i >= nn) return;
+  const uint8_t* vg = valid + (int64_t)g * nn;
+  if (!vg[i]) return;
+  const float* row = D2 + ((int64_t)g * nn + i) * nn;
+  int32_t* out = nbr + ((int64_t)g * nn + i) * k;
+  int* hist = s_hist[w];
+  unsigned* ck = s_key[w];
+  uint16_t* cc = s_col[w];
+  const int ngrp = (nn + AFF_GROUP - 1) / AFF_GROUP;
+  const unsigned* gr = gmin + ((int64_t)g * nn + i) * aff_gstride(nn);
+  // tau: any key with at least k group minima at or below it bounds the cut; T - 1 when exactly k
+  // minima lie below T
+  unsigned T;
+  int need_eq;
+  warp_kth_key(ngrp, k, [&](int j) { return __ldg(gr + j); }, hist, lane, T, need_eq);
+  int cnt = 0;
+  if (T != 0xffffffffu) {
+    const unsigned tau = need_eq == 0 ? T - 1u : T;
+    const float4* row4 = reinterpret_cast<const float4*>(row);
+    const uint32_t* vw = reinterpret_cast<const uint32_t*>(vg);
+    const unsigned lt_mask = (1u << lane) - 1u;
+    const int nq = nn / 4;
+    // SELB_LOADS 16-byte loads per lane are issued before any of them is used: the compaction's
+    // ballots and shared-memory stores would otherwise hold every load back behind the last one
+    for (int q0 = 0; q0 < nq; q0 += 32 * SELB_LOADS) {
+      float4 vv[SELB_LOADS];
+      uint32_t vbs[SELB_LOADS];
+#pragma unroll
+      for (int u = 0; u < SELB_LOADS; ++u) {
+        const int q = q0 + 32 * u + lane;
+        vv[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+        vbs[u] = 0;
+        if (q < nq) {
+          vv[u] = __ldcs(row4 + q);
+          vbs[u] = __ldg(vw + q);
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < SELB_LOADS; ++u) {
+        const int q = q0 + 32 * u + lane;  // columns 4 q .. 4 q + 3
+        const float e[4] = {vv[u].x, vv[u].y, vv[u].z, vv[u].w};
+        bool c[4];
+        int nc = 0;
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+          c[t] = ((vbs[u] >> (8 * t)) & 0xffu) && 4 * q + t != i && dist_key(e[t]) <= tau;
+          nc += c[t];
+        }
+        // ordered compaction: exclusive prefix of the lanes' counts (0..4) from three bit ballots
+        const unsigned m0 = __ballot_sync(0xffffffffu, nc & 1),
+                       m1 = __ballot_sync(0xffffffffu, nc & 2),
+                       m2 = __ballot_sync(0xffffffffu, nc & 4);
+        int p = cnt + __popc(m0 & lt_mask) + 2 * __popc(m1 & lt_mask) + 4 * __popc(m2 & lt_mask);
+#pragma unroll
+        for (int t = 0; t < 4; ++t)
+          if (c[t]) {
+            if (p < SELB_CAP) {
+              ck[p] = dist_key(e[t]);
+              cc[p] = (uint16_t)(4 * q + t);
+            }
+            ++p;
+          }
+        cnt += __popc(m0) + 2 * __popc(m1) + 4 * __popc(m2);
+      }
+    }
+    __syncwarp();
+  }
+  if (T != 0xffffffffu && cnt <= SELB_CAP) {
+    warp_kth_key(cnt, k, [&](int j) { return ck[j]; }, hist, lane, T, need_eq);
+    warp_emit_selected(cnt, k, [&](int j) { return ck[j]; }, [&](int j) { return (int)cc[j]; }, T,
+                       need_eq, lane, out);
+  } else {
+    auto key_at = [&](int j) {
+      return (vg[j] && j != i) ? dist_key(__ldcg(row + j)) : 0xffffffffu;
+    };
+    warp_kth_key(nn, k, key_at, hist, lane, T, need_eq);
+    warp_emit_selected(nn, k, key_at, [](int j) { return j; }, T, need_eq, lane, out);
   }
 }
 
@@ -2024,23 +2243,46 @@ __global__ void confusion_kernel(const int32_t* __restrict__ pred, const int64_t
 // --------------------------------------------------------------------------------------------
 // launchers
 // --------------------------------------------------------------------------------------------
+// The bounded select pays where a row's candidates fit the warp's buffer with room to spare.  Were
+// the row's columns in random order, a group's minimum would lie below distance quantile p with
+// probability 1 - (1 - p)^AFF_GROUP; the k-th smallest minimum sits where that equals k / groups,
+// and about nn p columns lie below it.  That count must be at most half the buffer.  Rows that
+// still overflow take the exact fallback.
+static bool bounded_select_pays(int nn, int k) {
+  const double groups = (nn + AFF_GROUP - 1) / AFF_GROUP;
+  if (groups <= k) return false;
+  return nn * (1.0 - pow(1.0 - k / groups, 1.0 / AFF_GROUP)) <= SELB_CAP / 2;
+}
+
 int launch_affinity(const float* F, int64_t graph_rows, int64_t row_off, const uint8_t* valid,
-                    int G, int nn, int D, int k, float sigma, float* norms, float* D2, int32_t* nbr,
-                    float* sim, cudaStream_t st, const StageRec* sr) {
+                    int G, int nn, int D, int k, float sigma, float* norms, float* D2,
+                    unsigned* gmin, int32_t* nbr, float* sim, cudaStream_t st,
+                    const StageRec* sr) {
   if (D % 4 != 0 || D > 32 * LP_MAX_F4 || k > 1024 || nn > 65535) return R3DFS_E_UNSUPPORTED;
   R3DFS_TRY(launch_row_norms_batched(F + row_off * D, graph_rows * D, G, nn, D, D, norms, st));
   // Squared-L2 matrix in Gram form (what faiss.IndexFlatL2 ranks by, models/mpti.py:733-735):
-  // the TMEM-operand kernel (linear_ts_kernel<128, true>); the register-fed one when TMA cannot
-  // address the feature matrix, or under R3DFS_DIST_TC=1 in the measurement build
+  // the TMEM-operand kernel (linear_ts_kernel<128, true>), which also writes the group minima that
+  // bound the select; the register-fed one, without bounds, when TMA cannot address the feature
+  // matrix, or under R3DFS_DIST_TC=1 in the measurement build
+  static const bool sel_block = R3DFS_GETENV("R3DFS_SELECT_BLOCK") != nullptr;
+  if (sel_block || !bounded_select_pays(nn, k) || nn % 4 != 0 ||
+      (reinterpret_cast<uintptr_t>(valid) & 3) != 0)
+    gmin = nullptr;
   static const bool dist_tc = R3DFS_GETENV("R3DFS_DIST_TC") != nullptr;
   int rc = dist_tc ? R3DFS_E_UNSUPPORTED
-                   : launch_gram_dist_ts(F, graph_rows, row_off, G, nn, D, norms, D2, st);
-  if (rc == R3DFS_E_UNSUPPORTED)
+                   : launch_gram_dist_ts(F, graph_rows, row_off, G, nn, D, norms, D2, valid, gmin,
+                                         st);
+  if (rc == R3DFS_E_UNSUPPORTED) {
+    gmin = nullptr;
     rc = launch_gram_dist_tc(F, graph_rows, row_off, G, nn, D, norms, D2, st);
+  }
   R3DFS_TRY(rc);
   if (sr) sr->mark(R3DFS_ST_DIST, st);
-  static const bool sel_block = R3DFS_GETENV("R3DFS_SELECT_BLOCK") != nullptr;
-  if (nn <= 32 * 80 && !sel_block) {
+  if (gmin) {
+    knn_select_bounded_kernel<<<dim3((nn + SELB_WARPS - 1) / SELB_WARPS, G), SELB_WARPS * 32, 0,
+                                st>>>(D2, valid, gmin, nn, k, nbr);
+    R3DFS_CHECK_LAUNCH();
+  } else if (nn <= 32 * 80 && !sel_block) {
     const dim3 gs((nn + SELW_WARPS - 1) / SELW_WARPS, G);
     if (nn <= 32 * 40)
       knn_select_warp_kernel<40><<<gs, SELW_WARPS * 32, 0, st>>>(D2, valid, nn, k, nbr);

@@ -2,9 +2,14 @@
 #pragma once
 #include "common.cuh"
 
+// gmin: affinity_gmin_words(G, nn) u32 of scratch for the group minima that bound the select
 int launch_affinity(const float* F, int64_t graph_rows, int64_t row_off, const uint8_t* valid,
-                    int G, int nn, int D, int k, float sigma, float* norms, float* D2, int32_t* nbr,
-                    float* sim, cudaStream_t st, const StageRec* sr = nullptr);
+                    int G, int nn, int D, int k, float sigma, float* norms, float* D2,
+                    unsigned* gmin, int32_t* nbr, float* sim, cudaStream_t st,
+                    const StageRec* sr = nullptr);
+inline size_t affinity_gmin_words(size_t G, size_t nn) {
+  return G * nn * (size_t)aff_gstride((int)nn);
+}
 int launch_label_propagate(const int32_t* nbr, float* sim, const uint8_t* valid, int G, int nn,
                            int k, const float* Y, int nc, float alpha, float tol, int max_iter,
                            int32_t* in_cnt, int32_t* in_ptr, int32_t* in_src, float* in_w,

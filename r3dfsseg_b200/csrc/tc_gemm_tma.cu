@@ -263,12 +263,17 @@ __device__ __forceinline__ float4 ts_raw_chunk(const unsigned char* tile, int r,
 // linear_tc_kernel<128, true>, which this replaces): X = W = the node features of graph blockIdx.z
 // (rows zrow * z + row0 .. of the matrix behind tmX), Y[m][n] = (s[m] + s[n]) - 2 acc with s the
 // squared row norms; only the tiles on and above the diagonal are computed, an off-diagonal tile
-// is stored twice (as is, and mirrored).
+// is stored twice (as is, and mirrored).  With gmin, every stored value also enters its row's
+// group minimum: gmin[z][row][col / AFF_GROUP] (row stride aff_gstride(nn)) = min dist_key over the
+// group's columns, where the row's own column and the columns of invalid nodes (valid[z][col] == 0)
+// count as 0xffffffff.
 template <int BN, bool DIST = false>
 __global__ __launch_bounds__(TM_ALL_THREADS, 2) void linear_ts_kernel(
     const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmW,
     const float* __restrict__ s, const float* __restrict__ t, int act, int64_t M, int K, int Nout,
-    float* __restrict__ Y, int ldy, RowMap map, int64_t zrow = 0, int64_t row0 = 0) {
+    float* __restrict__ Y, int ldy, RowMap map, int64_t zrow = 0, int64_t row0 = 0,
+    const uint8_t* __restrict__ valid = nullptr, unsigned* __restrict__ gmin = nullptr) {
+  static_assert(!DIST || (BN == TM_BM && 32 % AFF_GROUP == 0), "DIST: square tiles, groups in a chunk");
   if (DIST && blockIdx.y < blockIdx.x) return;
   extern __shared__ unsigned char smem_raw[];
   using S = TsSmem<BN>;
@@ -294,10 +299,14 @@ __global__ __launch_bounds__(TM_ALL_THREADS, 2) void linear_ts_kernel(
   constexpr uint32_t COL_A = 128;
   const int KB = (K + TM_BK - 1) / TM_BK;
 
-  if (!DIST && tid < BN) {
+  if (tid < BN) {
     const int n = n0 + tid;
-    s_sc[tid] = (s && n < Nout) ? s[n] : 1.f;
-    s_sh[tid] = (t && n < Nout) ? t[n] : 0.f;
+    if (DIST) {  // the column norms
+      s_sc[tid] = n < Nout ? s[n] : 0.f;
+    } else {
+      s_sc[tid] = (s && n < Nout) ? s[n] : 1.f;
+      s_sh[tid] = (t && n < Nout) ? t[n] : 0.f;
+    }
   }
   if (tid == 0) {
     for (int i = 0; i < TS_RAW_STAGES; ++i) tc::mbar_init(&bar_full[i], 1);
@@ -410,7 +419,7 @@ __global__ __launch_bounds__(TM_ALL_THREADS, 2) void linear_ts_kernel(
         const int64_t m = (int64_t)m0 + rbase + lane;
         const float sm = (m < M) ? s[m] : 0.f;
 #pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] = (sm + ((nb + j < Nout) ? s[nb + j] : 0.f)) - 2.f * v[j];
+        for (int j = 0; j < 32; ++j) v[j] = (sm + s_sc[cbase + cc + j]) - 2.f * v[j];
         if (blockIdx.y > blockIdx.x && m < M) {
           // mirrored tile: a lane holds one row, so for a fixed column the warp's 32 values are
           // consecutive in the transposed row — coalesced as they stand
@@ -427,6 +436,41 @@ __global__ __launch_bounds__(TM_ALL_THREADS, 2) void linear_ts_kernel(
         const int64_t m = (int64_t)m0 + rbase + r;
         return (m < M) ? Y + map(m) * (int64_t)ldy + nb : nullptr;
       });
+      if (DIST && gmin) {
+        // group minima, read back from the transpose buffer the store just filled: wbuf[r][c] is
+        // row m0 + rbase + r, column nb + c, and lane-indexed reads are conflict-free either way.
+        // A lane stores the 4 minima of its row in this chunk as one 16-byte vector.
+        static_assert(32 / AFF_GROUP == 4, "one uint4 of minima per row and chunk");
+        const int gstride = aff_gstride(Nout);
+        const uint8_t* vz = valid + (int64_t)blockIdx.z * M;
+        uint4* gz = reinterpret_cast<uint4*>(gmin + (int64_t)blockIdx.z * M * gstride);
+        const int64_t m = (int64_t)m0 + rbase + lane;
+        const int self = (blockIdx.x == blockIdx.y) ? (int)(m - nb) : -1;
+        unsigned cvalid = __ballot_sync(0xffffffffu, nb + lane < Nout && vz[nb + lane]);
+        unsigned g4[4] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu};
+#pragma unroll
+        for (int c = 0; c < 32; ++c)
+          g4[c / AFF_GROUP] = min(g4[c / AFF_GROUP], (((cvalid >> c) & 1u) && c != self)
+                                                         ? dist_key(wbuf[lane * 33 + c])
+                                                         : 0xffffffffu);
+        if (m < M && nb < Nout)
+          gz[(m * gstride + nb / AFF_GROUP) / 4] = make_uint4(g4[0], g4[1], g4[2], g4[3]);
+        if (blockIdx.y > blockIdx.x) {  // mirrored: row nb + lane over the columns m0 + rbase + r
+          const int64_t c0 = (int64_t)m0 + rbase;
+          cvalid = __ballot_sync(0xffffffffu, m < M && vz[m]);
+#pragma unroll
+          for (int q = 0; q < 4; ++q) g4[q] = 0xffffffffu;
+#pragma unroll
+          for (int r = 0; r < 32; ++r)
+            g4[r / AFF_GROUP] = min(g4[r / AFF_GROUP], ((cvalid >> r) & 1u)
+                                                           ? dist_key(wbuf[r * 33 + lane])
+                                                           : 0xffffffffu);
+          if (nb + lane < Nout && c0 < M)
+            gz[((int64_t)(nb + lane) * gstride + c0 / AFF_GROUP) / 4] =
+                make_uint4(g4[0], g4[1], g4[2], g4[3]);
+        }
+        __syncwarp();  // the next chunk overwrites wbuf
+      }
     }
   }
   tc::tc_fence_before();
@@ -498,9 +542,11 @@ static int launch_ts_bn(const CUtensorMap& tx, const CUtensorMap& tw, const floa
 }
 
 // D2[g][i][j] = |f_i|^2 + |f_j|^2 - 2 f_i.f_j for G graphs of nn nodes (rows of D floats) on the
-// TMEM-operand kernel; R3DFS_E_UNSUPPORTED when TMA cannot address the feature matrix
+// TMEM-operand kernel (+ the group minima of every row when gmin is given);
+// R3DFS_E_UNSUPPORTED when TMA cannot address the feature matrix
 int launch_gram_dist_ts(const float* F, int64_t graph_rows, int64_t row_off, int G, int nn, int D,
-                        const float* norms, float* D2, cudaStream_t st) {
+                        const float* norms, float* D2, const uint8_t* valid, unsigned* gmin,
+                        cudaStream_t st) {
   if ((D & 3) != 0 || (reinterpret_cast<uintptr_t>(F) & 15) != 0 ||
       (int64_t)G * graph_rows >= (1ll << 31))
     return R3DFS_E_UNSUPPORTED;
@@ -512,7 +558,8 @@ int launch_gram_dist_ts(const float* F, int64_t graph_rows, int64_t row_off, int
   if (e != cudaSuccess) return (int)e;
   dim3 grid((nn + TM_BM - 1) / TM_BM, (nn + 127) / 128, G);
   linear_ts_kernel<128, true><<<grid, TM_ALL_THREADS, S::TOTAL, st>>>(
-      tf, tf, norms, nullptr, 0, nn, D, nn, D2, nn, identity_map(), graph_rows, row_off);
+      tf, tf, norms, nullptr, 0, nn, D, nn, D2, nn, identity_map(), graph_rows, row_off, valid,
+      gmin);
   R3DFS_CHECK_LAUNCH();
   return 0;
 }
