@@ -221,6 +221,8 @@ int r3dfs_affinity_knn(const float* node_feat, const uint8_t* valid, int n_graph
  * zero diagonal; S = D^-1/2 W D^-1/2 with D = rowsum(W) + eps; solve (I - alpha S) Z = Y by FP32
  * conjugate gradients on the sparse graph (the reference inverts the dense matrix).
  * Y, Z: (n_graphs, n_max, n_cls) fp32, n_cls <= 8.  Rows of invalid nodes are written as 0.
+ * n_max <= 8192 for n_cls <= 4 and n_max <= 5376 for n_cls 5..8 (the CG solve stages every node's
+ * search direction in shared memory); larger graphs return R3DFS_E_UNSUPPORTED before any launch.
  * iters_out (n_graphs) int32 / resid_out (n_graphs) fp32: optional CG diagnostics (may be NULL). */
 size_t r3dfs_label_propagate_workspace(int n_graphs, int64_t n_max, int k, int n_cls);
 int r3dfs_label_propagate(const int32_t* nbr, const float* sim, const uint8_t* valid, int n_graphs,
@@ -295,6 +297,11 @@ typedef struct r3dfs_episode_diag {
 /* Number of kernels this thread has launched through the library so far (diagnostic counter). */
 long long r3dfs_launch_count(void);
 
+/* Episode envelope (every episode entry point; the workspace queries return 0 outside it and the
+ * calls R3DFS_E_UNSUPPORTED, before any launch): 1 <= n_way <= 7, 1 <= k_shot <= 32,
+ * n_points >= 64, 1 <= n_subprototypes <= 127, 1 <= k_connect <= 1024, k_connect < n_query *
+ * n_points, and graph nodes = roundup64((n_way + 1) * (n_subprototypes + 1)) + n_query * n_points
+ * <= 8192, or <= 5376 when n_way >= 4 (the label-propagation limit at n_way + 1 classes). */
 size_t r3dfs_mpti_workspace(const r3dfs_episode_cfg_t* h_cfg, int n_episodes);
 
 /* E = n_episodes independent episodes in one call (reference: one per forward call).

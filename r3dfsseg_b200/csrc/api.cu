@@ -519,7 +519,7 @@ int r3dfs_label_propagate(const int32_t* nbr, const float* sim, const uint8_t* v
                           size_t ws_bytes, r3dfs_stream_t stream) {
   if (!nbr || !sim || !valid || !Y || !Z || !wsp || n_graphs <= 0 || n_max <= 0 || k <= 0)
     return R3DFS_E_BADARG;
-  if (n_graphs > 65535) return R3DFS_E_UNSUPPORTED;
+  if (n_graphs > 65535 || n_max > lp_max_nodes(n_cls)) return R3DFS_E_UNSUPPORTED;
   if (ws_bytes < r3dfs_label_propagate_workspace(n_graphs, n_max, k, n_cls))
     return R3DFS_E_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
@@ -621,7 +621,8 @@ int episode_dims(const r3dfs_episode_cfg_t* c, EpisodeDims& d) {
   d.ns_pts = d.C * c->n_points;
   d.cpe = c->n_query + d.C;
   d.ep_rows = (int64_t)d.nn + d.ns_pts;
-  if (d.nn > 8192 || c->k_connect >= d.nq_pts) return R3DFS_E_UNSUPPORTED;
+  // the graph must fit the CG solve at n_way + 1 classes (lp_max_nodes: 8192, 5376 from 4 ways)
+  if (d.nn > lp_max_nodes(d.nc) || c->k_connect >= d.nq_pts) return R3DFS_E_UNSUPPORTED;
   return 0;
 }
 

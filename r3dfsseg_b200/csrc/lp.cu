@@ -677,10 +677,18 @@ __global__ __launch_bounds__(SELB_WARPS * 32) void knn_select_bounded_kernel(
 // --------------------------------------------------------------------------------------------
 // Gaussian similarity of the kept edges (models/mpti.py:745-746) with torch<=1.8
 // pairwise_distance: dist = || f_i - f_j + 1e-6 ||_2 by direct differences, sim = exp(-0.5 (dist/sigma)^2).
-// One warp per node, 8 lanes per neighbour.
+// One warp per node, 8 lanes per neighbour.  VEC: the feature rows are 16-byte aligned (read as
+// float4); otherwise each float4 is assembled from four scalar loads.
 // --------------------------------------------------------------------------------------------
 #define LP_MAX_F4 8
 
+template <bool VEC>
+__device__ __forceinline__ float4 ld_f4(const float* p) {
+  if (VEC) return *reinterpret_cast<const float4*>(p);
+  return make_float4(p[0], p[1], p[2], p[3]);
+}
+
+template <bool VEC>
 __global__ __launch_bounds__(256) void edge_sim_kernel(const float* __restrict__ F,
                                                        int64_t graph_rows, int64_t row_off, int nn,
                                                        int D, const uint8_t* __restrict__ valid,
@@ -694,11 +702,11 @@ __global__ __launch_bounds__(256) void edge_sim_kernel(const float* __restrict__
   const float* Fg = F + ((int64_t)g * graph_rows + row_off) * D;
   const int D4 = D >> 2;
   float4 xf[LP_MAX_F4];
-  const float4* xrow = reinterpret_cast<const float4*>(Fg + (int64_t)i * D);
+  const float* xrow = Fg + (int64_t)i * D;
 #pragma unroll
   for (int u = 0; u < LP_MAX_F4; ++u) {
     int c4 = sub + 8 * u;
-    xf[u] = (c4 < D4) ? xrow[c4] : make_float4(0.f, 0.f, 0.f, 0.f);
+    xf[u] = (c4 < D4) ? ld_f4<VEC>(xrow + 4 * c4) : make_float4(0.f, 0.f, 0.f, 0.f);
   }
   const int32_t* nb = nbr + ((int64_t)g * nn + i) * k;
   float* so = sim + ((int64_t)g * nn + i) * k;
@@ -706,13 +714,13 @@ __global__ __launch_bounds__(256) void edge_sim_kernel(const float* __restrict__
     const int t = t0 + grp;
     const bool ok = t < k;
     const int j = ok ? nb[t] : i;
-    const float4* yrow = reinterpret_cast<const float4*>(Fg + (int64_t)j * D);
+    const float* yrow = Fg + (int64_t)j * D;
     float acc = 0.f;
 #pragma unroll
     for (int u = 0; u < LP_MAX_F4; ++u) {
       int c4 = sub + 8 * u;
       if (c4 < D4) {
-        float4 y = yrow[c4];
+        float4 y = ld_f4<VEC>(yrow + 4 * c4);
         float d0 = __fadd_rn(xf[u].x - y.x, 1e-6f), d1 = __fadd_rn(xf[u].y - y.y, 1e-6f),
               d2 = __fadd_rn(xf[u].z - y.z, 1e-6f), d3 = __fadd_rn(xf[u].w - y.w, 1e-6f);
         acc = fmaf(d0, d0, acc);
@@ -1126,6 +1134,7 @@ __global__ void normalize_merged_kernel(const int32_t* __restrict__ rowptr,
 #define CG_TAB_HDR 4      // lo, hi, passes, segments of split rows
 #define CG_TAB_INTS (CG_TAB_HDR + 32 * CG_MAXPASS * 2 + CG_MAXPASS * CGC_MAXT * 2)
 #define CG_PK_SMEM (4096 * 4 + 8192 * 4 * 2)
+#define CG_SMEM_MAX (200 * 1024)  // dynamic shared memory of lp_cg_kernel: P + split-row partials
 
 struct CgExchange {
   float slot[2][CG_CL_MAX][CG_MAXC];
@@ -1734,7 +1743,7 @@ static int launch_cg(int CL, int G, size_t smem, cudaStream_t st, const int32_t*
                      float* AP, int32_t* iters_out, float* resid_out, void* scratch,
                      size_t scratch_bytes) {
   cudaError_t e = cudaFuncSetAttribute(lp_cg_kernel<NCV>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, CG_SMEM_MAX);
   if (e != cudaSuccess) return (int)e;
   if (CL > 8) {
     e = cudaFuncSetAttribute(lp_cg_kernel<NCV>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
@@ -2306,11 +2315,27 @@ int launch_affinity(const float* F, int64_t graph_rows, int64_t row_off, const u
     R3DFS_CHECK_LAUNCH();
   }
   if (sr) sr->mark(R3DFS_ST_SELECT, st);
-  edge_sim_kernel<<<dim3((nn + 7) / 8, G), 256, 0, st>>>(F, graph_rows, row_off, nn, D, valid, nbr,
-                                                        k, sigma, sim);
+  const dim3 gs((nn + 7) / 8, G);
+  if ((reinterpret_cast<uintptr_t>(F) & 15) == 0)
+    edge_sim_kernel<true><<<gs, 256, 0, st>>>(F, graph_rows, row_off, nn, D, valid, nbr, k, sigma,
+                                              sim);
+  else  // a feature matrix TMA could not address either (the register-fed GEMM ran)
+    edge_sim_kernel<false><<<gs, 256, 0, st>>>(F, graph_rows, row_off, nn, D, valid, nbr, k, sigma,
+                                               sim);
   R3DFS_CHECK_LAUNCH();
   if (sr) sr->mark(R3DFS_ST_SIM, st);
   return 0;
+}
+
+// Every CTA of lp_cg_kernel stages the whole of P (nn x NCV floats) and the partial sums of up to
+// CG_MAXPART split-row segments (CG_MAXPART x NCV floats) in its CG_SMEM_MAX bytes of dynamic shared
+// memory; cg_pack_kernel's row prefix and the 16-bit merged columns cap any graph at 8192 nodes.
+// NCV = 4 (n_cls <= 4): 8192 nodes; NCV = 8 (n_cls 5..8): 204800 / 32 - 1024 = 5376 nodes.
+int lp_max_nodes(int n_cls) {
+  if (n_cls < 1 || n_cls > CG_MAXC) return 0;
+  const int ncv = n_cls <= 4 ? 4 : 8;
+  const int fit = (int)(CG_SMEM_MAX / (sizeof(float) * ncv)) - CG_MAXPART;
+  return fit < 8192 ? fit : 8192;
 }
 
 // (I - alpha S) X = RHS on merged rows that are already built and normalised (the label-propagation
@@ -2324,7 +2349,7 @@ int launch_lp_solve(const int32_t* rowptr, const int32_t* rowlen, const uint16_t
   // padded vector width: one or two float4 per node
   const int ncv = nc <= 4 ? 4 : 8;
   const size_t smem_cg = sizeof(float) * (size_t)nn * ncv;
-  if (smem_cg > 200 * 1024) return R3DFS_E_UNSUPPORTED;
+  if (smem_cg > CG_SMEM_MAX) return R3DFS_E_UNSUPPORTED;
   int rc = -1000;
   if (latency) {  // matrix resident in shared memory, groups of CTAs (cooperative launch)
     const size_t scratch_floats = (size_t)G * nn * ncv;
@@ -2335,6 +2360,7 @@ int launch_lp_solve(const int32_t* rowptr, const int32_t* rowlen, const uint16_t
     if (rc == 0) return 0;
     if (rc != -1000) return rc;
   }
+  if (nn > lp_max_nodes(nc)) return R3DFS_E_UNSUPPORTED;  // the cluster solve's limit
   // One CTA per SM (the kernel keeps a queue of matrix rounds in 128 registers per thread), so a
   // batch of graphs gets as many CTAs per graph as keep ALL graphs in flight in one wave (25 graphs
   // on 148 SMs: clusters of 5); a handful of graphs gets 16.  A warp keeps the metadata of at most

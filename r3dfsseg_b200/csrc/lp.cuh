@@ -32,6 +32,9 @@ int launch_lp_solve(const int32_t* rowptr, const int32_t* rowlen, const uint16_t
                     int nc, float alpha, float tol, int max_iter, float* Z, float* X, float* R,
                     float* P, float* AP, int32_t* iters_out, float* resid_out, cudaStream_t st,
                     bool latency = false, void* scratch = nullptr, size_t scratch_bytes = 0);
+// Largest graph (nodes) the cluster CG solve of launch_lp_solve takes at n_cls classes (0 when n_cls
+// is outside 1..8): 8192 for n_cls <= 4, 5376 for n_cls 5..8.
+int lp_max_nodes(int n_cls);
 // latency = true (a handful of graphs, e.g. the single episode of a training step): the whole GPU
 // works on min(G, 4) graphs at a time with the matrix resident in shared memory (lp_cg_group_kernel);
 // the default is one thread-block cluster per graph, which has the higher throughput on a batch.

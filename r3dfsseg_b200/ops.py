@@ -422,8 +422,9 @@ def _episode_ws(need: int, cfg: EpisodeCfg, dev: torch.device,
             "episode configuration outside what libr3dfs is built for: n_way 1..7, k_shot 1..32, "
             "n_points >= 64, n_subprototypes 1..127, k_connect 1..1024 and < n_queries * n_points, "
             "graph nodes = roundup64((n_way + 1) * (n_subprototypes + 1)) + n_queries * n_points "
-            "<= 8192 (the merged rows index columns with 16 bits and the CG kernels stage 8192 "
-            f"nodes); got n_way={cfg.n_way} k_shot={cfg.k_shot} n_query={cfg.n_query} "
+            "<= 8192, and <= 5376 when n_way >= 4 (the merged rows index columns with 16 bits, and "
+            "the CG solve stages all nodes in shared memory: 8192 nodes at up to 4 classes, 5376 at "
+            f"5 to 8); got n_way={cfg.n_way} k_shot={cfg.k_shot} n_query={cfg.n_query} "
             f"n_points={cfg.n_points} n_subprototypes={cfg.n_subprototypes} "
             f"k_connect={cfg.k_connect}")
     return workspace if workspace is not None and workspace.numel() >= need else _ws(need, dev)

@@ -38,6 +38,35 @@ def test_workspace_queries_are_pure_host_calls():
     assert L.r3dfs_knn_workspace(4, 9, 2048, 20) > 0
 
 
+def test_episode_envelope_follows_the_cg_node_limit():
+    """The episode workspace queries refuse a graph the CG solve cannot stage: 8192 nodes up to
+    3 ways (n_cls <= 4), 5376 from 4 ways on (n_cls 5..8 pad P to 8 floats a node), where
+    nodes = roundup64((n_way + 1) * (n_subprototypes + 1)) + n_query * n_points."""
+    from r3dfsseg_b200 import _lib, ops
+    L = _lib.lib()
+    # the largest accepted: 4-way, 4 queries x 1216 points (512 + 4864 = 5376 nodes) and the
+    # benchmark's 2-way episode with two 2048-point queries (320 + 4096 = 4416 nodes)
+    for cfg in (ops.make_cfg(4, 1, 4, 1216), ops.make_cfg(2, 5, 2, 2048),
+                ops.make_cfg(3, 1, 3, 2560), ops.make_cfg(7, 1, 7, 640)):
+        assert L.r3dfs_mpti_workspace(cfg, 1) > 0
+        assert L.r3dfs_mpti_query_workspace(cfg, 1) > 0
+        assert L.r3dfs_mpti_support_workspace(cfg, 1) > 0
+    # rejected: 4-way at 1536 points (512 + 6144 = 6656 nodes), a 4-way query of three 2048-point
+    # clouds (512 + 6144), 4-way at 1280 points (512 + 5120 = 5632), and 3-way past 8192 nodes
+    for cfg in (ops.make_cfg(4, 1, 4, 1536), ops.make_cfg(4, 1, 3, 2048),
+                ops.make_cfg(4, 1, 4, 1280), ops.make_cfg(3, 1, 3, 2816)):
+        assert L.r3dfs_mpti_workspace(cfg, 1) == 0
+        assert L.r3dfs_mpti_query_workspace(cfg, 1) == 0
+        assert L.r3dfs_mpti_support_workspace(cfg, 1) == 0
+    # the stand-alone solve checks the same limit before it touches any buffer (these addresses
+    # are never dereferenced): n_cls 5 at 5377 nodes, n_cls 4 past 8192, n_cls outside 1..8
+    fake = 4096
+    for n, nc in ((5377, 5), (5377, 8), (8193, 4), (1000, 9)):
+        rc = L.r3dfs_label_propagate(fake, fake, fake, 1, n, 16, fake, nc, 0.99, 1e-6, 200, fake,
+                                     None, None, fake, 1 << 62, None)
+        assert rc == -2, (n, nc, rc)   # R3DFS_E_UNSUPPORTED
+
+
 def test_product_path_rejects_cpu_tensors():
     from r3dfsseg_b200 import ops
     with pytest.raises(RuntimeError, match="CUDA tensors only"):
